@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- frame-pairs/s of the geometry hot path (match + RANSAC H + scan) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4|5]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4|5] [--dump-outputs DIR]
 
 A step is one pass of the hot path over one batch of synthetic input:
   config 2 (default, BASELINE.json configs[1]): 2048 SIFT-like keypoints/frame x 10 000 frame
@@ -12,6 +12,9 @@ A step is one pass of the hot path over one batch of synthetic input:
 Inputs are 2.6 GB per step (> 126 MB L2), so no explicit L2 flush is needed between steps.
 Multi-GPU: one process per GPU (torchrun), pairs sharded by contiguous range, weak scaling,
 one NCCL all-gather of the 160-byte shard summaries per step.
+The inputs are generated from fixed seeds, so a run with the same arguments sees the same inputs; --dump-outputs DIR
+writes what the last timed step computed (see dump_outputs) for comparing two builds output for output.
+Nothing is written into the tree the benchmark runs from (it may be read-only), not even bytecode caches.
 """
 import argparse
 import json
@@ -260,6 +263,77 @@ def parity_check(eng, st, keep, coords_h, desc_h, n_hyp, pair_base, n_pairs):
             "bit-exact; H within 1e-3 px)", "failures": bad}
 
 
+# --dump-outputs: per-pair outputs of up to DUMP_PAIRS pairs, per-row outputs of the pairs that hold about DUMP_ROWS query
+# keypoints (both seeded samples of the step's pairs, the second inside the first), DUMP_MAX_BYTES in all
+DUMP_PAIRS = 16384
+DUMP_ROWS = 1 << 18
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, st, r, S, Hf, moved, K):
+    """Writes what the last timed step returned to its caller as out_dir/<name>.npy, float32 or float64 (integer outputs
+    as float64, which holds them exactly), so that two builds can be compared output for output on the same inputs.
+    Outputs past the stage that failed a pair are not defined by the path: they are NaN (per pair) or left out (per row)
+    wherever the pair's final status is not 0.
+
+    per pair, for the pairs in `pair` (indices into the step's pairs): status, n_filtered, m_cnt, S and H_fixed [n,3,3],
+    remap [n*K,2] (the K object points of each pair's frame, configs with remap points); where status is 0: H (the
+    homography compute_homography returns), H1, H1_best, H2_best [n,3,3], best_hyp1/2, best_cnt1/2, inl1/2, static_cnt,
+    static_r, flags.
+    per row, concatenated over the pairs in `row_pair`: top2_idx, top2_d2 [.,2] and surv over the query keypoints;
+    m_idx [.,2] and m_pts [.,4] over the matches, with mask1 and mask1_best (NaN where status is not 0); static_pts [.,4],
+    mask2 and mask2_best over the static points of the pairs whose status is 0."""
+    import torch
+    P = int(r.status.numel())
+    perm = np.random.default_rng(0).permutation(P)
+    pairs = np.sort(perm[:DUMP_PAIRS])
+    row_pairs = np.sort(perm[:max(1, DUMP_ROWS // max(st.max_kp, 1))])
+
+    def take(t, idx):
+        v = t[torch.from_numpy(np.asarray(idx, np.int64)).to(t.device)].cpu().numpy()
+        return v if v.dtype in (np.float32, np.float64) else v.astype(np.float64)
+
+    status = take(r.status, pairs)
+    out = {"pair": pairs.astype(np.float64), "status": status, "n_filtered": take(r.n_filtered, pairs),
+           "m_cnt": take(r.m_cnt, pairs), "S": take(S, pairs).reshape(-1, 3, 3), "H_fixed": take(Hf, pairs).reshape(-1, 3, 3)}
+    if moved is not None:
+        out["remap"] = take(moved, (pairs[:, None] * K + np.arange(K)).ravel())
+    late = {"H": r.H, "H1": r.H1, "H1_best": r.extra["H1_best"], "H2_best": r.extra["H2_best"], "best_hyp1": r.best_hyp1,
+            "best_hyp2": r.best_hyp2, "best_cnt1": r.best_cnt1, "best_cnt2": r.best_cnt2, "inl1": r.inl1, "inl2": r.inl2,
+            "static_cnt": r.static_cnt, "static_r": r.static_r, "flags": r.flags}
+    for name, t in late.items():
+        v = take(t, pairs)
+        v[status != 0] = np.nan
+        out[name] = v.reshape(-1, 3, 3) if v.ndim == 2 else v
+
+    off = take(r.out_off, row_pairs).astype(np.int64)
+    n_q = st.n_kp_h[take(r.pair_q, row_pairs).astype(np.int64)]
+    ok = take(r.status, row_pairs) == 0
+    m_cnt = take(r.m_cnt, row_pairs).astype(np.int64)
+    s_cnt = np.where(ok, take(r.static_cnt, row_pairs), 0).astype(np.int64)
+    span = lambda cnt: np.concatenate([np.arange(o, o + c) for o, c in zip(off, cnt)])
+    q_rows, m_rows, s_rows = span(n_q), span(m_cnt), span(s_cnt)
+    out["row_pair"] = row_pairs.astype(np.float64)
+    for name in ("top2_idx", "top2_d2", "surv"):
+        out[name] = take(getattr(r, name), q_rows)
+    out["m_idx"], out["m_pts"] = take(r.m_idx, m_rows), take(r.m_pts, m_rows)
+    for name in ("mask1", "mask1_best"):
+        v = take(getattr(r, name), m_rows)
+        v[np.repeat(~ok, m_cnt)] = np.nan
+        out[name] = v
+    out["static_pts"] = take(r.static_pts, s_rows)
+    for name in ("mask2", "mask2_best"):
+        out[name] = take(getattr(r, name), s_rows)
+
+    total = sum(v.nbytes for v in out.values())
+    if total > DUMP_MAX_BYTES:
+        raise SystemExit(f"bench.py: --dump-outputs would write {total} bytes, more than {DUMP_MAX_BYTES}")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v)
+    print(f"bench.py: {len(out)} arrays of the last timed step ({total / 1e6:.1f} MB) written to {out_dir}", file=sys.stderr)
+
+
 def run_ours(args, cfg):
     import torch
     import torch.distributed as dist
@@ -338,12 +412,13 @@ def run_ours(args, cfg):
             if timed: e[2].record()
             S, Hf = scan_sharded(eng, r.H, r.status, True)     # one all-gather of 160 B per rank when world > 1
             if timed: e[3].record()
+            moved = None
             if obj is not None:
-                eng.remap(obj[0], obj[1], S, 400.0 / 1920.0, 224.0 / 1080.0, False)     # frames 2.. of the shard
+                moved = eng.remap(obj[0], obj[1], S, 400.0 / 1920.0, 224.0 / 1080.0, False)     # frames 2.. of the shard
             if timed: e[4].record()
             h1 = dict(mask_best=r.mask1_best)
             h2 = dict(mask_best=r.mask2_best, H=r.H)
-            return (r, h1, r.static_pts, r.static_cnt, h2), S, e
+            return (r, h1, r.static_pts, r.static_cnt, h2), (S, Hf, moved), e
         return step
 
     def timed_run(step, steps, warmup):
@@ -355,7 +430,7 @@ def run_ours(args, cfg):
         w_begin = time.time()
         t0.record()
         for _ in range(steps):
-            keep, S, e = step(True)
+            keep, scan, e = step(True)
             evs.append(e)
         t1.record()
         sync_all()
@@ -365,7 +440,7 @@ def run_ours(args, cfg):
         if os.environ.get("EVZ_BENCH_DEBUG"):
             print(f"[rank {rank}] per-step stage ms:\n{np.round(per_step, 3)}", file=sys.stderr, flush=True)
         stage = per_step.mean(0)
-        return total_ms, stage, keep, S, (w_begin, w_end)
+        return total_ms, stage, keep, scan, (w_begin, w_end)
 
     tile = int(cfg.get("tile", 1))
     st, desc_h, coords_h = make_store(P, tile if P + 1 >= 2 * tile else 1, strong)
@@ -375,13 +450,15 @@ def run_ours(args, cfg):
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    total_ms, stage, keep, S, (w_begin, w_end) = timed_run(step, args.steps, max(args.warmup, 3))
+    total_ms, stage, keep, scan, (w_begin, w_end) = timed_run(step, args.steps, max(args.warmup, 3))
     if os.environ.get("EVZ_BENCH_DEBUG"):
         print(f"[rank {rank}] total {total_ms / args.steps:.3f} ms/step, stages {[round(float(x), 3) for x in stage]}", file=sys.stderr, flush=True)
     clocks = sampler.stop(w_begin, w_end) if rank == 0 else None
     # per-launch duration of the dominant kernel (the last min(steps, 16) launches, all inside the timed region)
     kern_ms = [eng.match_kernel_ms(k) for k in range(min(args.steps, 16))]
     r = keep[0]
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, st, r, *scan, K)
     n_ok = int((r.status == 0).sum().item())
     mean_matches = float(r.m_cnt.float().mean().item())
     mean_static = float(keep[3].float().mean().item())
@@ -394,7 +471,7 @@ def run_ours(args, cfg):
     flann_rows = [(int(st.row_off_h[q]), int(st.n_kp_h[q])) for q in range(1, flann_pairs + 1)]
     flann_idx = [r.top2_idx[o:o + n, 0].cpu().numpy() for o, n in flann_rows]
     flann_surv = [r.surv[o:o + n].cpu().numpy().astype(bool) for o, n in flann_rows]
-    del r, keep, S
+    del r, keep, scan
 
     # ---- end to end through the public host API (pinned host buffers in, host arrays out)
     out = None
@@ -441,7 +518,7 @@ def run_ours(args, cfg):
         P5 = (args.pairs * 10 if args.pairs else c5cfg["pairs"]) // world
         st5, _, _ = make_store(P5, c5cfg["tile"], True, want_host=False)
         step5 = make_step(st5, P5, rank * P5, c5cfg["remap_points"], c5cfg["n_hyp"])
-        t5, stage5, keep5, S5, _ = timed_run(step5, 2, 2)
+        t5, stage5, keep5, (S5, _, _), _ = timed_run(step5, 2, 2)
         # scan check: every rank gathers all G / status / S; the single-GPU scan over the whole video must reproduce
         # the sharded one
         G5, s5 = keep5[4]["H"].contiguous(), keep5[0].status.contiguous()
@@ -538,6 +615,8 @@ def run_ours(args, cfg):
 
 
 def main():
+    sys.dont_write_bytecode = True
+    os.environ["PYTHONDONTWRITEBYTECODE"] = "1"         # and in the CPU arm's worker processes
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=20)
@@ -548,7 +627,11 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the bounded CPU baseline")
     ap.add_argument("--no-parity", action="store_true", help="skip the oracle check of the last timed step")
     ap.add_argument("--no-c5", action="store_true", help="N > 1: skip the sharded 100k-pair video (config 5) and its scan check")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="--impl ours: write the outputs of the last timed step to DIR/<name>.npy (rank 0's pairs when N > 1)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     cfg = CONFIGS[args.config]
     if args.impl == "reference":
         run_reference(args, cfg)
