@@ -58,10 +58,11 @@ extern "C" int evz_set_option(evz_handle* h, int option, int value) {
     if (!h) return EVZ_E_ARG;
     switch (option) {
         case EVZ_OPT_RANSAC_EXACT: h->opt_ransac_exact = value; return EVZ_OK;
-        case EVZ_OPT_MATCH_VARIANT: h->opt_match_variant = value; return EVZ_OK;
+        case EVZ_OPT_MATCH_VARIANT:
+            EVZ_REQUIRE(h, value == 0 || value == 5, "EVZ_OPT_MATCH_VARIANT must be 0 (default routing) or 5 (key-space kernel for every pair)");
+            h->opt_match_variant = value; return EVZ_OK;
         case EVZ_OPT_RANSAC_NO_PRUNE: h->opt_ransac_no_prune = value; return EVZ_OK;
         case EVZ_OPT_TIME_MATCH: h->opt_time_match = value; return EVZ_OK;
-        case EVZ_OPT_MATCH_DEBUG: h->opt_match_debug = value; return EVZ_OK;
         default: EVZ_SET_ERR(h, "evz_set_option: unknown option %d", option); return EVZ_E_ARG;
     }
 }

@@ -21,12 +21,11 @@ struct evz_handle {
     size_t scratch_bytes = 0;
     // cached TMA descriptor of the descriptor store
     CUtensorMap tmap;
-    CUtensorMap tmap_half;         // same store, 128-row boxes (CTA-pair match kernel)
     const void* tmap_ptr = nullptr;
     int64_t tmap_rows = 0;
     evz_encode_tiled_fn encode = nullptr;
     // cudaFuncSetAttribute(MaxDynamicSharedMemorySize) is per device: remembered per handle, not per process
-    unsigned attr_match = 0;       // bit per match kernel instance
+    unsigned attr_match = 0;       // bit 0: key-space kernel, bit 1: V-space kernel
     bool attr_static = false, attr_canon = false, attr_concat = false;
     int attr_filter = 0, attr_score = 0, attr_refit = 0;
     // options (evz_set_option)
@@ -34,7 +33,6 @@ struct evz_handle {
     int opt_ransac_no_prune = 0;
     int opt_match_variant = 0;
     int opt_time_match = 0;
-    int opt_match_debug = 0;
     // EVZ_OPT_TIME_MATCH: ring of event pairs around the main match kernel
     cudaEvent_t match_ev[16][2] = {};
     bool match_ev_made = false;

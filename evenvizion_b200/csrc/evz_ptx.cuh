@@ -9,15 +9,6 @@ namespace evz {
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
     return static_cast<uint32_t>(__cvta_generic_to_shared(p));
 }
-__device__ __forceinline__ uint32_t lane_id() {
-    uint32_t l; asm volatile("mov.u32 %0, %%laneid;" : "=r"(l)); return l;
-}
-__device__ __forceinline__ bool elect_one() {
-    uint32_t pred;
-    asm volatile("{\n\t.reg .pred p;\n\telect.sync _|p, 0xffffffff;\n\tselp.u32 %0, 1, 0, p;\n\t}" : "=r"(pred));
-    return pred != 0;
-}
-
 // ---------------------------------------------------------------- mbarrier
 __device__ __forceinline__ void mbar_init(uint64_t* bar, uint32_t count) {
     asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" :: "r"(smem_u32(bar)), "r"(count) : "memory");
@@ -133,59 +124,6 @@ __device__ __forceinline__ void umma_commit(uint64_t* bar) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];"
                  :: "r"(smem_u32(bar)) : "memory");
 }
-// ---------------------------------------------------------------- clusters / CTA pairs (cta_group::2)
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r;
-}
-// all threads of all CTAs of the cluster
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// shared::cluster address of `smem_addr` (a shared::cta address of this CTA) in the CTA of rank `rank`
-__device__ __forceinline__ uint32_t mapa_u32(uint32_t smem_addr, uint32_t rank) {
-    uint32_t r; asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(smem_addr), "r"(rank)); return r;
-}
-// arrive on an mbarrier of any CTA of the cluster (address from mapa_u32)
-__device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {
-    asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" :: "r"(cluster_addr) : "memory");
-}
-// spinning wait on a local mbarrier whose arrivals come from the peer CTA (cluster-scope acquire)
-__device__ __forceinline__ void mbar_wait_spin_cluster(uint64_t* bar, uint32_t parity) {
-    uint32_t ok;
-    do {
-        asm volatile("{\n\t.reg .pred p;\n\t"
-                     "mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-                     "selp.u32 %0, 1, 0, p;\n\t}"
-                     : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-        if (!ok) __nanosleep(20);
-    } while (!ok);
-}
-__device__ __forceinline__ void tmem_alloc_pair(uint32_t* smem_result, uint32_t ncols) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;"
-                 :: "r"(smem_u32(smem_result)), "r"(ncols) : "memory");
-}
-__device__ __forceinline__ void tmem_relinquish_pair() {
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc_pair(uint32_t taddr, uint32_t ncols) {
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" :: "r"(taddr), "r"(ncols) : "memory");
-}
-// D[tmem of both CTAs] (+)= A . B^T, one 256 x N x 32 step of a CTA pair: rows 0-127 of A and D live in the
-// leader CTA (rank 0), rows 128-255 in its peer; each CTA holds N/2 rows of B at the same shared-memory
-// offset.  Issued by ONE thread of the leader CTA.
-__device__ __forceinline__ void umma_i8_pair(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
-    asm volatile("{\n\t.reg .pred p;\n\t"
-                 "setp.ne.b32 p, %4, 0;\n\t"
-                 "tcgen05.mma.cta_group::2.kind::i8 [%0], %1, %2, %3, p;\n\t}"
-                 :: "r"(tmem_d), "l"(desc_a), "l"(desc_b), "r"(idesc), "r"(accumulate) : "memory");
-}
-// arrive on the mbarrier at this shared-memory offset in BOTH CTAs of the pair when all previously issued
-// tcgen05.mma of this thread have completed
-__device__ __forceinline__ void umma_commit_pair(uint64_t* bar) {
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-                 :: "r"(smem_u32(bar)), "h"(static_cast<uint16_t>(3)) : "memory");
-}
-
 // TMEM -> registers: this warp's 32 lanes x 32 consecutive 32-bit columns.
 __device__ __forceinline__ void tmem_ld_32x32b_x32(uint32_t taddr, uint32_t (&r)[32]) {
     asm volatile("tcgen05.ld.sync.aligned.32x32b.x32.b32 "
@@ -197,59 +135,12 @@ __device__ __forceinline__ void tmem_ld_32x32b_x32(uint32_t taddr, uint32_t (&r)
                    "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
                  : "r"(taddr) : "memory");
 }
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
 // wait for outstanding tcgen05.ld and make the destination registers depend on the wait, so that
 // neither nvcc nor ptxas can schedule a use of them ahead of it
 __device__ __forceinline__ void tmem_ld_wait_dep(uint32_t (&r)[32]) {
     asm volatile("tcgen05.wait::ld.sync.aligned;"
                  : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]), "+r"(r[8]), "+r"(r[9]), "+r"(r[10]), "+r"(r[11]), "+r"(r[12]), "+r"(r[13]), "+r"(r[14]), "+r"(r[15]), "+r"(r[16]), "+r"(r[17]), "+r"(r[18]), "+r"(r[19]), "+r"(r[20]), "+r"(r[21]), "+r"(r[22]), "+r"(r[23]), "+r"(r[24]), "+r"(r[25]), "+r"(r[26]), "+r"(r[27]), "+r"(r[28]), "+r"(r[29]), "+r"(r[30]), "+r"(r[31]));
 }
-
-// TMEM -> registers: this warp's 32 lanes x 16 consecutive 32-bit columns.
-__device__ __forceinline__ void tmem_ld_32x32b_x16(uint32_t taddr, uint32_t (&r)[16]) {
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-                 "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]),
-                   "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15])
-                 : "r"(taddr) : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait_dep(uint32_t (&r)[16]) {
-    asm volatile("tcgen05.wait::ld.sync.aligned;"
-                 : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]), "+r"(r[8]), "+r"(r[9]), "+r"(r[10]), "+r"(r[11]), "+r"(r[12]), "+r"(r[13]), "+r"(r[14]), "+r"(r[15]));
-}
-
-// TMEM -> registers: this warp's 32 lanes x 64 consecutive 32-bit columns.
-__device__ __forceinline__ void tmem_ld_32x32b_x64(uint32_t taddr, uint32_t (&r)[64]) {
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x64.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31, %32, %33, %34, %35, %36, %37, %38, %39, %40, %41, %42, %43, %44, %45, %46, %47, %48, %49, %50, %51, %52, %53, %54, %55, %56, %57, %58, %59, %60, %61, %62, %63}, [%64];"
-                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]), "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]), "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]), "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31]), "=r"(r[32]), "=r"(r[33]), "=r"(r[34]), "=r"(r[35]), "=r"(r[36]), "=r"(r[37]), "=r"(r[38]), "=r"(r[39]), "=r"(r[40]), "=r"(r[41]), "=r"(r[42]), "=r"(r[43]), "=r"(r[44]), "=r"(r[45]), "=r"(r[46]), "=r"(r[47]), "=r"(r[48]), "=r"(r[49]), "=r"(r[50]), "=r"(r[51]), "=r"(r[52]), "=r"(r[53]), "=r"(r[54]), "=r"(r[55]), "=r"(r[56]), "=r"(r[57]), "=r"(r[58]), "=r"(r[59]), "=r"(r[60]), "=r"(r[61]), "=r"(r[62]), "=r"(r[63])
-                 : "r"(taddr) : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait_dep(uint32_t (&r)[64]) {
-    asm volatile("tcgen05.wait::ld.sync.aligned;"
-                 : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]), "+r"(r[8]), "+r"(r[9]), "+r"(r[10]), "+r"(r[11]), "+r"(r[12]), "+r"(r[13]), "+r"(r[14]), "+r"(r[15]), "+r"(r[16]), "+r"(r[17]), "+r"(r[18]), "+r"(r[19]), "+r"(r[20]), "+r"(r[21]), "+r"(r[22]), "+r"(r[23]), "+r"(r[24]), "+r"(r[25]), "+r"(r[26]), "+r"(r[27]), "+r"(r[28]), "+r"(r[29]), "+r"(r[30]), "+r"(r[31]), "+r"(r[32]), "+r"(r[33]), "+r"(r[34]), "+r"(r[35]), "+r"(r[36]), "+r"(r[37]), "+r"(r[38]), "+r"(r[39]), "+r"(r[40]), "+r"(r[41]), "+r"(r[42]), "+r"(r[43]), "+r"(r[44]), "+r"(r[45]), "+r"(r[46]), "+r"(r[47]), "+r"(r[48]), "+r"(r[49]), "+r"(r[50]), "+r"(r[51]), "+r"(r[52]), "+r"(r[53]), "+r"(r[54]), "+r"(r[55]), "+r"(r[56]), "+r"(r[57]), "+r"(r[58]), "+r"(r[59]), "+r"(r[60]), "+r"(r[61]), "+r"(r[62]), "+r"(r[63]));
-}
-
-// TMEM -> registers, shape 16x256b.x2: 16 lanes x 16 consecutive 32-bit columns.  Thread t receives, of lane
-// (lane base + t/4): r0, r1 = columns 2(t%4), 2(t%4)+1 and r4, r5 = columns 8+2(t%4), 8+2(t%4)+1; r2, r3, r6, r7 = the same
-// columns of lane (lane base + 8 + t/4) -- i.e. a quad of threads holds one whole 16-column row segment (measured:
-// scripts/microbench/mb2.cu "ld16").  The lane base is the warp's lane quarter or that + 16.
-__device__ __forceinline__ void tmem_ld_16x256b_x2(uint32_t taddr, uint32_t (&r)[8]) {
-    asm volatile("tcgen05.ld.sync.aligned.16x256b.x2.b32 {%0, %1, %2, %3, %4, %5, %6, %7}, [%8];"
-                 : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7])
-                 : "r"(taddr) : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait_dep(uint32_t (&r)[8]) {
-    asm volatile("tcgen05.wait::ld.sync.aligned;"
-                 : "+r"(r[0]), "+r"(r[1]), "+r"(r[2]), "+r"(r[3]), "+r"(r[4]), "+r"(r[5]), "+r"(r[6]), "+r"(r[7]));
-}
-__device__ __forceinline__ uint32_t redux_or(uint32_t v) {
-    uint32_t r;
-    asm volatile("redux.sync.or.b32 %0, %1, 0xffffffff;" : "=r"(r) : "r"(v));
-    return r;
-}
-// register reallocation between warpgroups (all four warps of a warpgroup execute it)
-template <int kRegs> __device__ __forceinline__ void setmaxnreg_inc() { asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" :: "n"(kRegs)); }
-template <int kRegs> __device__ __forceinline__ void setmaxnreg_dec() { asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" :: "n"(kRegs)); }
 
 __device__ __forceinline__ void named_bar_sync(uint32_t id, uint32_t nthreads) {
     asm volatile("bar.sync %0, %1;" :: "r"(id), "r"(nthreads) : "memory");

@@ -7,9 +7,12 @@
 //
 //  * match_top2_vkernel ("V-space", default; second half of this file): the train norm enters the accumulator
 //    through a fifth K block, so the epilogue is a max tree over raw accumulator values -- about half the
-//    instructions per output of the key-space epilogue.
-//  * match_top2_kernel ("key-space", this half; EVZ_OPT_MATCH_VARIANT 5 / 1 / 2 and the fallback for pairs
-//    whose train frame has a norm range the fifth K block cannot encode).
+//    instructions per output of the key-space epilogue.  Rows it cannot certify are recomputed by
+//    match_fixup_kernel; match_prepare_kernel writes its fifth K block.
+//  * match_top2_kernel ("key-space", this half): the fallback for pairs whose train frame has a norm range the
+//    fifth K block cannot encode, and every pair with EVZ_OPT_MATCH_VARIANT = 5.
+// The other epilogues tried for both kernels, and why they lost, are in DESIGN.md K1; their source is in the
+// history of this file.
 //
 // Key-space epilogue, per accumulator element (row r = query, column c = train):
 //   key = ckey[c] - 512 * acc = ((||t_c||^2 - 2 q.t_c) << 8) | c      (one IMAD on the FMA pipe; the
@@ -21,12 +24,12 @@
 // added once per row after the reduction.
 //
 // The K dimension is only 128, so the kernel is bound by the epilogue's instruction issue, not by
-// the tensor pipe: an exact running top-2 costs 2.5 min/max per element on the ALU pipe (kChunk = 0,
-// kept for A/B).  The default epilogue spends ~1 ALU op per element instead:
-//   * every aligned chunk of kChunk (8 or 16) columns is reduced to its minimum key with 3-input
-//     mins, and a running top-2 of CHUNK minima is kept per thread;
+// the tensor pipe: an exact running top-2 costs 2.5 min/max per element on the ALU pipe.  This
+// epilogue spends ~1 ALU op per element instead:
+//   * every aligned chunk of 8 columns is reduced to its minimum key with 3-input mins, and a
+//     running top-2 of CHUNK minima is kept per thread;
 //   * whenever a chunk minimum beats the thread's running best, the chunk's raw keys are saved to
-//     a per-thread shared-memory slot by two (four) predicated 128-bit stores, so at the end of the
+//     a per-thread shared-memory slot by two predicated 128-bit stores, so at the end of the
 //     item the slot holds the keys of the chunk that contains the nearest neighbour;
 //   * the second neighbour is the smaller of the second-best chunk minimum and the best of the
 //     other keys in that slot -- both exact, no recomputation.
@@ -57,19 +60,19 @@ struct Item {
     int q_row0, nq_left, t_row0, nt, n_tiles, n_sub, out_row0, pad;
 };
 
-// kEW epilogue warps (8); kChunk keys per save slot (8 or 16; 0 = exact per-element top-2, no slots).
-// Every epilogue thread drains two query rows (one per sub-tile); the two accumulators alternate between
-// the sub-tiles.
-template <int kChunk, int kEW>
+// Key-space kernel.  Every epilogue thread drains two query rows (one per sub-tile); the two accumulators
+// alternate between the sub-tiles.
 struct MatchCfg {
-    static constexpr int epi_threads = kEW * 32;
+    static constexpr int epi_warps   = 8;                         // two column halves x four TMEM lane quarters
+    static constexpr int epi_threads = epi_warps * 32;
     static constexpr int threads     = 128 + epi_threads;
     static constexpr int groups      = 2;                         // column groups of the accumulator
     static constexpr int cols        = kBlockT / groups;          // accumulator columns per epilogue thread and tile
     static constexpr int rows_per_thread = 2;                     // query rows (sub-tiles) per epilogue thread
-    static constexpr int acc_readers = kEW;                       // epilogue warps that drain one accumulator
+    static constexpr int acc_readers = epi_warps;                 // epilogue warps that drain one accumulator
+    static constexpr int chunk       = 8;                         // keys per save slot
     static constexpr int part_stride = epi_threads * 16;          // save slots are laid out [sub][part][thread] x 16 B
-    static constexpr int parts       = kChunk / 4;
+    static constexpr int parts       = chunk / 4;
     // offsets into dynamic shared memory (base aligned to 1024)
     static constexpr int q_off     = 0;                               // 2 x 32 KB
     static constexpr int t_off     = q_off + 2 * kQBytes;             // kStages x 32 KB
@@ -84,7 +87,6 @@ struct MatchCfg {
     static constexpr int total     = tmem_off + 16;
     static constexpr int smem_bytes = total + 1024;               // + alignment slack
     static_assert(smem_bytes <= 227 * 1024, "match kernel shared memory exceeds 227 KB");
-    static_assert(kEW == 8, "two column halves x four TMEM lane quarters");
 };
 
 struct MatchArgs {
@@ -107,9 +109,10 @@ struct MatchArgs {
     int32_t* fix_count;        // number of rows left to match_fixup_kernel (reset by match_prepare_kernel)
     int32_t* fix_list;         // [fix_capacity] item * 256 + row
     int fix_capacity;
-    int dbg;                   // EVZ_OPT_MATCH_DEBUG: 1 = the V-space epilogue releases every accumulator without draining it
-    int pair_mode;             // 1: items are (pair, block of 512 query rows) shared by a CTA pair; work item index =
-                               //    2 * list index + CTA rank (match_top2_vkernel_t<2>)
+    int pair_mode;             // always 0.  1 decoded items of 512 query rows for the CTA-pair kernel removed after round 2;
+                               //    the decode stays in load_item because without it the V-space kernel measured 0.2 %
+                               //    slower at ORB width (B200 at 1000 W, same-run A/B: 1.030 vs 1.028 ms per 2 000 pairs;
+                               //    removing only this field did not change that), an effect of code placement
     int n_kb;                  // data K blocks of 32 bytes that hold descriptor bytes: 4 for SIFT (128 B), 1 for ORB (32 B);
                                //    the rest of the 128-byte row is zero padding and is not multiplied (match_top2_vkernel)
 };
@@ -122,12 +125,12 @@ __device__ __forceinline__ Item load_item(const MatchArgs& a, int it) {
     const int qf = a.pair_q[p], tf = a.pair_t[p];
     const int nq = a.n_kp[qf];
     int sub_left = nq - blk * kBlockQ;
-    if (a.pair_mode) {                              // both CTAs of a pair issue the same MMAs: the sub-tile count is
-        sub_left = nq - 2 * blk * kBlockQ;          // that of the first (fuller) block; the second block may be empty
+    if (a.pair_mode) {                              // never taken (see MatchArgs::pair_mode)
+        sub_left = nq - 2 * blk * kBlockQ;
         blk = 2 * blk + (it & 1);
     }
     r.q_row0 = a.row_off[qf] + blk * kBlockQ;
-    r.nq_left = nq - blk * kBlockQ;                 // valid query rows in this block (may exceed 256, or be <= 0 for the peer block)
+    r.nq_left = nq - blk * kBlockQ;                 // valid query rows in this block (may exceed 256)
     r.n_sub = sub_left > 128 ? 2 : 1;
     r.t_row0 = a.row_off[tf];
     r.nt = a.n_kp[tf];
@@ -158,17 +161,15 @@ __device__ __forceinline__ int mad_key(uint32_t acc, int mul, int ck) {
     return r;
 }
 
-// ---- kChunk = 0: exact running top-2 of packed keys, two elements at a time (5 ALU ops / 2 elements)
+// exact running top-2 of packed keys, two elements at a time (5 ALU ops / 2 elements)
 __device__ __forceinline__ void top2_pair(int k0, int k1, int& m1, int& m2) {
     const int lo = min(k0, k1), hi = max(k0, k1);
     m2 = __vimin3_s32(m2, hi, max(m1, lo));
     m1 = min(m1, lo);
 }
 
-// ---- kChunk = 8 / 16: chunk minima + predicated save of the best chunk's keys
-// returns min(cm, m1); when cm < m1 the chunk's keys go to the slot (setp + selp fuse into one
-// VIMNMX with a predicate output)
-template <int kStride>
+// chunk minimum + predicated save of the best chunk's keys: returns min(cm, m1); when cm < m1 the
+// chunk's keys go to the slot (setp + selp fuse into one VIMNMX with a predicate output)
 __device__ __forceinline__ int save_if_less8(int cm, int m1, uint32_t slot, const int* k) {
     int mn;
     asm volatile("{\n\t.reg .pred p;\n\t"
@@ -177,61 +178,28 @@ __device__ __forceinline__ int save_if_less8(int cm, int m1, uint32_t slot, cons
                  "@p st.shared.v4.b32 [%3], {%4, %5, %6, %7};\n\t"
                  "@p st.shared.v4.b32 [%3+%12], {%8, %9, %10, %11};\n\t}"
                  : "=r"(mn) : "r"(cm), "r"(m1), "r"(slot), "r"(k[0]), "r"(k[1]), "r"(k[2]), "r"(k[3]),
-                    "r"(k[4]), "r"(k[5]), "r"(k[6]), "r"(k[7]), "n"(kStride));
-    return mn;
-}
-template <int kStride>
-__device__ __forceinline__ int save_if_less16(int cm, int m1, uint32_t slot, const int* k) {
-    int mn;
-    asm volatile("{\n\t.reg .pred p;\n\t"
-                 "setp.lt.s32 p, %1, %2;\n\t"
-                 "selp.s32 %0, %1, %2, p;\n\t"
-                 "@p st.shared.v4.b32 [%3], {%4, %5, %6, %7};\n\t"
-                 "@p st.shared.v4.b32 [%3+%20], {%8, %9, %10, %11};\n\t"
-                 "@p st.shared.v4.b32 [%3+2*%20], {%12, %13, %14, %15};\n\t"
-                 "@p st.shared.v4.b32 [%3+3*%20], {%16, %17, %18, %19};\n\t}"
-                 : "=r"(mn) : "r"(cm), "r"(m1), "r"(slot), "r"(k[0]), "r"(k[1]), "r"(k[2]), "r"(k[3]),
-                    "r"(k[4]), "r"(k[5]), "r"(k[6]), "r"(k[7]), "r"(k[8]), "r"(k[9]), "r"(k[10]), "r"(k[11]),
-                    "r"(k[12]), "r"(k[13]), "r"(k[14]), "r"(k[15]), "n"(kStride));
+                    "r"(k[4]), "r"(k[5]), "r"(k[6]), "r"(k[7]), "n"(MatchCfg::part_stride));
     return mn;
 }
 
 // 32 accumulator columns (r) against their ckey values (ck): update the thread's running (m1, m2)
-template <int kChunk, int kEW>
 __device__ __forceinline__ void pass32(const uint32_t (&r)[32], const int4 (&ck)[8], int mul, int& m1, int& m2,
-                                       int& b1, int& b2, uint32_t slot) {
-    if (kChunk == 0) {
+                                       uint32_t slot) {
 #pragma unroll
-        for (int j = 0; j < 8; ++j) {
-            top2_pair(mad_key(r[4 * j + 0], mul, ck[j].x), mad_key(r[4 * j + 1], mul, ck[j].y), m1, m2);
-            top2_pair(mad_key(r[4 * j + 2], mul, ck[j].z), mad_key(r[4 * j + 3], mul, ck[j].w), b1, b2);
+    for (int q = 0; q < 4; ++q) {
+        int k[8];
+#pragma unroll
+        for (int j = 0; j < 2; ++j) {
+            const int4 c = ck[q * 2 + j];
+            k[4 * j + 0] = mad_key(r[q * 8 + 4 * j + 0], mul, c.x);
+            k[4 * j + 1] = mad_key(r[q * 8 + 4 * j + 1], mul, c.y);
+            k[4 * j + 2] = mad_key(r[q * 8 + 4 * j + 2], mul, c.z);
+            k[4 * j + 3] = mad_key(r[q * 8 + 4 * j + 3], mul, c.w);
         }
-    } else {
-        constexpr int kC = kChunk == 0 ? 8 : kChunk;
-#pragma unroll
-        for (int q = 0; q < 32 / kC; ++q) {
-            int k[16];
-#pragma unroll
-            for (int j = 0; j < kC / 4; ++j) {
-                const int4 c = ck[q * (kC / 4) + j];
-                k[4 * j + 0] = mad_key(r[q * kC + 4 * j + 0], mul, c.x);
-                k[4 * j + 1] = mad_key(r[q * kC + 4 * j + 1], mul, c.y);
-                k[4 * j + 2] = mad_key(r[q * kC + 4 * j + 2], mul, c.z);
-                k[4 * j + 3] = mad_key(r[q * kC + 4 * j + 3], mul, c.w);
-            }
-            int cm, mn;
-            if (kC == 8) {
-                cm = __vimin3_s32(__vimin3_s32(k[0], k[1], k[2]), __vimin3_s32(k[3], k[4], k[5]), min(k[6], k[7]));
-                mn = save_if_less8<MatchCfg<kC, kEW>::part_stride>(cm, m1, slot, k);
-            } else {
-                const int a = __vimin3_s32(k[0], k[1], k[2]), b = __vimin3_s32(k[3], k[4], k[5]), c = __vimin3_s32(k[6], k[7], k[8]);
-                const int d = __vimin3_s32(k[9], k[10], k[11]), e = __vimin3_s32(k[12], k[13], k[14]);
-                cm = min(__vimin3_s32(a, b, c), __vimin3_s32(d, e, k[15]));
-                mn = save_if_less16<MatchCfg<kC, kEW>::part_stride>(cm, m1, slot, k);
-            }
-            m2 = min(m2, max(m1, cm));
-            m1 = mn;
-        }
+        const int cm = __vimin3_s32(__vimin3_s32(k[0], k[1], k[2]), __vimin3_s32(k[3], k[4], k[5]), min(k[6], k[7]));
+        const int mn = save_if_less8(cm, m1, slot, k);
+        m2 = min(m2, max(m1, cm));
+        m1 = mn;
     }
 }
 
@@ -241,13 +209,10 @@ __device__ __forceinline__ void pass32(const uint32_t (&r)[32], const int4 (&ck)
 // b+1 are issued before batch b is processed, so only the first load of an accumulator is exposed (the two
 // epilogue warps of a scheduler drain the same accumulator in lockstep and cannot hide each other's load
 // latency).
-template <int kChunk, int kEW>
 __device__ __forceinline__ void drain_acc(uint32_t taddr, uint32_t ck, int mul, int& m1, int& m2, uint32_t slot,
                                           uint64_t* acc_empty, int lane) {
-    constexpr int kCols = MatchCfg<kChunk, kEW>::cols;
-    constexpr int kBatches = kCols / 32;
+    constexpr int kBatches = MatchCfg::cols / 32;
     constexpr int kBuf = 2;
-    int b1 = INT_MAX, b2 = INT_MAX;            // kChunk = 0: second interleaved chain
     uint32_t r[kBuf][32];
     int4 ckv[kBuf][8];
     auto issue = [&](int b) {
@@ -265,19 +230,13 @@ __device__ __forceinline__ void drain_acc(uint32_t taddr, uint32_t ck, int mul, 
             __syncwarp();
             if (lane == 0) mbar_arrive(acc_empty);
         }
-        pass32<kChunk, kEW>(r[b % kBuf], ckv[b % kBuf], mul, m1, m2, b1, b2, slot);
-    }
-    if (kChunk == 0) {
-        const int lo = min(m1, b1);
-        m2 = __vimin3_s32(max(m1, b1), m2, b2);
-        m1 = lo;
+        pass32(r[b % kBuf], ckv[b % kBuf], mul, m1, m2, slot);
     }
 }
 
-template <int kChunk, int kEW>
-__global__ void __launch_bounds__(MatchCfg<kChunk, kEW>::threads, 1)
+__global__ void __launch_bounds__(MatchCfg::threads, 1)
 match_top2_kernel(const __grid_constant__ CUtensorMap tmap, const MatchArgs args) {
-    using Cfg = MatchCfg<kChunk, kEW>;
+    using Cfg = MatchCfg;
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     uint8_t* q_s = smem + Cfg::q_off;
@@ -289,11 +248,11 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap, const MatchArgs args
     uint64_t* full = bars;                       // [kStages] train tile landed (TMA tx)
     uint64_t* empty = full + kStages;            // [kStages] MMA commit
     uint64_t* ck_full = empty + kStages;         // [kCkStages] ckey tile landed
-    uint64_t* ck_empty = ck_full + kCkStages;    // [kCkStages] kEW arrivals
+    uint64_t* ck_empty = ck_full + kCkStages;    // [kCkStages] epilogue warp arrivals
     uint64_t* q_full = ck_empty + kCkStages;     // [2] query block landed + item descriptor published
-    uint64_t* q_empty = q_full + 2;              // [2] MMA commit + kEW arrivals
+    uint64_t* q_empty = q_full + 2;              // [2] MMA commit + epilogue warp arrivals
     uint64_t* acc_full = q_empty + 2;            // [2] accumulator ready (MMA commit)
-    uint64_t* acc_empty = acc_full + 2;          // [2] accumulator drained (kEW arrivals)
+    uint64_t* acc_empty = acc_full + 2;          // [2] accumulator drained (epilogue warp arrivals)
     uint32_t* tmem_ptr_s = reinterpret_cast<uint32_t*>(smem + Cfg::tmem_off);
 
     const int warp = threadIdx.x >> 5;
@@ -302,9 +261,9 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap, const MatchArgs args
     if (warp == 0 && lane == 0) {
         tma_prefetch_desc(&tmap);
         for (int i = 0; i < kStages; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
-        for (int i = 0; i < kCkStages; ++i) { mbar_init(&ck_full[i], 1); mbar_init(&ck_empty[i], kEW); }
+        for (int i = 0; i < kCkStages; ++i) { mbar_init(&ck_full[i], 1); mbar_init(&ck_empty[i], Cfg::epi_warps); }
         for (int i = 0; i < 2; ++i) {
-            mbar_init(&q_full[i], 1); mbar_init(&q_empty[i], 1 + kEW);
+            mbar_init(&q_full[i], 1); mbar_init(&q_empty[i], 1 + Cfg::epi_warps);
             mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], Cfg::acc_readers);
         }
         fence_mbar_init();
@@ -424,30 +383,17 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap, const MatchArgs args
                         mbar_wait(&acc_full[acc], aph);
                         tc_fence_after();
                         const uint32_t taddr = tmem_base + acc * kBlockT + colbase + (static_cast<uint32_t>(quarter * 32) << 16);
-                        if (kChunk == 0) {
-                            int m1 = INT_MAX, m2 = INT_MAX;
-                            drain_acc<kChunk, kEW>(taddr, ck, args.neg512, m1, m2, 0u, &acc_empty[acc], lane);
-                            // a later tile only displaces an earlier one with a strictly smaller distance
-#pragma unroll
-                            for (int w = 0; w < 2; ++w) {
-                                const int k = w ? m2 : m1;
-                                if ((k >> 8) < (B1[s] >> 8))      { B2[s] = B1[s]; T2[s] = T1[s]; B1[s] = k; T1[s] = n; }
-                                else if ((k >> 8) < (B2[s] >> 8)) { B2[s] = k; T2[s] = n; }
-                            }
-                        } else {
-                            // the running best enters the tile as a sentinel: a chunk only wins (and is saved)
-                            // with a strictly smaller distance
-                            const int sentinel = (B1[s] & ~255) - sent_adj;
-                            int m1 = sentinel, m2 = INT_MAX;
-                            drain_acc<kChunk, kEW>(taddr, ck, args.neg512, m1, m2, slot0 + s * (Cfg::parts * Cfg::part_stride),
-                                                   &acc_empty[acc], lane);
-                            if (m1 != sentinel) {
-                                const bool demote = m2 == sentinel;      // the old best is the new second best
-                                B2[s] = demote ? B1[s] : m2; T2[s] = demote ? T1[s] : n;
-                                B1[s] = m1; T1[s] = n;
-                            } else if (m2 < (B2[s] & ~255)) {
-                                B2[s] = m2; T2[s] = n;
-                            }
+                        // the running best enters the tile as a sentinel: a chunk only wins (and is saved)
+                        // with a strictly smaller distance
+                        const int sentinel = (B1[s] & ~255) - sent_adj;
+                        int m1 = sentinel, m2 = INT_MAX;
+                        drain_acc(taddr, ck, args.neg512, m1, m2, slot0 + s * (Cfg::parts * Cfg::part_stride), &acc_empty[acc], lane);
+                        if (m1 != sentinel) {
+                            const bool demote = m2 == sentinel;      // the old best is the new second best
+                            B2[s] = demote ? B1[s] : m2; T2[s] = demote ? T1[s] : n;
+                            B1[s] = m1; T1[s] = n;
+                        } else if (m2 < (B2[s] & ~255)) {
+                            B2[s] = m2; T2[s] = n;
                         }
                         ++g;
                     }
@@ -462,24 +408,22 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap, const MatchArgs args
                 V1[s] = T1[s] >= 0 ? B1[s] >> 8 : kAbsent; I1[s] = T1[s] >= 0 ? T1[s] * kBlockT + (B1[s] & 255) : -1;
                 V2[s] = T2[s] >= 0 ? B2[s] >> 8 : kAbsent; I2[s] = T2[s] >= 0 ? T2[s] * kBlockT + (B2[s] & 255) : -1;
             }
-            if (kChunk != 0) {
-                // exact second neighbour: the other keys of the chunk that holds the nearest one
+            // exact second neighbour: the other keys of the chunk that holds the nearest one
 #pragma unroll
-                for (int s = 0; s < kR; ++s) {
-                    if (I1[s] >= 0) {
-                        const int wkey = B1[s];
-                        int cand = INT_MAX;
+            for (int s = 0; s < kR; ++s) {
+                if (I1[s] >= 0) {
+                    const int wkey = B1[s];
+                    int cand = INT_MAX;
 #pragma unroll
-                        for (int part = 0; part < Cfg::parts; ++part) {
-                            const int4 k = lds128(slot0 + s * (Cfg::parts * Cfg::part_stride) + part * Cfg::part_stride);
-                            cand = min(cand, k.x == wkey ? INT_MAX : k.x);
-                            cand = min(cand, k.y == wkey ? INT_MAX : k.y);
-                            cand = min(cand, k.z == wkey ? INT_MAX : k.z);
-                            cand = min(cand, k.w == wkey ? INT_MAX : k.w);
-                        }
-                        const int v = cand >> 8, i = (I1[s] & ~255) + (cand & 255);
-                        if (v < V2[s] || (v == V2[s] && i < I2[s])) { V2[s] = v; I2[s] = i; }
+                    for (int part = 0; part < Cfg::parts; ++part) {
+                        const int4 k = lds128(slot0 + s * (Cfg::parts * Cfg::part_stride) + part * Cfg::part_stride);
+                        cand = min(cand, k.x == wkey ? INT_MAX : k.x);
+                        cand = min(cand, k.y == wkey ? INT_MAX : k.y);
+                        cand = min(cand, k.z == wkey ? INT_MAX : k.z);
+                        cand = min(cand, k.w == wkey ? INT_MAX : k.w);
                     }
+                    const int v = cand >> 8, i = (I1[s] & ~255) + (cand & 255);
+                    if (v < V2[s] || (v == V2[s] && i < I2[s])) { V2[s] = v; I2[s] = i; }
                 }
             }
             // merge the two column groups through shared memory: group 1 hands its candidates to group 0 and
@@ -521,11 +465,11 @@ match_top2_kernel(const __grid_constant__ CUtensorMap tmap, const MatchArgs args
     if (warp == 2) tmem_dealloc(tmem_base, 512);
 }
 
-// items[i] = (pair, query block): one entry per block of rows_per_item (256; 512 for CTA pairs) rows of every pair's query frame.
+// items[i] = (pair, query block): one entry per block of kBlockQ rows of every pair's query frame.
 // Single CTA; pairs are scanned in chunks of blockDim.x.
 __global__ void build_items_kernel(const int32_t* n_kp, const int32_t* pair_q, int n_pairs,
                                    int32_t* items, int32_t* n_items, int capacity,
-                                   const int32_t* pair_flag, int want, int rows_per_item) {
+                                   const int32_t* pair_flag, int want) {
     __shared__ int warp_sums[32];
     __shared__ int base_s;
     if (threadIdx.x == 0) base_s = 0;
@@ -533,9 +477,9 @@ __global__ void build_items_kernel(const int32_t* n_kp, const int32_t* pair_q, i
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nwarps = blockDim.x >> 5;
     for (int p0 = 0; p0 < n_pairs; p0 += blockDim.x) {
         const int p = p0 + threadIdx.x;
-        // pair_flag selects the pairs of this list (V-space kernel: 0, legacy fallback: 1)
+        // pair_flag selects the pairs of this list (V-space kernel: 0, key-space fallback: 1)
         const bool take = p < n_pairs && (pair_flag == nullptr || pair_flag[p] == want);
-        const int nb = take ? (n_kp[pair_q[p]] + rows_per_item - 1) / rows_per_item : 0;
+        const int nb = take ? (n_kp[pair_q[p]] + kBlockQ - 1) / kBlockQ : 0;
         int incl = nb;
 #pragma unroll
         for (int d = 1; d < 32; d <<= 1) { const int t = __shfl_up_sync(0xffffffff, incl, d); if (lane >= d) incl += t; }
@@ -587,35 +531,23 @@ __global__ void build_items_kernel(const int32_t* n_kp, const int32_t* pair_q, i
 //
 // Measured (B200, 2048 keypoints/frame, profiles/r01e_*, r01f): 1.8 warp instructions per 32 outputs against 3.3
 // in the key-space kernel; tensor pipe active 56 % (45 % algorithmic + the fifth K block), issue slots 45 %,
-// ALU pipe 57 %.  The TMA / tcgen05 front end alone (EVZ_OPT_MATCH_DEBUG = 1: accumulators released undrained)
-// runs at 2.75 POP/s (2048 keypoints) to 3.2 POP/s (8192), the rate of the cuBLASLt int8 GEMM; the kernel runs at
-// 1.9-2.0 / 2.3, so the epilogue is the bound.  What the r01f experiments showed about it (all bit-exact):
-//   * the four predicated STS.128 of a chunk cost 22 % of the kernel whether or not any lane stores (all-false
-//     predicates: no change; stores compiled out: 1.14 -> 0.89 ms per 2 000 pairs), but skipping them with a
-//     warp-uniform vote + branch when no lane saves is 18 % SLOWER in a same-run A/B (per chunk, or after both chunks of a
-//     batch), also at 8192 keypoints where 60 % of the chunks have no saving lane;
-//   * it is not the shared-memory data pipe (the r01e reading): CTA pairs (cta_group::2, variant 7: half the TMA
-//     writes, a third less operand fetch per SM) are 5 % slower than this kernel, not faster;
-//   * it is not the accumulator hand-off either: eight warps per accumulator (column halves, merged at the end
-//     of the item; possible with the smaller rings of the pair layout) are 25 % slower with 8 epilogue warps (all
-//     of them wait for the same accumulator) and 9 % slower with 16;
-//   * 32-column loads one batch ahead (this kernel) and 16-column loads two chunks ahead (the pair template; 144 ->
-//     112 registers) are equal;
-//   * the single-CTA instance of the pair template is 4 % slower than this hand-specialised kernel (same-run A/B,
-//     although nothing that runs differs in the source), and a run-time test of the debug option in the tile loop
-//     costs another 1.4 %: the default kernel is kept as its own code, the debug modes are template instances.
-// Chunks of 32 columns, N = 128 MMAs and polling barriers from all threads measured equal or slower in r01e;
-// chunks of 8 (kVC) halve the saved bytes but add instructions: faster at 1024 keypoints, slower at 8192.
-// See DESIGN.md.
+// ALU pipe 57 %.  The TMA / tcgen05 front end alone (accumulators released undrained) runs at 2.75 POP/s (2048
+// keypoints) to 3.2 POP/s (8192), the rate of the cuBLASLt int8 GEMM; the kernel runs at 1.9-2.0 / 2.3, so the
+// epilogue is the bound, and in it the four predicated STS.128 of a chunk: they cost 22 % of the kernel whether
+// or not any lane stores (see vchunk).  Neither the shared-memory data pipe nor the accumulator hand-off is the
+// bound: CTA pairs (cta_group::2), eight or sixteen drain warps per accumulator, a two-pass drain and 16-column
+// TMEM loads all measured equal or slower (DESIGN.md K1), as did chunks of 32 columns, N = 128 MMAs and polling
+// barriers from all threads (r01e).  Chunks of 8 columns halve the saved bytes but add instructions: faster at
+// 1024 keypoints, slower at 8192.
+// The kernel is plain, non-templated code on purpose: a template instance of the same source compiled to a 4 %
+// slower kernel (same-run A/B, r01g), and a run-time option test in the tile loop cost another 1.4 %.
 constexpr int kECodeBytes = kBlockT * 32;                 // fifth K block of one train tile
 constexpr int kEMax       = 255 * (30 * 255) + 254;       // largest representable E_c
 constexpr int kFlagged    = -2;                           // top2_idx[row][0] of a row left to the fix-up kernel
 
-constexpr int kVC   = 16;                // columns per chunk of the V-space epilogue (8 or 16)
-constexpr int kVCps = kBlockT / kVC;     // chunks per tile
-constexpr int kVClog = kVC == 8 ? 5 : 4; // log2(kVCps)
-// ---- single-CTA kernel (default).  Kept as its own, non-templated code: the instance of the CTA-pair template below
-// for one CTA compiled to a 4 % slower kernel (same-run A/B, r01g), although the source differs in nothing that runs.
+constexpr int kVC    = 16;               // columns per chunk of the V-space epilogue
+constexpr int kVCps  = kBlockT / kVC;    // chunks per tile
+constexpr int kVClog = 4;                // log2(kVCps)
 struct VCfg {
     static constexpr int threads   = 384;
     static constexpr int q_off     = 0;                                // 2 x 32 KB
@@ -639,77 +571,36 @@ struct VCfg {
 // one chunk of kVC raw accumulator values: chunk key, sorted top-3 update, predicated save
 __device__ __forceinline__ void vchunk(const uint32_t* r, uint32_t tagc, uint32_t mul, uint32_t& M1, uint32_t& M2,
                                        uint32_t& M3, uint32_t& sec, uint32_t sum) {
-    uint32_t cm;
-    if (kVC == 16) {
-        const uint32_t a = __vimax3_u32(r[0], r[1], r[2]), b = __vimax3_u32(r[3], r[4], r[5]), c = __vimax3_u32(r[6], r[7], r[8]);
-        const uint32_t d = __vimax3_u32(r[9], r[10], r[11]), e = __vimax3_u32(r[12], r[13], r[14]);
-        cm = max(__vimax3_u32(a, b, c), __vimax3_u32(d, e, r[15]));
-    } else {
-        cm = __vimax3_u32(__vimax3_u32(r[0], r[1], r[2]), __vimax3_u32(r[3], r[4], r[5]), max(r[6], r[7]));
-    }
+    static_assert(kVC == 16, "four 128-bit stores per chunk");
+    const uint32_t a = __vimax3_u32(r[0], r[1], r[2]), b = __vimax3_u32(r[3], r[4], r[5]), c = __vimax3_u32(r[6], r[7], r[8]);
+    const uint32_t d = __vimax3_u32(r[9], r[10], r[11]), e = __vimax3_u32(r[12], r[13], r[14]);
+    const uint32_t cm = max(__vimax3_u32(a, b, c), __vimax3_u32(d, e, r[15]));
     uint32_t cmk;
     asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(cmk) : "r"(cm), "r"(mul), "r"(tagc));
     // the next store address goes to a different register (early clobber): overwriting `sec` in place would wait
     // for the stores to have read it (write-after-read on the short scoreboard, ~35 clk per chunk)
     const uint32_t alt = sum - sec;
     uint32_t nsec;
-    if (kVC == 16) {
-        asm volatile("{\n\t.reg .pred p1, p2;\n\t"
-                     "setp.gt.u32 p2, %2, %4;\n\t"
-                     "setp.gt.u32 p1, %2, %3;\n\t"
-                     "@p2 st.shared.v4.b32 [%1], {%6, %7, %8, %9};\n\t"
-                     "@p2 st.shared.v4.b32 [%1+%22], {%10, %11, %12, %13};\n\t"
-                     "@p2 st.shared.v4.b32 [%1+2*%22], {%14, %15, %16, %17};\n\t"
-                     "@p2 st.shared.v4.b32 [%1+3*%22], {%18, %19, %20, %21};\n\t"
-                     "selp.u32 %0, %5, %1, p1;\n\t}"
-                     : "=&r"(nsec) : "r"(sec), "r"(cmk), "r"(M1), "r"(M2), "r"(alt),
-                       "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]),
-                       "r"(r[8 % kVC]), "r"(r[9 % kVC]), "r"(r[10 % kVC]), "r"(r[11 % kVC]), "r"(r[12 % kVC]), "r"(r[13 % kVC]),
-                       "r"(r[14 % kVC]), "r"(r[15 % kVC]), "n"(VCfg::part_stride) : "memory");
-    } else {
-        asm volatile("{\n\t.reg .pred p1, p2;\n\t"
-                     "setp.gt.u32 p2, %2, %4;\n\t"
-                     "setp.gt.u32 p1, %2, %3;\n\t"
-                     "@p2 st.shared.v4.b32 [%1], {%6, %7, %8, %9};\n\t"
-                     "@p2 st.shared.v4.b32 [%1+%14], {%10, %11, %12, %13};\n\t"
-                     "selp.u32 %0, %5, %1, p1;\n\t}"
-                     : "=&r"(nsec) : "r"(sec), "r"(cmk), "r"(M1), "r"(M2), "r"(alt),
-                       "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]),
-                       "n"(VCfg::part_stride) : "memory");
-    }
+    // (a predicated-off STS.128 still costs its LSU issue slot: all-false predicates measured no faster, removing the
+    // four stores +28 %; skipping them with a warp-uniform vote + branch when no lane saves measured 18 % SLOWER)
+    asm volatile("{\n\t.reg .pred p1, p2;\n\t"
+                 "setp.gt.u32 p2, %2, %4;\n\t"
+                 "setp.gt.u32 p1, %2, %3;\n\t"
+                 "@p2 st.shared.v4.b32 [%1], {%6, %7, %8, %9};\n\t"
+                 "@p2 st.shared.v4.b32 [%1+%22], {%10, %11, %12, %13};\n\t"
+                 "@p2 st.shared.v4.b32 [%1+2*%22], {%14, %15, %16, %17};\n\t"
+                 "@p2 st.shared.v4.b32 [%1+3*%22], {%18, %19, %20, %21};\n\t"
+                 "selp.u32 %0, %5, %1, p1;\n\t}"
+                 : "=&r"(nsec) : "r"(sec), "r"(cmk), "r"(M1), "r"(M2), "r"(alt),
+                   "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]),
+                   "r"(r[8]), "r"(r[9]), "r"(r[10]), "r"(r[11]), "r"(r[12]), "r"(r[13]),
+                   "r"(r[14]), "r"(r[15]), "n"(VCfg::part_stride) : "memory");
     sec = nsec;
     const uint32_t t = min(M1, cmk), u = __vimin3_u32(M1, M2, cmk);
     M1 = max(M1, cmk);
     M3 = max(M3, u);
     M2 = max(M2, t);
 }
-
-// kCtas = 1: one CTA per work item (256 query rows).  kCtas = 2: a CTA pair (cta_group::2) shares every train
-// tile -- each CTA stages half of it (128 rows + their 4 KB of the fifth K block) and drains its own 256 query rows.
-template <int kCtas>
-struct VCfgT {
-    static constexpr int threads   = 384;
-    static constexpr int stages    = kCtas == 2 ? 5 : kStages;         // train-tile ring depth
-    static constexpr int tile_rows = kBlockT / kCtas;                  // train rows this CTA stages per tile
-    static constexpr int tile_bytes = tile_rows * kRowBytes;
-    static constexpr int ecode_bytes = tile_rows * 32;
-    static constexpr int q_off     = 0;                                // 2 x 32 KB
-    static constexpr int t_off     = q_off + 2 * kQBytes;              // stages x 32 (16) KB
-    static constexpr int e_off     = t_off + stages * tile_bytes;      // stages x 8 (4) KB
-    static constexpr int a_off     = e_off + stages * ecode_bytes;     // 4 KB: query-side fifth K block
-    static constexpr int slot_off  = a_off + 128 * 32;                 // [slot 2][part 4][row 256] x 16 B
-    static constexpr int part_stride = 256 * 16;
-    static constexpr int slot_stride = (kVC / 4) * part_stride;
-    static constexpr int pb_bytes  = (EVZ_MAX_KP / kBlockT) * 32;      // norm parity bitmap of one train frame
-    static constexpr int pb_off    = slot_off + 2 * slot_stride;       // 2 x pb_bytes, alternating per item
-    static constexpr int item_off  = pb_off + 2 * pb_bytes;
-    static constexpr int bar_off   = item_off + 2 * static_cast<int>(sizeof(Item));
-    static constexpr int n_bars    = 2 * stages + 2 + 2 + 2 + 2 + (kCtas == 2 ? stages + 2 : 0);
-    static constexpr int tmem_off  = bar_off + n_bars * 8;
-    static constexpr int total     = tmem_off + 16;
-    static constexpr int smem_bytes = total + 1024;
-    static_assert(smem_bytes <= 227 * 1024, "V-space match kernel shared memory exceeds 227 KB");
-};
 
 // K-major operand tile without swizzle: 8-row x 16-byte core matrices (128 contiguous bytes); lbo = byte
 // distance between the two core matrices along K, sbo = byte distance between 8-row groups.
@@ -720,57 +611,6 @@ __device__ __forceinline__ uint64_t umma_desc_nosw(uint32_t smem_addr_bytes, uin
     d |= static_cast<uint64_t>(sbo >> 4) << 32;
     d |= static_cast<uint64_t>(1) << 46;                                 // version = 1 (sm_100), layout = none
     return d;
-}
-
-// one chunk of kVC raw accumulator values: chunk key, sorted top-3 update, predicated save
-template <int kPartStride>
-__device__ __forceinline__ void vchunk(const uint32_t* r, uint32_t tagc, uint32_t mul, uint32_t& M1, uint32_t& M2,
-                                       uint32_t& M3, uint32_t& sec, uint32_t sum) {
-    uint32_t cm;
-    if (kVC == 16) {
-        const uint32_t a = __vimax3_u32(r[0], r[1], r[2]), b = __vimax3_u32(r[3], r[4], r[5]), c = __vimax3_u32(r[6], r[7], r[8]);
-        const uint32_t d = __vimax3_u32(r[9], r[10], r[11]), e = __vimax3_u32(r[12], r[13], r[14]);
-        cm = max(__vimax3_u32(a, b, c), __vimax3_u32(d, e, r[15]));
-    } else {
-        cm = __vimax3_u32(__vimax3_u32(r[0], r[1], r[2]), __vimax3_u32(r[3], r[4], r[5]), max(r[6], r[7]));
-    }
-    uint32_t cmk;
-    asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(cmk) : "r"(cm), "r"(mul), "r"(tagc));
-    // the next store address goes to a different register (early clobber): overwriting `sec` in place would wait
-    // for the stores to have read it (write-after-read on the short scoreboard, ~35 clk per chunk)
-    const uint32_t alt = sum - sec;
-    uint32_t nsec;
-    if (kVC == 16) {
-        // (a predicated-off STS.128 still costs its LSU issue slot: all-false predicates measured no faster, removing the
-        // four stores +28 %; skipping them with a warp-uniform vote + branch when no lane saves measured 18 % SLOWER)
-        asm volatile("{\n\t.reg .pred p1, p2;\n\t"
-                     "setp.gt.u32 p2, %2, %4;\n\t"
-                     "setp.gt.u32 p1, %2, %3;\n\t"
-                     "selp.u32 %0, %5, %1, p1;\n\t"
-                     "@p2 st.shared.v4.b32 [%1], {%6, %7, %8, %9};\n\t"
-                     "@p2 st.shared.v4.b32 [%1+%22], {%10, %11, %12, %13};\n\t"
-                     "@p2 st.shared.v4.b32 [%1+2*%22], {%14, %15, %16, %17};\n\t"
-                     "@p2 st.shared.v4.b32 [%1+3*%22], {%18, %19, %20, %21};\n\t}"
-                     : "=&r"(nsec) : "r"(sec), "r"(cmk), "r"(M1), "r"(M2), "r"(alt),
-                       "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]),
-                       "r"(r[8 % kVC]), "r"(r[9 % kVC]), "r"(r[10 % kVC]), "r"(r[11 % kVC]), "r"(r[12 % kVC]), "r"(r[13 % kVC]),
-                       "r"(r[14 % kVC]), "r"(r[15 % kVC]), "n"(kPartStride) : "memory");
-    } else {
-        asm volatile("{\n\t.reg .pred p1, p2;\n\t"
-                     "setp.gt.u32 p2, %2, %4;\n\t"
-                     "setp.gt.u32 p1, %2, %3;\n\t"
-                     "@p2 st.shared.v4.b32 [%1], {%6, %7, %8, %9};\n\t"
-                     "@p2 st.shared.v4.b32 [%1+%14], {%10, %11, %12, %13};\n\t"
-                     "selp.u32 %0, %5, %1, p1;\n\t}"
-                     : "=&r"(nsec) : "r"(sec), "r"(cmk), "r"(M1), "r"(M2), "r"(alt),
-                       "r"(r[0]), "r"(r[1]), "r"(r[2]), "r"(r[3]), "r"(r[4]), "r"(r[5]), "r"(r[6]), "r"(r[7]),
-                       "n"(kPartStride) : "memory");
-    }
-    sec = nsec;
-    const uint32_t t = min(M1, cmk), u = __vimin3_u32(M1, M2, cmk);
-    M1 = max(M1, cmk);
-    M3 = max(M3, u);
-    M2 = max(M2, t);
 }
 
 // keeps 16 registers allocated up to this point: the predicated stores of a chunk read them late, and a
@@ -803,31 +643,6 @@ __device__ __forceinline__ void drain_v(uint32_t taddr, uint32_t mul, uint32_t& 
     }
 }
 
-// timing probe (kDbg = 3): one column half (128 columns, chunk tags b0 * 2 ...) of an accumulator row
-__device__ __forceinline__ void drain_v_half(uint32_t taddr, int b0, uint32_t mul, uint32_t& M1, uint32_t& M2, uint32_t& M3,
-                                             uint32_t& sec, uint32_t sum, uint64_t* acc_empty, int lane) {
-    uint32_t r[2][32];
-    tmem_ld_32x32b_x32(taddr, r[0]);
-#pragma unroll
-    for (int b = 0; b < 4; ++b) {
-        tmem_ld_wait_dep(r[b & 1]);
-        if (b + 1 < 4) {
-            tmem_ld_32x32b_x32(taddr + (b + 1) * 32, r[(b + 1) & 1]);
-        } else {
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) mbar_arrive(acc_empty);
-        }
-#pragma unroll
-        for (int c = 0; c < 32 / kVC; ++c) vchunk(&r[b & 1][kVC * c], 254 - (32 / kVC) * (b0 + b) - c, mul, M1, M2, M3, sec, sum);
-        keep_alive16(&r[b & 1][0]);
-        keep_alive16(&r[b & 1][16]);
-    }
-}
-
-// kDbg (EVZ_OPT_MATCH_DEBUG, measurement only): 1 = accumulators released undrained, 2 = TMEM loads only; the
-// production instance is kDbg = 0 (a run-time test in the tile loop costs 1.4 %).
-template <int kDbg>
 __global__ void __launch_bounds__(VCfg::threads, 1)
 match_top2_vkernel(const __grid_constant__ CUtensorMap tmap, const MatchArgs args) {
     using Cfg = VCfg;
@@ -855,7 +670,7 @@ match_top2_vkernel(const __grid_constant__ CUtensorMap tmap, const MatchArgs arg
         for (int i = 0; i < kStages; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
         for (int i = 0; i < 2; ++i) {
             mbar_init(&q_full[i], 1); mbar_init(&q_empty[i], 1 + 8);
-            mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], kDbg == 3 ? 8 : 4);
+            mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], 4);
         }
         fence_mbar_init();
     }
@@ -956,71 +771,6 @@ match_top2_vkernel(const __grid_constant__ CUtensorMap tmap, const MatchArgs arg
                 umma_commit(&q_empty[qb]);
             }
         }
-    } else if (kDbg == 3 && warp >= 4) {
-        // ------------------------------------------------------------- timing probe: all eight drain warps work on ONE
-        // accumulator at a time (column halves), then on the other.  The two halves of a row share their save slots, so
-        // the RESULTS ARE WRONG; the instruction and shared-memory traffic are those of a kernel with per-half slots.
-        const int half = (warp - 4) >> 2;
-        const int quarter = warp & 3;
-        uint32_t g = 0, qi = 0;
-        for (int it = blockIdx.x; it < n_items; it += gridDim.x) {
-            const uint32_t qb = qi & 1, qph = (qi >> 1) & 1;
-            ++qi;
-            mbar_wait(&q_full[qb], qph);
-            const Item im = item_s[qb];
-            uint32_t M1[2] = {0, 0}, M2[2] = {0, 0}, M3[2] = {0, 0}, sec[2], sum[2];
-#pragma unroll
-            for (int sub = 0; sub < 2; ++sub) {
-                const int row = sub * 128 + quarter * 32 + lane;
-                const uint32_t slot_a = smem_u32(smem + Cfg::slot_off) + row * 16, slot_b = slot_a + Cfg::slot_stride;
-                sum[sub] = slot_a + slot_b; sec[sub] = slot_b;
-            }
-            for (int n = 0; n < im.n_tiles; ++n) {
-#pragma unroll
-                for (int sub = 0; sub < 2; ++sub) {
-                    if (sub < im.n_sub) {
-                        M1[sub] |= 255u; M2[sub] |= 255u; M3[sub] |= 255u;
-                        mbar_wait(&acc_full[sub], g & 1);
-                        tc_fence_after();
-                        const uint32_t taddr = tmem_base + sub * kBlockT + half * 128 + (static_cast<uint32_t>(quarter * 32) << 16);
-                        drain_v_half(taddr, half * 4, args.mul256, M1[sub], M2[sub], M3[sub], sec[sub], sum[sub], &acc_empty[sub], lane);
-                    }
-                }
-                ++g;
-            }
-            // end of item: the cost of the exact evaluation of two slots per tracker (values discarded)
-            int acc = 0;
-#pragma unroll
-            for (int sub = 0; sub < 2; ++sub) {
-                if (sub < im.n_sub) {
-                    int k[2 * kVC];
-#pragma unroll
-                    for (int sidx = 0; sidx < 2; ++sidx) {
-                        const uint32_t sa = sidx == 0 ? sum[sub] - sec[sub] : sec[sub];
-#pragma unroll
-                        for (int part = 0; part < kVC / 4; ++part) {
-                            const int4 v = lds128(sa + part * Cfg::part_stride);
-                            k[sidx * kVC + part * 4 + 0] = mad_key(v.x, args.neg512, part);
-                            k[sidx * kVC + part * 4 + 1] = mad_key(v.y, args.neg512, part + 1);
-                            k[sidx * kVC + part * 4 + 2] = mad_key(v.z, args.neg512, part + 2);
-                            k[sidx * kVC + part * 4 + 3] = mad_key(v.w, args.neg512, part + 3);
-                        }
-                    }
-                    int m1 = INT_MAX, m2 = INT_MAX;
-#pragma unroll
-                    for (int i = 0; i < kVC; ++i) top2_pair(k[2 * i], k[2 * i + 1], m1, m2);
-                    acc += m1 ^ m2 ^ static_cast<int>(M3[sub]);
-                }
-            }
-            const int row0 = quarter * 32 + lane;
-            if (half == 0 && row0 < im.nq_left) {
-                const int64_t o_row = static_cast<int64_t>(im.out_row0) + row0;
-                reinterpret_cast<int2*>(args.top2_idx)[o_row] = make_int2(acc, -1);
-                reinterpret_cast<int2*>(args.top2_d2)[o_row] = make_int2(acc, -1);
-            }
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&q_empty[qb]);
-        }
     } else if (warp >= 4) {
         // ------------------------------------------------------------- epilogue
         const int grp = (warp - 4) >> 2;                       // query sub-tile = accumulator
@@ -1047,24 +797,6 @@ match_top2_vkernel(const __grid_constant__ CUtensorMap tmap, const MatchArgs arg
                     const uint32_t o1 = M1, o2 = M2;
                     mbar_wait(&acc_full[grp], g & 1);
                     tc_fence_after();
-                    if constexpr (kDbg != 0) {
-                        if (kDbg == 2) {                  // every column loaded and waited for, no arithmetic, no saves
-                            uint32_t r[2][32];
-                            tmem_ld_32x32b_x32(taddr, r[0]);
-#pragma unroll
-                            for (int b = 0; b < 8; ++b) {
-                                tmem_ld_wait_dep(r[b & 1]);
-                                if (b + 1 < 8) tmem_ld_32x32b_x32(taddr + (b + 1) * 32, r[(b + 1) & 1]);
-                                keep_alive16(&r[b & 1][0]);
-                                keep_alive16(&r[b & 1][16]);
-                            }
-                        }
-                        tc_fence_before();
-                        __syncwarp();
-                        if (lane == 0) mbar_arrive(&acc_empty[grp]);
-                        ++g;
-                        continue;
-                    }
                     drain_v(taddr, args.mul256, M1, M2, M3, sec, sum, &acc_empty[grp], lane);
                     ++g;
                     const int nTb = M1 == o1 ? Tb : n * kVCps + 254 - static_cast<int>(M1 & 255u);
@@ -1086,8 +818,7 @@ match_top2_vkernel(const __grid_constant__ CUtensorMap tmap, const MatchArgs arg
                         const int base = (T >> kVClog) * kBlockT + (T & (kVCps - 1)) * kVC;
                         const int cs = (2 * hm1) * 256 + ((s == 0) == best_first ? 0 : kVC);
                         uint32_t ps;                       // norm parity of the chunk's columns, moved to bits 8..
-                        if (kVC == 16) asm volatile("ld.shared.u16 %0, [%1];" : "=r"(ps) : "r"(smem_u32(smem + Cfg::pb_off) + qb * Cfg::pb_bytes + (base >> 3)));
-                        else           asm volatile("ld.shared.u8 %0, [%1];" : "=r"(ps) : "r"(smem_u32(smem + Cfg::pb_off) + qb * Cfg::pb_bytes + (base >> 3)));
+                        asm volatile("ld.shared.u16 %0, [%1];" : "=r"(ps) : "r"(smem_u32(smem + Cfg::pb_off) + qb * Cfg::pb_bytes + (base >> 3)));
                         ps <<= 8;
 #pragma unroll
                         for (int part = 0; part < kVC / 4; ++part) {
@@ -1137,959 +868,6 @@ match_top2_vkernel(const __grid_constant__ CUtensorMap tmap, const MatchArgs arg
     tc_fence_before();
     __syncthreads();
     if (warp == 2) tmem_dealloc(tmem_base, 512);
-}
-
-
-// =====================================================================================================
-// Two-pass V-space kernel (match_top2_wkernel, EVZ_OPT_MATCH_VARIANT = 8; a measured NEGATIVE result of round 2: bit-identical,
-// a quarter of the shared-memory store cycles, and 2.4 x slower than match_top2_vkernel -- pass B is a serial chain of ~15
-// ballot / TMEM load / store steps per tile and warp, ~55 instructions each, with nothing to hide its latencies behind;
-// pass A alone already takes as long as the whole one-pass drain because the accumulator is held until the end).
-// Same TMA / tcgen05 front end, same
-// V = q.t + E_c accumulators, same exact end-of-item resolution and certification as match_top2_vkernel; what
-// changes is how the two best chunks of a row reach shared memory.
-//
-// What bounds match_top2_vkernel (round-2 microbenchmarks, scripts/microbench/mb2.cu): a STS.128 occupies the
-// shared-memory store path for ~4.4 clk per SM as soon as ONE lane is active (1 clk when none is), so the four
-// predicated stores of a chunk cost ~17 clk whenever any of the warp's 32 rows saves -- which, with 32 independent
-// rows per warp, is 62 % of all chunks at 2 048 keypoints: ~1 560 clk of store path per 256-row tile against the
-// 1 500 clk the ten tcgen05.mma of a tile take.  With short descriptors (one K block instead of four) the kernel is
-// only 6 % faster: the drain, i.e. the store path, is the bound.
-//
-// Here the drain of an accumulator row is two passes over tensor memory (reading TMEM is cheap: a drain that only
-// loads runs at the front-end rate):
-//   pass A  (shape 32x32b, thread = row) every 16-column chunk -> its maximum -> chunk key -> sorted top-3 of chunk
-//           keys, exactly as before, but NOTHING is stored and no slot bookkeeping is done per chunk;
-//   after the tile's 16 chunks a row knows which of them (at most two) now belong to its two best chunks;
-//   pass B  only those chunks are read again, with shape 16x256b.x2, in which a QUAD of threads holds one row's 16
-//           columns (4 each): one STS.128 per thread saves the chunk, and one store instruction serves 8 rows.
-//           The (chunk, half-warp) pairs with a saving row come from one redux.or; who saves and into which slot
-//           travels by two ballots.  A chunk that only one row wants costs ~5.5 clk of store path instead of ~17,
-//           chunks nobody wants cost nothing, and the tile's transient records (chunks that were among the row's
-//           best two for a while but not at the end of the tile) are never stored.
-// Slot layout: [slot 2][row 256][part 4] x 16 B; part q of a slot holds columns 2q, 2q+1, 8+2q, 8+2q+1 of the chunk.
-__device__ __forceinline__ void wchunk_key(const uint32_t* r, uint32_t tagc, uint32_t mul, uint32_t& M1, uint32_t& M2, uint32_t& M3) {
-    const uint32_t a = __vimax3_u32(r[0], r[1], r[2]), b = __vimax3_u32(r[3], r[4], r[5]), c = __vimax3_u32(r[6], r[7], r[8]);
-    const uint32_t d = __vimax3_u32(r[9], r[10], r[11]), e = __vimax3_u32(r[12], r[13], r[14]);
-    const uint32_t cm = max(__vimax3_u32(a, b, c), __vimax3_u32(d, e, r[15]));
-    uint32_t cmk;
-    asm("mad.lo.u32 %0, %1, %2, %3;" : "=r"(cmk) : "r"(cm), "r"(mul), "r"(tagc));
-    const uint32_t t = min(M1, cmk), u = __vimin3_u32(M1, M2, cmk);
-    M1 = max(M1, cmk);
-    M3 = max(M3, u);
-    M2 = max(M2, t);
-}
-
-__global__ void __launch_bounds__(VCfg::threads, 1)
-match_top2_wkernel(const __grid_constant__ CUtensorMap tmap, const MatchArgs args) {
-    using Cfg = VCfg;
-    static_assert(kVC == 16, "the two-pass kernel saves 16-column chunks");
-    extern __shared__ uint8_t smem_raw[];
-    uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-    uint8_t* q_s = smem + Cfg::q_off;
-    uint8_t* t_s = smem + Cfg::t_off;
-    uint8_t* e_s = smem + Cfg::e_off;
-    uint8_t* a_s = smem + Cfg::a_off;
-    Item* item_s = reinterpret_cast<Item*>(smem + Cfg::item_off);
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + Cfg::bar_off);
-    uint64_t* full = bars;                       // [kStages] train tile + its fifth K block landed (TMA tx)
-    uint64_t* empty = full + kStages;            // [kStages] MMA commit
-    uint64_t* q_full = empty + kStages;          // [2] query block landed + item descriptor published
-    uint64_t* q_empty = q_full + 2;              // [2] MMA commit + 8 epilogue warps
-    uint64_t* acc_full = q_empty + 2;            // [2] accumulator (= query sub-tile) ready (MMA commit)
-    uint64_t* acc_empty = acc_full + 2;          // [2] accumulator drained (4 epilogue warps each)
-    uint32_t* tmem_ptr_s = reinterpret_cast<uint32_t*>(smem + Cfg::tmem_off);
-
-    const int warp = threadIdx.x >> 5;
-    const int lane = threadIdx.x & 31;
-
-    if (warp == 0 && lane == 0) {
-        tma_prefetch_desc(&tmap);
-        for (int i = 0; i < kStages; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
-        for (int i = 0; i < 2; ++i) {
-            mbar_init(&q_full[i], 1); mbar_init(&q_empty[i], 1 + 8);
-            mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], 4);
-        }
-        fence_mbar_init();
-    }
-    if (warp == 2) {
-        tmem_alloc(tmem_ptr_s, 512);
-        tmem_relinquish();
-    }
-    if (warp == 3) {
-        // query-side fifth K block: every row = (255 x 30, 1, 0), no-swizzle core-matrix layout
-        for (int i = lane; i < 256; i += 32) {
-            const bool second = (i >> 3) & 1;          // [group 16][k half 2][row 8] x 16 B
-            reinterpret_cast<uint4*>(a_s)[i] = make_uint4(0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu, second ? 0x0001FFFFu : 0xFFFFFFFFu);
-        }
-        fence_proxy_async();
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_ptr_s;
-    const int n_items = *args.n_items;
-
-    if (warp == 0) {
-        // ------------------------------------------------------------- TMA producer (polling waits, single thread)
-        if (lane == 0) {
-            uint32_t stage = 0, sphase = 0, qi = 0;
-            for (int it = blockIdx.x; it < n_items; it += gridDim.x) {
-                const Item im = load_item(args, it);
-                const uint32_t qb = qi & 1, qph = (qi >> 1) & 1;
-                ++qi;
-                mbar_wait_spin(&q_empty[qb], qph ^ 1);
-                item_s[qb] = im;
-                if (im.n_tiles == 0) { mbar_arrive(&q_full[qb]); continue; }
-                mbar_arrive_expect_tx(&q_full[qb], kQBytes + im.n_tiles * 32);
-                tma_load_2d(q_s + qb * kQBytes, &tmap, 0, im.q_row0, &q_full[qb]);
-                bulk_load_1d(smem + Cfg::pb_off + qb * Cfg::pb_bytes, args.pbits + static_cast<size_t>(im.t_row0 >> 8) * 8,
-                             im.n_tiles * 32, &q_full[qb]);
-                const uint8_t* ecode = args.ecode + static_cast<size_t>(im.t_row0 >> 8) * kECodeBytes;
-                for (int n = 0; n < im.n_tiles; ++n) {
-                    if (n + kStages < im.n_tiles) {
-                        tma_prefetch_2d(&tmap, 0, im.t_row0 + (n + kStages) * kBlockT);
-                        bulk_prefetch_1d(ecode + static_cast<size_t>(n + kStages) * kECodeBytes, kECodeBytes);
-                    }
-                    mbar_wait_spin(&empty[stage], sphase ^ 1);
-                    mbar_arrive_expect_tx(&full[stage], kTileBytes + kECodeBytes);
-                    tma_load_2d(t_s + stage * kTileBytes, &tmap, 0, im.t_row0 + n * kBlockT, &full[stage]);
-                    bulk_load_1d(e_s + stage * kECodeBytes, ecode + static_cast<size_t>(n) * kECodeBytes, kECodeBytes, &full[stage]);
-                    if (++stage == kStages) { stage = 0; sphase ^= 1; }
-                }
-            }
-        }
-    } else if (warp == 1) {
-        // ------------------------------------------------------------- MMA issuer (see match_top2_vkernel)
-        if (lane == 0) {
-            constexpr uint32_t idesc = umma_idesc_u8(128, kBlockT);
-            const uint64_t da_e = umma_desc_nosw(smem_u32(a_s), 128, 256);
-            const int n_kb = args.n_kb;
-            uint32_t stage = 0, sphase = 0, qi = 0, gs[2] = {0, 0};
-            for (int it = blockIdx.x; it < n_items; it += gridDim.x) {
-                const uint32_t qb = qi & 1, qph = (qi >> 1) & 1;
-                ++qi;
-                mbar_wait_spin(&q_full[qb], qph);
-                const int n_tiles = item_s[qb].n_tiles, n_sub = item_s[qb].n_sub;
-                const uint32_t q_addr = smem_u32(q_s + qb * kQBytes);
-                for (int n = 0; n < n_tiles; ++n) {
-                    mbar_wait_spin(&full[stage], sphase);
-                    const uint32_t t_addr = smem_u32(t_s + stage * kTileBytes);
-                    const uint64_t db_e = umma_desc_nosw(smem_u32(e_s + stage * kECodeBytes), 128, 256);
-                    for (int sub = 0; sub < n_sub; ++sub) {
-                        const uint32_t aph = gs[sub]++ & 1;
-                        mbar_wait_spin(&acc_empty[sub], aph ^ 1);
-                        tc_fence_after();
-                        if (n_kb == kRowBytes / 32) {
-#pragma unroll
-                            for (int k = 0; k < kRowBytes / 32; ++k) {
-                                const uint64_t da = umma_desc_sw128(q_addr + sub * (128 * kRowBytes) + k * 32);
-                                const uint64_t db = umma_desc_sw128(t_addr + k * 32);
-                                umma_i8(tmem_base + sub * kBlockT, da, db, idesc, k > 0 ? 1u : 0u);
-                            }
-                        } else {
-                            for (int k = 0; k < n_kb; ++k) {
-                                const uint64_t da = umma_desc_sw128(q_addr + sub * (128 * kRowBytes) + k * 32);
-                                const uint64_t db = umma_desc_sw128(t_addr + k * 32);
-                                umma_i8(tmem_base + sub * kBlockT, da, db, idesc, k > 0 ? 1u : 0u);
-                            }
-                        }
-                        umma_i8(tmem_base + sub * kBlockT, da_e, db_e, idesc, 1u);
-                        umma_commit(&acc_full[sub]);
-                    }
-                    umma_commit(&empty[stage]);
-                    if (++stage == kStages) { stage = 0; sphase ^= 1; }
-                }
-                umma_commit(&q_empty[qb]);
-            }
-        }
-    } else if (warp >= 4) {
-        // ------------------------------------------------------------- epilogue
-        const int grp = (warp - 4) >> 2;                       // query sub-tile = accumulator
-        const int quarter = warp & 3;                          // TMEM lane quarter this warp may read
-        const int row = grp * 128 + quarter * 32 + lane;       // query row within the block
-        const uint32_t slot_base = smem_u32(smem + Cfg::slot_off);
-        const uint32_t taddr = tmem_base + grp * kBlockT + (static_cast<uint32_t>(quarter * 32) << 16);
-        // pass B: this thread's quad position and the two rows (of either half-warp) it stores for
-        const int q4 = lane & 3, r8 = lane >> 2, hl = lane >> 4;
-        const uint32_t quad_base = slot_base + static_cast<uint32_t>(grp * 128 + quarter * 32 + r8) * 64 + q4 * 16;
-        uint32_t g = 0, qi = 0;
-        for (int it = blockIdx.x; it < n_items; it += gridDim.x) {
-            const uint32_t qb = qi & 1, qph = (qi >> 1) & 1;
-            ++qi;
-            mbar_wait(&q_full[qb], qph);
-            const Item im = item_s[qb];
-            if (grp < im.n_sub) {
-                const int qkey = __ldg(args.ckey + im.q_row0 + row);
-                // sorted top-3 of chunk keys, the physical slot (0 / 1) that holds the second-best chunk, and the position
-                // (tile * 16 + chunk) of the chunks in the best / second-best slot
-                uint32_t M1 = 0, M2 = 0, M3 = 0, secbit = 1;
-                int Tb = -1, Ts = -1;
-                for (int n = 0; n < im.n_tiles; ++n) {
-                    // keys of earlier tiles beat every key of this tile with the same V (lowest index wins)
-                    M1 |= 255u; M2 |= 255u; M3 |= 255u;
-                    mbar_wait(&acc_full[grp], g & 1);
-                    tc_fence_after();
-                    // ---- pass A: chunk maxima and top-3 of chunk keys, nothing stored
-                    {
-                        uint32_t r[2][32];
-                        tmem_ld_32x32b_x32(taddr, r[0]);
-#pragma unroll
-                        for (int b = 0; b < 8; ++b) {
-                            tmem_ld_wait_dep(r[b & 1]);
-                            if (b + 1 < 8) tmem_ld_32x32b_x32(taddr + (b + 1) * 32, r[(b + 1) & 1]);
-                            wchunk_key(&r[b & 1][0], 254 - 2 * b, args.mul256, M1, M2, M3);
-                            wchunk_key(&r[b & 1][16], 253 - 2 * b, args.mul256, M1, M2, M3);
-                        }
-                    }
-                    // ---- which chunks of this tile are now the row's best / second-best chunk
-                    const bool nb = (M1 & 255u) != 255u, ns = (M2 & 255u) != 255u;
-                    const int jA = nb ? 254 - static_cast<int>(M1 & 255u) : -1, jB = ns ? 254 - static_cast<int>(M2 & 255u) : -1;
-                    const uint32_t tgtA = secbit;                 // a new best chunk replaces the old second-best one ...
-                    if (nb) secbit ^= 1u;                         // ... and the old best chunk becomes the second-best
-                    const uint32_t tgtB = secbit;
-                    Ts = ns ? n * kVCps + jB : (nb ? Tb : Ts);
-                    Tb = nb ? n * kVCps + jA : Tb;
-                    // ---- pass B: (chunk, half-warp) pairs with a saving row
-                    uint32_t U2 = redux_or((nb ? 1u << (2 * jA + hl) : 0u) | (ns ? 1u << (2 * jB + hl) : 0u));
-                    if (args.dbg == 3) U2 = 0;                      // measurement only: pass A alone (results are garbage)
-                    uint32_t s0[8], s1[8];
-                    int bit = U2 ? __ffs(U2) - 1 : -1;
-                    if (bit >= 0) tmem_ld_16x256b_x2(taddr + (bit >> 1) * kVC + (static_cast<uint32_t>((bit & 1) * 16) << 16), s0);
-                    auto save = [&](uint32_t (&cur)[8], uint32_t (&nxt)[8]) {
-                        U2 &= U2 - 1;
-                        const int nbit = U2 ? __ffs(U2) - 1 : -1;
-                        const int j = bit >> 1, h = bit & 1;
-                        const unsigned W = __ballot_sync(0xffffffffu, jA == j || jB == j);
-                        const unsigned Sb = __ballot_sync(0xffffffffu, (jA == j ? tgtA : tgtB) != 0u);
-                        tmem_ld_wait_dep(cur);
-                        if (nbit >= 0) tmem_ld_16x256b_x2(taddr + (nbit >> 1) * kVC + (static_cast<uint32_t>((nbit & 1) * 16) << 16), nxt);
-                        const int ra = 16 * h + r8, rb = ra + 8;
-                        const uint32_t aa = quad_base + (16 * h) * 64 + ((Sb >> ra) & 1u) * Cfg::slot_stride;
-                        const uint32_t ab = quad_base + (16 * h + 8) * 64 + ((Sb >> rb) & 1u) * Cfg::slot_stride;
-                        asm volatile("{\n\t.reg .pred pa, pb;\n\t"
-                                     "setp.ne.u32 pa, %10, 0;\n\t"
-                                     "setp.ne.u32 pb, %11, 0;\n\t"
-                                     "@pa st.shared.v4.b32 [%0], {%2, %3, %6, %7};\n\t"
-                                     "@pb st.shared.v4.b32 [%1], {%4, %5, %8, %9};\n\t}"
-                                     :: "r"(aa), "r"(ab), "r"(cur[0]), "r"(cur[1]), "r"(cur[2]), "r"(cur[3]), "r"(cur[4]), "r"(cur[5]),
-                                        "r"(cur[6]), "r"(cur[7]), "r"((W >> ra) & 1u), "r"((W >> rb) & 1u) : "memory");
-                        bit = nbit;
-                    };
-                    while (bit >= 0) {
-                        save(s0, s1);
-                        if (bit < 0) break;
-                        save(s1, s0);
-                    }
-                    tc_fence_before();
-                    __syncwarp();
-                    if (lane == 0) mbar_arrive(&acc_empty[grp]);
-                    ++g;
-                }
-                // the saves of other lanes of this warp (pass B stores for 8 rows at a time) must be visible to the row's owner
-                __syncwarp();
-                // exact evaluation of the two saved chunks (see match_top2_vkernel); word i = 4 q + e of a slot is column
-                // 2q + (e & 1) + 8 (e >> 1) of the chunk
-                const int hm1 = im.pad + 1;
-                const bool best_first = Ts < 0 || Tb < Ts;
-                int k[2 * kVC];
-#pragma unroll
-                for (int s = 0; s < 2; ++s) {
-                    const int T = s == 0 ? Tb : Ts;
-                    const uint32_t sa = slot_base + (s == 0 ? (secbit ^ 1u) : secbit) * Cfg::slot_stride + row * 64;
-                    if (T >= 0) {
-                        const int base = (T >> kVClog) * kBlockT + (T & (kVCps - 1)) * kVC;
-                        const int cs = (2 * hm1) * 256 + ((s == 0) == best_first ? 0 : kVC);
-                        uint32_t ps;                       // norm parity of the chunk's columns, moved to bits 8..
-                        asm volatile("ld.shared.u16 %0, [%1];" : "=r"(ps) : "r"(smem_u32(smem + Cfg::pb_off) + qb * Cfg::pb_bytes + (base >> 3)));
-                        ps <<= 8;
-#pragma unroll
-                        for (int part = 0; part < 4; ++part) {
-                            const int4 v = lds128(sa + part * 16);
-                            const int c0 = 2 * part, c1 = 2 * part + 1, c2 = 8 + 2 * part, c3 = 9 + 2 * part;
-                            k[s * kVC + part * 4 + 0] = mad_key(v.x, args.neg512, cs) + (((ps >> c0) & 256) + c0);
-                            k[s * kVC + part * 4 + 1] = mad_key(v.y, args.neg512, cs) + (((ps >> c1) & 256) + c1);
-                            k[s * kVC + part * 4 + 2] = mad_key(v.z, args.neg512, cs) + (((ps >> c2) & 256) + c2);
-                            k[s * kVC + part * 4 + 3] = mad_key(v.w, args.neg512, cs) + (((ps >> c3) & 256) + c3);
-                        }
-                    } else {
-#pragma unroll
-                        for (int i = 0; i < kVC; ++i) k[s * kVC + i] = INT_MAX;
-                    }
-                }
-                int m1 = INT_MAX, m2 = INT_MAX;
-#pragma unroll
-                for (int i = 0; i < kVC; ++i) top2_pair(k[2 * i], k[2 * i + 1], m1, m2);
-                const int base_b = Tb >= 0 ? (Tb >> kVClog) * kBlockT + (Tb & (kVCps - 1)) * kVC : 0;
-                const int base_s = Ts >= 0 ? (Ts >> kVClog) * kBlockT + (Ts & (kVCps - 1)) * kVC : 0;
-                const int base_lo = best_first ? base_b : base_s, base_hi = best_first ? base_s : base_b;
-                const int c1 = ((m1 & kVC) ? base_hi : base_lo) + (m1 & (kVC - 1)), c2 = ((m2 & kVC) ? base_hi : base_lo) + (m2 & (kVC - 1));
-                const int I1 = (m1 != INT_MAX && c1 < im.nt) ? c1 : -1, I2 = (m2 != INT_MAX && c2 < im.nt) ? c2 : -1;
-                const int V1 = m1 >> 8, V2 = m2 >> 8;
-                // every column outside the two slots has V <= V3, i.e. ||t||^2 - 2 q.t >= 2 (hmax + 1 - V3)
-                const bool third = M3 > 255u;
-                const int bound = 2 * (hm1 - static_cast<int>(M3 >> 8));
-                const bool flagged = third && (I2 < 0 || V2 >= bound);
-                if (row < im.nq_left) {
-                    const int qn = qkey >> 8;
-                    const int64_t o_row = static_cast<int64_t>(im.out_row0) + row;
-                    int2 oi, od;
-                    oi.x = flagged ? kFlagged : I1; od.x = I1 >= 0 ? V1 + qn : -1;
-                    oi.y = I2;                      od.y = I2 >= 0 ? V2 + qn : -1;
-                    reinterpret_cast<int2*>(args.top2_idx)[o_row] = oi;
-                    reinterpret_cast<int2*>(args.top2_d2)[o_row] = od;
-                    if (flagged) {
-                        const int pos = atomicAdd(args.fix_count, 1);
-                        if (pos < args.fix_capacity) args.fix_list[pos] = it * 256 + row;
-                    }
-                }
-                // the slots are rewritten by the next item's pass B (any lane of the warp): every row must have read its own first
-                __syncwarp();
-            }
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&q_empty[qb]);
-        }
-    }
-
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 2) tmem_dealloc(tmem_base, 512);
-}
-
-
-// =====================================================================================================
-// Sixteen-warp V-space kernel (match_top2_xkernel, EVZ_OPT_MATCH_VARIANT = 9; a measured NEGATIVE result of round 2:
-// bit-identical, 19 % slower than match_top2_vkernel at 2 048 keypoints and 14 % at 8 192; the two-stage ring alone costs
-// the front end 15 % (0.80 vs 0.70 ms per 2 000 pairs), and with setmaxnreg (EVZ_X_SETMAXNREG: 40 / 112 registers) the
-// kernel hung on B200 -- it runs at the 96 registers of its launch bounds).  Same algorithm as match_top2_vkernel;
-// every accumulator is drained by EIGHT warps instead of four: warp = (accumulator, column half, TMEM lane quarter),
-// thread = one query row x 128 of the 256 columns of a tile.  Why: a warp reads tensor memory at ~61 B/clk
-// (profiles/r01b_tmem_read_microbench.txt: 244 B/clk/SM with 4 warps, ~390 with 8), so four warps need >= 540 clk to pull
-// a 128 KB accumulator through their registers -- with the max tree interleaved one batch behind the loads the drain
-// takes ~900 clk against the 750 clk the five tcgen05.mma of the other accumulator take, and nothing else in the SM
-// hides it (one drain warp per scheduler and accumulator).  Eight warps halve that and give every scheduler two
-// independent drains of the same accumulator.
-// The price is shared memory: each (row, column half) keeps its own two save slots (64 KB instead of 32), paid for with
-// a two-stage train-tile ring (a stage is released 1 500 clk before it is needed again; the TMA round trip is shorter).
-// At the end of an item both halves resolve their own exact top-2 (each certified against its own third chunk
-// maximum) and half 1 hands its result to half 0 through shared memory (named barrier per lane quarter), which
-// merges the four candidates and writes the row.  Registers: 640 threads leave 96 per thread at launch; the four
-// control warps give theirs back (setmaxnreg.dec 40) and the sixteen drain warps take 112.
-struct XCfg {
-    static constexpr int threads   = 128 + 512;
-    static constexpr int stages    = 2;
-    static constexpr int q_off     = 0;                                       // 2 x 32 KB
-    static constexpr int t_off     = q_off + 2 * kQBytes;                     // stages x 32 KB
-    static constexpr int e_off     = t_off + stages * kTileBytes;             // stages x 8 KB
-    static constexpr int a_off     = e_off + stages * kECodeBytes;            // 4 KB
-    static constexpr int slot_off  = a_off + 128 * 32;                        // [half 2][slot 2][part 4][row 256] x 16 B
-    static constexpr int part_stride = 256 * 16;
-    static constexpr int slot_stride = 4 * part_stride;
-    static constexpr int half_stride = 2 * slot_stride;
-    static constexpr int pb_bytes  = (EVZ_MAX_KP / kBlockT) * 32;
-    static constexpr int pb_off    = slot_off + 2 * half_stride;              // 2 x pb_bytes
-    static constexpr int merge_off = pb_off + 2 * pb_bytes;                   // 2 x [row 256] x (int4 + flag)
-    static constexpr int merge_bytes = 256 * 20;
-    static constexpr int item_off  = merge_off + 2 * merge_bytes;
-    static constexpr int bar_off   = item_off + 2 * static_cast<int>(sizeof(Item));
-    static constexpr int n_bars    = 2 * stages + 2 + 2 + 2 + 2;
-    static constexpr int tmem_off  = bar_off + n_bars * 8;
-    static constexpr int total     = tmem_off + 16;
-    static constexpr int smem_bytes = total + 1024;
-    static_assert(smem_bytes <= 227 * 1024, "sixteen-warp match kernel shared memory exceeds 227 KB");
-};
-
-__global__ void __launch_bounds__(XCfg::threads, 1)
-match_top2_xkernel(const __grid_constant__ CUtensorMap tmap, const MatchArgs args) {
-    using Cfg = XCfg;
-    constexpr int kSt = Cfg::stages;
-    static_assert(kVC == 16, "one TMEM load per chunk");
-    extern __shared__ uint8_t smem_raw[];
-    uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-    uint8_t* q_s = smem + Cfg::q_off;
-    uint8_t* t_s = smem + Cfg::t_off;
-    uint8_t* e_s = smem + Cfg::e_off;
-    uint8_t* a_s = smem + Cfg::a_off;
-    Item* item_s = reinterpret_cast<Item*>(smem + Cfg::item_off);
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + Cfg::bar_off);
-    uint64_t* full = bars;                       // [kSt] train tile + its fifth K block landed (TMA tx)
-    uint64_t* empty = full + kSt;                // [kSt] MMA commit
-    uint64_t* q_full = empty + kSt;              // [2] query block landed + item descriptor published
-    uint64_t* q_empty = q_full + 2;              // [2] MMA commit + 16 epilogue warps
-    uint64_t* acc_full = q_empty + 2;            // [2] accumulator (= query sub-tile) ready (MMA commit)
-    uint64_t* acc_empty = acc_full + 2;          // [2] accumulator drained (its 8 epilogue warps)
-    uint32_t* tmem_ptr_s = reinterpret_cast<uint32_t*>(smem + Cfg::tmem_off);
-
-    const int warp = threadIdx.x >> 5;
-    const int lane = threadIdx.x & 31;
-
-    if (warp == 0 && lane == 0) {
-        tma_prefetch_desc(&tmap);
-        for (int i = 0; i < kSt; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
-        for (int i = 0; i < 2; ++i) {
-            mbar_init(&q_full[i], 1); mbar_init(&q_empty[i], 1 + 16);
-            mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], 8);
-        }
-        fence_mbar_init();
-    }
-    if (warp == 2) {
-        tmem_alloc(tmem_ptr_s, 512);
-        tmem_relinquish();
-    }
-    if (warp == 3) {
-        for (int i = lane; i < 256; i += 32) {
-            const bool second = (i >> 3) & 1;          // [group 16][k half 2][row 8] x 16 B
-            reinterpret_cast<uint4*>(a_s)[i] = make_uint4(0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu, second ? 0x0001FFFFu : 0xFFFFFFFFu);
-        }
-        fence_proxy_async();
-    }
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_ptr_s;
-    const int n_items = *args.n_items;
-
-    if (warp < 4) {
-#ifdef EVZ_X_SETMAXNREG
-        setmaxnreg_dec<40>();
-#endif
-        if (warp == 0) {
-            // ------------------------------------------------------------- TMA producer (polling waits, single thread)
-            if (lane == 0) {
-                uint32_t stage = 0, sphase = 0, qi = 0;
-                for (int it = blockIdx.x; it < n_items; it += gridDim.x) {
-                    const Item im = load_item(args, it);
-                    const uint32_t qb = qi & 1, qph = (qi >> 1) & 1;
-                    ++qi;
-                    mbar_wait_spin(&q_empty[qb], qph ^ 1);
-                    item_s[qb] = im;
-                    if (im.n_tiles == 0) { mbar_arrive(&q_full[qb]); continue; }
-                    mbar_arrive_expect_tx(&q_full[qb], kQBytes + im.n_tiles * 32);
-                    tma_load_2d(q_s + qb * kQBytes, &tmap, 0, im.q_row0, &q_full[qb]);
-                    bulk_load_1d(smem + Cfg::pb_off + qb * Cfg::pb_bytes, args.pbits + static_cast<size_t>(im.t_row0 >> 8) * 8,
-                                 im.n_tiles * 32, &q_full[qb]);
-                    const uint8_t* ecode = args.ecode + static_cast<size_t>(im.t_row0 >> 8) * kECodeBytes;
-                    for (int n = 0; n < im.n_tiles; ++n) {
-                        if (n + kSt < im.n_tiles) {
-                            tma_prefetch_2d(&tmap, 0, im.t_row0 + (n + kSt) * kBlockT);
-                            bulk_prefetch_1d(ecode + static_cast<size_t>(n + kSt) * kECodeBytes, kECodeBytes);
-                        }
-                        mbar_wait_spin(&empty[stage], sphase ^ 1);
-                        mbar_arrive_expect_tx(&full[stage], kTileBytes + kECodeBytes);
-                        tma_load_2d(t_s + stage * kTileBytes, &tmap, 0, im.t_row0 + n * kBlockT, &full[stage]);
-                        bulk_load_1d(e_s + stage * kECodeBytes, ecode + static_cast<size_t>(n) * kECodeBytes, kECodeBytes, &full[stage]);
-                        if (++stage == kSt) { stage = 0; sphase ^= 1; }
-                    }
-                }
-            }
-        } else if (warp == 1) {
-            // ------------------------------------------------------------- MMA issuer (see match_top2_vkernel)
-            if (lane == 0) {
-                constexpr uint32_t idesc = umma_idesc_u8(128, kBlockT);
-                const uint64_t da_e = umma_desc_nosw(smem_u32(a_s), 128, 256);
-                const int n_kb = args.n_kb;
-                uint32_t stage = 0, sphase = 0, qi = 0, gs[2] = {0, 0};
-                for (int it = blockIdx.x; it < n_items; it += gridDim.x) {
-                    const uint32_t qb = qi & 1, qph = (qi >> 1) & 1;
-                    ++qi;
-                    mbar_wait_spin(&q_full[qb], qph);
-                    const int n_tiles = item_s[qb].n_tiles, n_sub = item_s[qb].n_sub;
-                    const uint32_t q_addr = smem_u32(q_s + qb * kQBytes);
-                    for (int n = 0; n < n_tiles; ++n) {
-                        mbar_wait_spin(&full[stage], sphase);
-                        const uint32_t t_addr = smem_u32(t_s + stage * kTileBytes);
-                        const uint64_t db_e = umma_desc_nosw(smem_u32(e_s + stage * kECodeBytes), 128, 256);
-                        for (int sub = 0; sub < n_sub; ++sub) {
-                            const uint32_t aph = gs[sub]++ & 1;
-                            mbar_wait_spin(&acc_empty[sub], aph ^ 1);
-                            tc_fence_after();
-                            if (n_kb == kRowBytes / 32) {
-#pragma unroll
-                                for (int k = 0; k < kRowBytes / 32; ++k) {
-                                    const uint64_t da = umma_desc_sw128(q_addr + sub * (128 * kRowBytes) + k * 32);
-                                    const uint64_t db = umma_desc_sw128(t_addr + k * 32);
-                                    umma_i8(tmem_base + sub * kBlockT, da, db, idesc, k > 0 ? 1u : 0u);
-                                }
-                            } else {
-                                for (int k = 0; k < n_kb; ++k) {
-                                    const uint64_t da = umma_desc_sw128(q_addr + sub * (128 * kRowBytes) + k * 32);
-                                    const uint64_t db = umma_desc_sw128(t_addr + k * 32);
-                                    umma_i8(tmem_base + sub * kBlockT, da, db, idesc, k > 0 ? 1u : 0u);
-                                }
-                            }
-                            umma_i8(tmem_base + sub * kBlockT, da_e, db_e, idesc, 1u);
-                            umma_commit(&acc_full[sub]);
-                        }
-                        umma_commit(&empty[stage]);
-                        if (++stage == kSt) { stage = 0; sphase ^= 1; }
-                    }
-                    umma_commit(&q_empty[qb]);
-                }
-            }
-        }
-    } else {
-#ifdef EVZ_X_SETMAXNREG
-        setmaxnreg_inc<112>();
-#endif
-        // ------------------------------------------------------------- epilogue
-        const int e = warp - 4;
-        const int quarter = warp & 3;                          // TMEM lane quarter this warp may read
-        const int grp = (e >> 2) & 1;                          // query sub-tile = accumulator
-        const int half = e >> 3;                               // column half of every tile
-        const int row = grp * 128 + quarter * 32 + lane;       // query row within the block
-        const uint32_t slot_a = smem_u32(smem + Cfg::slot_off) + half * Cfg::half_stride + row * 16, slot_b = slot_a + Cfg::slot_stride;
-        const uint32_t sum = slot_a + slot_b;
-        const uint32_t taddr = tmem_base + grp * kBlockT + half * (kBlockT / 2) + (static_cast<uint32_t>(quarter * 32) << 16);
-        const uint32_t acc_empty_a = smem_u32(&acc_empty[grp]);
-        const uint32_t bar_id = 1 + grp * 4 + quarter;         // the two warps that share this thread's rows
-        constexpr int kCh = kVCps / 2;                         // chunks of this thread per tile
-        uint32_t g = 0, qi = 0;
-        for (int it = blockIdx.x; it < n_items; it += gridDim.x) {
-            const uint32_t qb = qi & 1, qph = (qi >> 1) & 1;
-            ++qi;
-            mbar_wait(&q_full[qb], qph);
-            const Item im = item_s[qb];
-            if (grp < im.n_sub) {
-                uint32_t M1 = 0, M2 = 0, M3 = 0, sec = slot_b;
-                int Tb = -1, Ts = -1;
-                for (int n = 0; n < im.n_tiles; ++n) {
-                    M1 |= 255u; M2 |= 255u; M3 |= 255u;
-                    const uint32_t o1 = M1, o2 = M2;
-                    mbar_wait(&acc_full[grp], g & 1);
-                    tc_fence_after();
-                    if (args.dbg == 1) {                 // measurement of the TMA / MMA front end alone: results are garbage
-                        tc_fence_before();
-                        __syncwarp();
-                        if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" :: "r"(acc_empty_a) : "memory");
-                        ++g;
-                        continue;
-                    }
-                    {
-                        // eight loads of one chunk each, two ahead of the chunk being processed (four 16-register buffers)
-                        uint32_t r[4][16];
-                        tmem_ld_32x32b_x16(taddr, r[0]);
-                        tmem_ld_32x32b_x16(taddr + 16, r[1]);
-#pragma unroll
-                        for (int c = 0; c < kCh; ++c) {
-                            tmem_ld_wait_dep(r[c & 3]);
-                            if (c + 2 < kCh) {
-                                tmem_ld_32x32b_x16(taddr + (c + 2) * 16, r[(c + 2) & 3]);
-                            } else if (c + 2 == kCh) {
-                                tc_fence_before();
-                                __syncwarp();
-                                if (lane == 0) asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" :: "r"(acc_empty_a) : "memory");
-                            }
-                            vchunk<Cfg::part_stride>(&r[c & 3][0], 254 - half * kCh - c, args.mul256, M1, M2, M3, sec, sum);
-                            keep_alive16(&r[c & 3][0]);
-                        }
-                    }
-                    ++g;
-                    const int nTb = M1 == o1 ? Tb : n * kVCps + 254 - static_cast<int>(M1 & 255u);
-                    Ts = (M1 != o1 && M2 == o1) ? Tb : (M2 == o2 ? Ts : n * kVCps + 254 - static_cast<int>(M2 & 255u));
-                    Tb = nTb;
-                }
-                // exact evaluation of this half's two saved chunks (see match_top2_vkernel)
-                const int hm1 = im.pad + 1;
-                const bool best_first = Ts < 0 || Tb < Ts;
-                int k[2 * kVC];
-#pragma unroll
-                for (int s = 0; s < 2; ++s) {
-                    const int T = s == 0 ? Tb : Ts;
-                    const uint32_t sa = s == 0 ? sum - sec : sec;
-                    if (T >= 0) {
-                        const int base = (T >> kVClog) * kBlockT + (T & (kVCps - 1)) * kVC;
-                        const int cs = (2 * hm1) * 256 + ((s == 0) == best_first ? 0 : kVC);
-                        uint32_t ps;
-                        asm volatile("ld.shared.u16 %0, [%1];" : "=r"(ps) : "r"(smem_u32(smem + Cfg::pb_off) + qb * Cfg::pb_bytes + (base >> 3)));
-                        ps <<= 8;
-#pragma unroll
-                        for (int part = 0; part < kVC / 4; ++part) {
-                            const int4 v = lds128(sa + part * Cfg::part_stride);
-                            k[s * kVC + part * 4 + 0] = mad_key(v.x, args.neg512, cs) + (((ps >> (part * 4 + 0)) & 256) + part * 4 + 0);
-                            k[s * kVC + part * 4 + 1] = mad_key(v.y, args.neg512, cs) + (((ps >> (part * 4 + 1)) & 256) + part * 4 + 1);
-                            k[s * kVC + part * 4 + 2] = mad_key(v.z, args.neg512, cs) + (((ps >> (part * 4 + 2)) & 256) + part * 4 + 2);
-                            k[s * kVC + part * 4 + 3] = mad_key(v.w, args.neg512, cs) + (((ps >> (part * 4 + 3)) & 256) + part * 4 + 3);
-                        }
-                    } else {
-#pragma unroll
-                        for (int i = 0; i < kVC; ++i) k[s * kVC + i] = INT_MAX;
-                    }
-                }
-                int m1 = INT_MAX, m2 = INT_MAX;
-#pragma unroll
-                for (int i = 0; i < kVC; ++i) top2_pair(k[2 * i], k[2 * i + 1], m1, m2);
-                const int base_b = Tb >= 0 ? (Tb >> kVClog) * kBlockT + (Tb & (kVCps - 1)) * kVC : 0;
-                const int base_s = Ts >= 0 ? (Ts >> kVClog) * kBlockT + (Ts & (kVCps - 1)) * kVC : 0;
-                const int base_lo = best_first ? base_b : base_s, base_hi = best_first ? base_s : base_b;
-                const int c1 = ((m1 & kVC) ? base_hi : base_lo) + (m1 & (kVC - 1)), c2 = ((m2 & kVC) ? base_hi : base_lo) + (m2 & (kVC - 1));
-                int I1 = (m1 != INT_MAX && c1 < im.nt) ? c1 : -1, I2 = (m2 != INT_MAX && c2 < im.nt) ? c2 : -1;
-                int V1 = I1 >= 0 ? (m1 >> 8) : kAbsent, V2 = I2 >= 0 ? (m2 >> 8) : kAbsent;
-                // every column of this half outside its two slots has V <= V3, i.e. ||t||^2 - 2 q.t >= 2 (hmax + 1 - V3):
-                // this half's top-2 is exact unless its second distance reaches that bound
-                const bool third = M3 > 255u;
-                const int bound = 2 * (hm1 - static_cast<int>(M3 >> 8));
-                bool flagged = third && (I2 < 0 || V2 >= bound);
-                // merge the halves: the row's two nearest neighbours are among the two of either half
-                int4* mbuf = reinterpret_cast<int4*>(smem + Cfg::merge_off + (qi & 1) * Cfg::merge_bytes);
-                uint32_t* mflag = reinterpret_cast<uint32_t*>(mbuf + 256);
-                if (half == 1) {
-                    mbuf[row] = make_int4(V1, I1, V2, I2);
-                    mflag[row] = flagged ? 1u : 0u;
-                    named_bar_arrive(bar_id, 64);
-                } else {
-                    named_bar_sync(bar_id, 64);
-                    const int4 o = mbuf[row];
-                    flagged = flagged || mflag[row] != 0u;
-                    if (o.y >= 0) top2_insert(o.x, o.y, V1, I1, V2, I2);
-                    if (o.w >= 0) top2_insert(o.z, o.w, V1, I1, V2, I2);
-                    if (row < im.nq_left) {
-                        const int qn = __ldg(args.ckey + im.q_row0 + row) >> 8;
-                        const int64_t o_row = static_cast<int64_t>(im.out_row0) + row;
-                        int2 oi, od;
-                        oi.x = flagged ? kFlagged : I1; od.x = I1 >= 0 ? V1 + qn : -1;
-                        oi.y = I2;                      od.y = I2 >= 0 ? V2 + qn : -1;
-                        reinterpret_cast<int2*>(args.top2_idx)[o_row] = oi;
-                        reinterpret_cast<int2*>(args.top2_d2)[o_row] = od;
-                        if (flagged) {
-                            const int pos = atomicAdd(args.fix_count, 1);
-                            if (pos < args.fix_capacity) args.fix_list[pos] = it * 256 + row;
-                        }
-                    }
-                }
-            }
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&q_empty[qb]);
-        }
-    }
-
-    tc_fence_before();
-    __syncthreads();
-    if (warp == 2) tmem_dealloc(tmem_base, 512);
-}
-
-
-// ---- CTA-pair template (EVZ_OPT_MATCH_VARIANT = 7).  Only kCtas = 2 is instantiated; the kCtas == 1 branches are the
-// default kernel's code path (they are how the 4 % of the note above were measured) and compile to nothing.
-// one accumulator row (256 columns) in 16 loads of one chunk (16 columns) each, two loads ahead of the chunk being
-// processed, into four 16-register buffers: the load for chunk c + 2 overwrites the registers of chunk c - 2, whose
-// (predicated) stores were issued a whole chunk ago.  With 32-column loads one batch ahead, every load had to wait
-// for the stores of the batch just processed to read their operands (write-after-read on the registers, paid
-// whether or not the predicate is true).  The accumulator is handed back to the MMA warp as soon as its last
-// column is in registers.
-template <int kCtas>
-__device__ __forceinline__ void drain_v(uint32_t taddr, uint32_t mul, uint32_t& M1, uint32_t& M2, uint32_t& M3,
-                                        uint32_t& sec, uint32_t sum, uint32_t acc_empty, int lane) {
-    static_assert(kVC == 16, "one TMEM load per chunk");
-    uint32_t r[4][16];
-    tmem_ld_32x32b_x16(taddr, r[0]);
-    tmem_ld_32x32b_x16(taddr + 16, r[1]);
-#pragma unroll
-    for (int c = 0; c < kVCps; ++c) {
-        tmem_ld_wait_dep(r[c & 3]);
-        if (c + 2 < kVCps) {
-            tmem_ld_32x32b_x16(taddr + (c + 2) * 16, r[(c + 2) & 3]);
-        } else if (c + 2 == kVCps) {
-            tc_fence_before();
-            __syncwarp();
-            if (lane == 0) {
-                if (kCtas == 2) mbar_arrive_cluster(acc_empty);      // the leader CTA's barrier collects both CTAs
-                else asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" :: "r"(acc_empty) : "memory");
-            }
-        }
-        vchunk<VCfgT<kCtas>::part_stride>(&r[c & 3][0], 254 - c, mul, M1, M2, M3, sec, sum);
-        keep_alive16(&r[c & 3][0]);
-    }
-}
-
-template <int kCtas>
-__global__ void __launch_bounds__(VCfgT<kCtas>::threads, 1)
-match_top2_vkernel_t(const __grid_constant__ CUtensorMap tmap, const __grid_constant__ CUtensorMap tmap_half, const MatchArgs args) {
-    using Cfg = VCfgT<kCtas>;
-    constexpr int kSt = Cfg::stages;
-    extern __shared__ uint8_t smem_raw[];
-    uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
-    uint8_t* q_s = smem + Cfg::q_off;
-    uint8_t* t_s = smem + Cfg::t_off;
-    uint8_t* e_s = smem + Cfg::e_off;
-    uint8_t* a_s = smem + Cfg::a_off;
-    Item* item_s = reinterpret_cast<Item*>(smem + Cfg::item_off);
-    uint64_t* bars = reinterpret_cast<uint64_t*>(smem + Cfg::bar_off);
-    uint64_t* full = bars;                       // [kSt] this CTA's (part of the) train tile + its fifth K block landed (TMA tx)
-    uint64_t* empty = full + kSt;                // [kSt] MMA commit
-    uint64_t* q_full = empty + kSt;              // [2] query block landed + item descriptor published
-    uint64_t* q_empty = q_full + 2;              // [2] MMA commit + 8 epilogue warps
-    uint64_t* acc_full = q_empty + 2;            // [2] accumulator (= query sub-tile) ready (MMA commit)
-    uint64_t* acc_empty = acc_full + 2;          // [2] accumulator drained (its 4 epilogue warps; CTA pair: of both CTAs, on the leader's barrier)
-    uint64_t* pfull = acc_empty + 2;             // [kSt] CTA pair, leader only: the peer's half of the train tile landed
-    uint64_t* pq_full = pfull + kSt;             // [2]   CTA pair, leader only: the peer's query block landed
-    uint32_t* tmem_ptr_s = reinterpret_cast<uint32_t*>(smem + Cfg::tmem_off);
-
-    const int warp = threadIdx.x >> 5;
-    const int lane = threadIdx.x & 31;
-    const uint32_t rank = kCtas == 2 ? cluster_ctarank() : 0u;           // 0 = leader of the CTA pair (issues the MMAs)
-    const int unit = blockIdx.x / kCtas, n_units = gridDim.x / kCtas;   // CTA (pair) index: stride over the item list
-
-    if (warp == 0 && lane == 0) {
-        tma_prefetch_desc(&tmap);
-        if (kCtas == 2) tma_prefetch_desc(&tmap_half);
-        for (int i = 0; i < kSt; ++i) { mbar_init(&full[i], 1); mbar_init(&empty[i], 1); }
-        for (int i = 0; i < 2; ++i) {
-            mbar_init(&q_full[i], 1); mbar_init(&q_empty[i], 1 + 8);
-            mbar_init(&acc_full[i], 1); mbar_init(&acc_empty[i], 4 * kCtas);
-        }
-        if (kCtas == 2) {
-            for (int i = 0; i < kSt; ++i) mbar_init(&pfull[i], 1);
-            for (int i = 0; i < 2; ++i) mbar_init(&pq_full[i], 1);
-        }
-        fence_mbar_init();
-    }
-    if (warp == 2) {
-        if (kCtas == 2) { tmem_alloc_pair(tmem_ptr_s, 512); tmem_relinquish_pair(); }
-        else            { tmem_alloc(tmem_ptr_s, 512); tmem_relinquish(); }
-    }
-    if (warp == 3) {
-        // query-side fifth K block: every row = (255 x 30, 1, 0), no-swizzle core-matrix layout
-        for (int i = lane; i < 256; i += 32) {
-            const bool second = (i >> 3) & 1;          // [group 16][k half 2][row 8] x 16 B
-            reinterpret_cast<uint4*>(a_s)[i] = make_uint4(0xFFFFFFFFu, 0xFFFFFFFFu, 0xFFFFFFFFu, second ? 0x0001FFFFu : 0xFFFFFFFFu);
-        }
-        fence_proxy_async();
-    }
-    tc_fence_before();
-    if (kCtas == 2) cluster_sync_all();          // the peer's barriers must be initialised before anything arrives on them
-    else __syncthreads();
-    tc_fence_after();
-    const uint32_t tmem_base = *tmem_ptr_s;
-    const int n_items = *args.n_items;
-
-    if (warp == 0) {
-        // ------------------------------------------------------------- TMA producer (polling waits, single thread)
-        if (lane == 0) {
-            uint32_t stage = 0, sphase = 0, qi = 0;
-            for (int it = unit; it < n_items; it += n_units) {
-                const Item im = load_item(args, it * kCtas + rank);
-                const uint32_t qb = qi & 1, qph = (qi >> 1) & 1;
-                ++qi;
-                mbar_wait_spin(&q_empty[qb], qph ^ 1);
-                item_s[qb] = im;
-                if (im.n_tiles == 0) { mbar_arrive(&q_full[qb]); continue; }
-                mbar_arrive_expect_tx(&q_full[qb], kQBytes + im.n_tiles * 32);
-                tma_load_2d(q_s + qb * kQBytes, &tmap, 0, im.q_row0, &q_full[qb]);
-                bulk_load_1d(smem + Cfg::pb_off + qb * Cfg::pb_bytes, args.pbits + static_cast<size_t>(im.t_row0 >> 8) * 8,
-                             im.n_tiles * 32, &q_full[qb]);
-                // this CTA's part of every train tile: all 256 rows, or rows [128 rank, 128 rank + 128) of a CTA pair
-                const CUtensorMap* tm_t = kCtas == 2 ? &tmap_half : &tmap;
-                const int t_row = im.t_row0 + static_cast<int>(rank) * Cfg::tile_rows;
-                const uint8_t* ecode = args.ecode + static_cast<size_t>(im.t_row0 >> 8) * kECodeBytes + rank * Cfg::ecode_bytes;
-                for (int n = 0; n < im.n_tiles; ++n) {
-                    // the ring is only a few tiles deep: pull the tile that will be loaded kSt iterations from now
-                    // into L2 already, so that its TMA load is an L2 hit
-                    if (n + kSt < im.n_tiles) {
-                        tma_prefetch_2d(tm_t, 0, t_row + (n + kSt) * kBlockT);
-                        bulk_prefetch_1d(ecode + static_cast<size_t>(n + kSt) * kECodeBytes, Cfg::ecode_bytes);
-                    }
-                    mbar_wait_spin(&empty[stage], sphase ^ 1);
-                    mbar_arrive_expect_tx(&full[stage], Cfg::tile_bytes + Cfg::ecode_bytes);
-                    tma_load_2d(t_s + stage * Cfg::tile_bytes, tm_t, 0, t_row + n * kBlockT, &full[stage]);
-                    bulk_load_1d(e_s + stage * Cfg::ecode_bytes, ecode + static_cast<size_t>(n) * kECodeBytes, Cfg::ecode_bytes, &full[stage]);
-                    if (++stage == kSt) { stage = 0; sphase ^= 1; }
-                }
-            }
-        }
-    } else if (warp == 1) {
-        // ------------------------------------------------------------- MMA issuer
-        if (lane == 0 && rank == 0) {
-            // accumulator = query sub-tile.  The waits of this single thread poll: a tcgen05.mma issue blocks
-            // until the tensor pipe accepts it, so the pipe only stays fed while this thread is never late,
-            // and a suspended try_wait wakes up late.  CTA pair: this thread issues the 256-row MMAs of both
-            // CTAs (rows 0-127 = its own query sub-tile, 128-255 = the peer's; each CTA supplies 128 of the 256
-            // train rows) and its commits arrive on the barriers of both CTAs.
-            constexpr uint32_t idesc = umma_idesc_u8(128 * kCtas, kBlockT);
-            const uint64_t da_e = umma_desc_nosw(smem_u32(a_s), 128, 256);
-            uint32_t stage = 0, sphase = 0, qi = 0, gs[2] = {0, 0};
-            for (int it = unit; it < n_items; it += n_units) {
-                const uint32_t qb = qi & 1, qph = (qi >> 1) & 1;
-                ++qi;
-                mbar_wait_spin(&q_full[qb], qph);
-                if (kCtas == 2) mbar_wait_spin_cluster(&pq_full[qb], qph);
-                const int n_tiles = item_s[qb].n_tiles, n_sub = item_s[qb].n_sub;
-                const uint32_t q_addr = smem_u32(q_s + qb * kQBytes);
-                for (int n = 0; n < n_tiles; ++n) {
-                    mbar_wait_spin(&full[stage], sphase);
-                    if (kCtas == 2) mbar_wait_spin_cluster(&pfull[stage], sphase);
-                    const uint32_t t_addr = smem_u32(t_s + stage * Cfg::tile_bytes);
-                    const uint64_t db_e = umma_desc_nosw(smem_u32(e_s + stage * Cfg::ecode_bytes), 128, 256);
-                    for (int sub = 0; sub < n_sub; ++sub) {
-                        const uint32_t aph = gs[sub]++ & 1;
-                        if (kCtas == 2) mbar_wait_spin_cluster(&acc_empty[sub], aph ^ 1);
-                        else mbar_wait_spin(&acc_empty[sub], aph ^ 1);
-                        tc_fence_after();
-#pragma unroll
-                        for (int k = 0; k < kRowBytes / 32; ++k) {
-                            const uint64_t da = umma_desc_sw128(q_addr + sub * (128 * kRowBytes) + k * 32);
-                            const uint64_t db = umma_desc_sw128(t_addr + k * 32);
-                            if (kCtas == 2) umma_i8_pair(tmem_base + sub * kBlockT, da, db, idesc, k > 0 ? 1u : 0u);
-                            else umma_i8(tmem_base + sub * kBlockT, da, db, idesc, k > 0 ? 1u : 0u);
-                        }
-                        if (kCtas == 2) { umma_i8_pair(tmem_base + sub * kBlockT, da_e, db_e, idesc, 1u); umma_commit_pair(&acc_full[sub]); }
-                        else            { umma_i8(tmem_base + sub * kBlockT, da_e, db_e, idesc, 1u); umma_commit(&acc_full[sub]); }
-                    }
-                    if (kCtas == 2) umma_commit_pair(&empty[stage]); else umma_commit(&empty[stage]);
-                    if (++stage == kSt) { stage = 0; sphase ^= 1; }
-                }
-                if (kCtas == 2) umma_commit_pair(&q_empty[qb]); else umma_commit(&q_empty[qb]);
-            }
-        } else if (kCtas == 2 && lane == 0) {
-            // peer CTA of a pair: forward "my query block / my half of the tile has landed" to the leader's barriers
-            const uint32_t r_pfull = mapa_u32(smem_u32(pfull), 0), r_pq_full = mapa_u32(smem_u32(pq_full), 0);
-            uint32_t stage = 0, sphase = 0, qi = 0;
-            for (int it = unit; it < n_items; it += n_units) {
-                const uint32_t qb = qi & 1, qph = (qi >> 1) & 1;
-                ++qi;
-                mbar_wait_spin(&q_full[qb], qph);
-                const int n_tiles = item_s[qb].n_tiles;     // read before the leader can release the item
-                mbar_arrive_cluster(r_pq_full + qb * 8);
-                for (int n = 0; n < n_tiles; ++n) {
-                    mbar_wait_spin(&full[stage], sphase);
-                    mbar_arrive_cluster(r_pfull + stage * 8);
-                    if (++stage == kSt) { stage = 0; sphase ^= 1; }
-                }
-            }
-        }
-    } else if (warp >= 4) {
-        // ------------------------------------------------------------- epilogue
-        const int grp = (warp - 4) >> 2;                       // query sub-tile = accumulator
-        const int quarter = warp & 3;                          // TMEM lane quarter this warp may read
-        const int row = grp * 128 + quarter * 32 + lane;       // query row within the block
-        const uint32_t slot_a = smem_u32(smem + Cfg::slot_off) + row * 16, slot_b = slot_a + Cfg::slot_stride;
-        const uint32_t sum = slot_a + slot_b;
-        const uint32_t taddr = tmem_base + grp * kBlockT + (static_cast<uint32_t>(quarter * 32) << 16);
-        const uint32_t acc_empty_a = kCtas == 2 ? mapa_u32(smem_u32(&acc_empty[grp]), 0) : smem_u32(&acc_empty[grp]);
-        uint32_t g = 0, qi = 0;
-        for (int it = unit; it < n_items; it += n_units) {
-            const uint32_t qb = qi & 1, qph = (qi >> 1) & 1;
-            ++qi;
-            mbar_wait(&q_full[qb], qph);
-            const Item im = item_s[qb];
-            if (grp < im.n_sub) {
-                const int qkey = row < im.nq_left ? __ldg(args.ckey + im.q_row0 + row) : 0;
-                // sorted top-3 of chunk keys, the slot that holds the second-best chunk, and the position
-                // (tile * 16 + chunk) of the chunks in the best / second-best slot
-                uint32_t M1 = 0, M2 = 0, M3 = 0, sec = slot_b;
-                int Tb = -1, Ts = -1;
-                for (int n = 0; n < im.n_tiles; ++n) {
-                    // keys of earlier tiles beat every key of this tile with the same V (lowest index wins)
-                    M1 |= 255u; M2 |= 255u; M3 |= 255u;
-                    const uint32_t o1 = M1, o2 = M2;
-                    mbar_wait(&acc_full[grp], g & 1);
-                    tc_fence_after();
-                    if (args.dbg == 1) {                 // measurement of the TMA / MMA front end alone: results are garbage
-                        tc_fence_before();
-                        __syncwarp();
-                        if (lane == 0) {
-                            if (kCtas == 2) mbar_arrive_cluster(acc_empty_a);
-                            else asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" :: "r"(acc_empty_a) : "memory");
-                        }
-                        ++g;
-                        continue;
-                    }
-                    if (args.dbg == 2) {                 // measurement: TMEM loads only (no max tree, no saves); results are garbage
-                        uint32_t r[4][16];
-                        tmem_ld_32x32b_x16(taddr, r[0]);
-                        tmem_ld_32x32b_x16(taddr + 16, r[1]);
-#pragma unroll
-                        for (int c = 0; c < kVCps; ++c) {
-                            tmem_ld_wait_dep(r[c & 3]);
-                            if (c + 2 < kVCps) tmem_ld_32x32b_x16(taddr + (c + 2) * 16, r[(c + 2) & 3]);
-                            keep_alive16(&r[c & 3][0]);
-                        }
-                        tc_fence_before();
-                        __syncwarp();
-                        if (lane == 0) {
-                            if (kCtas == 2) mbar_arrive_cluster(acc_empty_a);
-                            else asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" :: "r"(acc_empty_a) : "memory");
-                        }
-                        ++g;
-                        continue;
-                    }
-                    drain_v<kCtas>(taddr, args.mul256, M1, M2, M3, sec, sum, acc_empty_a, lane);
-                    ++g;
-                    const int nTb = M1 == o1 ? Tb : n * kVCps + 254 - static_cast<int>(M1 & 255u);
-                    Ts = (M1 != o1 && M2 == o1) ? Tb : (M2 == o2 ? Ts : n * kVCps + 254 - static_cast<int>(M2 & 255u));
-                    Tb = nTb;
-                }
-                // exact evaluation of the two saved chunks: ||t||^2 - 2 q.t = 2 (hmax + 1 - V) + parity, packed
-                // with the ordinal of the column among the 32 candidates (the slot with the lower position
-                // first), so that a signed min is the lexicographic (distance, index) minimum.  Padding
-                // columns have V = 0, i.e. a distance above every real column: they sort last by themselves.
-                const int hm1 = im.pad + 1;
-                const bool best_first = Ts < 0 || Tb < Ts;
-                int k[2 * kVC];
-#pragma unroll
-                for (int s = 0; s < 2; ++s) {
-                    const int T = s == 0 ? Tb : Ts;
-                    const uint32_t sa = s == 0 ? sum - sec : sec;
-                    if (T >= 0) {
-                        const int base = (T >> kVClog) * kBlockT + (T & (kVCps - 1)) * kVC;
-                        const int cs = (2 * hm1) * 256 + ((s == 0) == best_first ? 0 : kVC);
-                        uint32_t ps;                       // norm parity of the chunk's columns, moved to bits 8..
-                        if (kVC == 16) asm volatile("ld.shared.u16 %0, [%1];" : "=r"(ps) : "r"(smem_u32(smem + Cfg::pb_off) + qb * Cfg::pb_bytes + (base >> 3)));
-                        else           asm volatile("ld.shared.u8 %0, [%1];" : "=r"(ps) : "r"(smem_u32(smem + Cfg::pb_off) + qb * Cfg::pb_bytes + (base >> 3)));
-                        ps <<= 8;
-#pragma unroll
-                        for (int part = 0; part < kVC / 4; ++part) {
-                            const int4 v = lds128(sa + part * Cfg::part_stride);
-                            k[s * kVC + part * 4 + 0] = mad_key(v.x, args.neg512, cs) + (((ps >> (part * 4 + 0)) & 256) + part * 4 + 0);
-                            k[s * kVC + part * 4 + 1] = mad_key(v.y, args.neg512, cs) + (((ps >> (part * 4 + 1)) & 256) + part * 4 + 1);
-                            k[s * kVC + part * 4 + 2] = mad_key(v.z, args.neg512, cs) + (((ps >> (part * 4 + 2)) & 256) + part * 4 + 2);
-                            k[s * kVC + part * 4 + 3] = mad_key(v.w, args.neg512, cs) + (((ps >> (part * 4 + 3)) & 256) + part * 4 + 3);
-                        }
-                    } else {
-#pragma unroll
-                        for (int i = 0; i < kVC; ++i) k[s * kVC + i] = INT_MAX;
-                    }
-                }
-                int m1 = INT_MAX, m2 = INT_MAX;
-#pragma unroll
-                for (int i = 0; i < kVC; ++i) top2_pair(k[2 * i], k[2 * i + 1], m1, m2);
-                const int base_b = Tb >= 0 ? (Tb >> kVClog) * kBlockT + (Tb & (kVCps - 1)) * kVC : 0;
-                const int base_s = Ts >= 0 ? (Ts >> kVClog) * kBlockT + (Ts & (kVCps - 1)) * kVC : 0;
-                const int base_lo = best_first ? base_b : base_s, base_hi = best_first ? base_s : base_b;
-                const int c1 = ((m1 & kVC) ? base_hi : base_lo) + (m1 & (kVC - 1)), c2 = ((m2 & kVC) ? base_hi : base_lo) + (m2 & (kVC - 1));
-                const int I1 = (m1 != INT_MAX && c1 < im.nt) ? c1 : -1, I2 = (m2 != INT_MAX && c2 < im.nt) ? c2 : -1;
-                const int V1 = m1 >> 8, V2 = m2 >> 8;
-                // every column outside the two slots has V <= V3, i.e. ||t||^2 - 2 q.t >= 2 (hmax + 1 - V3)
-                const bool third = M3 > 255u;
-                const int bound = 2 * (hm1 - static_cast<int>(M3 >> 8));
-                const bool flagged = third && (I2 < 0 || V2 >= bound);
-                if (row < im.nq_left) {
-                    const int qn = qkey >> 8;
-                    const int64_t o_row = static_cast<int64_t>(im.out_row0) + row;
-                    int2 oi, od;
-                    oi.x = flagged ? kFlagged : I1; od.x = I1 >= 0 ? V1 + qn : -1;
-                    oi.y = I2;                      od.y = I2 >= 0 ? V2 + qn : -1;
-                    reinterpret_cast<int2*>(args.top2_idx)[o_row] = oi;
-                    reinterpret_cast<int2*>(args.top2_d2)[o_row] = od;
-                    if (flagged) {
-                        const int pos = atomicAdd(args.fix_count, 1);
-                        if (pos < args.fix_capacity) args.fix_list[pos] = (it * kCtas + static_cast<int>(rank)) * 256 + row;
-                    }
-                }
-            }
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&q_empty[qb]);
-        }
-        }
-
-    tc_fence_before();
-    if (kCtas == 2) {
-        // neither CTA may leave (or free its TMEM) while the peer can still touch its shared memory or barriers
-        cluster_sync_all();
-        if (warp == 2) tmem_dealloc_pair(tmem_base, 512);
-    } else {
-        __syncthreads();
-        if (warp == 2) tmem_dealloc(tmem_base, 512);
-    }
 }
 
 // Per pair: hmax / range test of the train frame, then the 32 code bytes of every train row in the
@@ -2117,7 +895,7 @@ match_prepare_kernel(const int32_t* ckey, const int32_t* row_off, const int32_t*
     hmax = s_max[0]; hmin = s_min[0];
 #pragma unroll
     for (int w = 1; w < 8; ++w) { hmax = max(hmax, s_max[w]); hmin = min(hmin, s_min[w]); }
-    // (frames above EVZ_MAX_KP would overflow the kernel's parity bitmap buffers: legacy kernel as well)
+    // (frames above EVZ_MAX_KP would overflow the kernel's parity bitmap buffers: key-space kernel as well)
     const bool wide = nt > 0 && (hmax - hmin + 1 > kEMax || nt > EVZ_MAX_KP);
     if (tid == 0) { pair_hmax[p] = hmax; pair_flag[p] = wide ? 1 : 0; }
     if (wide) return;
@@ -2223,15 +1001,6 @@ static int ensure_tmap(evz_handle* h, const uint8_t* desc, int64_t total_rows) {
         EVZ_SET_ERR(h, "cuTensorMapEncodeTiled failed with CUresult %d (rows=%lld)", static_cast<int>(r), static_cast<long long>(total_rows));
         return EVZ_E_CUDA;
     }
-    // CTA-pair kernel: each CTA of a pair stages 128 of the 256 rows of a train tile
-    const cuuint32_t box_half[2] = {static_cast<cuuint32_t>(evz::kRowBytes), 128u};
-    const CUresult r2 = h->encode(&h->tmap_half, CU_TENSOR_MAP_DATA_TYPE_UINT8, 2, const_cast<uint8_t*>(desc), dims, strides, box_half, estr,
-                                  CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                                  CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r2 != CUDA_SUCCESS) {
-        EVZ_SET_ERR(h, "cuTensorMapEncodeTiled (half tiles) failed with CUresult %d (rows=%lld)", static_cast<int>(r2), static_cast<long long>(total_rows));
-        return EVZ_E_CUDA;
-    }
     h->tmap_ptr = desc;
     h->tmap_rows = total_rows;
     return EVZ_OK;
@@ -2261,11 +1030,9 @@ extern "C" int evz_match_top2_d(evz_handle* h, const uint8_t* desc, int desc_byt
     // every pair owns at most ceil(n_kp/256) <= rows/256 + 1 items
     const size_t capacity = static_cast<size_t>(total_rows / evz::kBlockQ) + static_cast<size_t>(n_pairs);
     EVZ_REQUIRE(h, capacity < (size_t(1) << 30), "too many work items");
-    // EVZ_OPT_MATCH_VARIANT: 0 = V-space kernel (norm in a fifth K block; default); legacy kernel: 1 = exact
-    // per-element top-2, 2 = chunk minima of 16, 5 (and any other value) = chunk minima of 8
-    const int variant = h->opt_match_variant;
-    const bool vpair = variant == 7;                 // V-space kernel on CTA pairs (cta_group::2)
-    const bool vspace = variant == 0 || vpair || variant == 8 || variant == 9;
+    // EVZ_OPT_MATCH_VARIANT: 0 = V-space kernel for the pairs it can encode, key-space kernel for the rest (default);
+    // 5 = key-space kernel for every pair (evz_set_option accepts no other value)
+    const bool vspace = h->opt_match_variant == 0;
     // scratch: [counters 256 B][items A][items B][pair_hmax][pair_flag][ecode]
     const size_t items_bytes = evz_align_up(capacity * 8, 256), pair_bytes = evz_align_up(static_cast<size_t>(n_pairs) * 4, 256);
     const size_t fix_bytes = evz_align_up(capacity * 256 * 4, 256);          // every row of every item, at worst
@@ -2279,18 +1046,7 @@ extern "C" int evz_match_top2_d(evz_handle* h, const uint8_t* desc, int desc_byt
     int32_t* n_items = reinterpret_cast<int32_t*>(sb);
     int32_t* items = reinterpret_cast<int32_t*>(sb + 256);
     evz::MatchArgs a{ckey, row_off, n_kp, pair_q, pair_t, out_off, items, n_items, top2_idx, top2_d2, -512, nullptr, nullptr, nullptr, 256u,
-                     nullptr, nullptr, 0, h->opt_match_debug, 0, (desc_bytes + 31) / 32};
-#define EVZ_MATCH_LAUNCH(CH, EW)                                                                                         \
-    do {                                                                                                                 \
-        using Cfg = evz::MatchCfg<CH, EW>;                                                                               \
-        constexpr unsigned kBit = CH == 0 ? 1u : CH == 8 ? 2u : 4u;                                                      \
-        if (!(h->attr_match & kBit)) {                                                                                   \
-            EVZ_CUDA_CHECK(h, cudaFuncSetAttribute(evz::match_top2_kernel<CH, EW>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                                                   Cfg::smem_bytes));                                                    \
-            h->attr_match |= kBit;                                                                                       \
-        }                                                                                                                \
-        evz::match_top2_kernel<CH, EW><<<h->sm_count, Cfg::threads, Cfg::smem_bytes, st>>>(h->tmap, a);                  \
-    } while (0)
+                     nullptr, nullptr, 0, 0, (desc_bytes + 31) / 32};
     if (vspace) {
         int32_t* n_items_slow = n_items + 16;
         int32_t* items_slow = reinterpret_cast<int32_t*>(sb + 256 + items_bytes);
@@ -2304,22 +1060,14 @@ extern "C" int evz_match_top2_d(evz_handle* h, const uint8_t* desc, int desc_byt
         a.pbits = pbits;
         evz::match_prepare_kernel<<<n_pairs, 256, 0, st>>>(ckey, row_off, n_kp, pair_t, pair_hmax, pair_flag, ecode, pbits, a.fix_count);
         EVZ_LAUNCH_CHECK(h);
-        evz::build_items_kernel<<<1, 1024, 0, st>>>(n_kp, pair_q, n_pairs, items, n_items, static_cast<int>(capacity), pair_flag, 0,
-                                                    vpair ? 2 * evz::kBlockQ : evz::kBlockQ);
-        evz::build_items_kernel<<<1, 1024, 0, st>>>(n_kp, pair_q, n_pairs, items_slow, n_items_slow, static_cast<int>(capacity), pair_flag, 1,
-                                                    evz::kBlockQ);
+        evz::build_items_kernel<<<1, 1024, 0, st>>>(n_kp, pair_q, n_pairs, items, n_items, static_cast<int>(capacity), pair_flag, 0);
+        evz::build_items_kernel<<<1, 1024, 0, st>>>(n_kp, pair_q, n_pairs, items_slow, n_items_slow, static_cast<int>(capacity), pair_flag, 1);
         EVZ_LAUNCH_CHECK(h);
         a.pair_hmax = pair_hmax;
         a.ecode = ecode;
-        if (!(h->attr_match & 8u)) {
-            EVZ_CUDA_CHECK(h, cudaFuncSetAttribute(evz::match_top2_vkernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, evz::VCfg::smem_bytes));
-            EVZ_CUDA_CHECK(h, cudaFuncSetAttribute(evz::match_top2_vkernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, evz::VCfg::smem_bytes));
-            EVZ_CUDA_CHECK(h, cudaFuncSetAttribute(evz::match_top2_vkernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, evz::VCfg::smem_bytes));
-            EVZ_CUDA_CHECK(h, cudaFuncSetAttribute(evz::match_top2_vkernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, evz::VCfg::smem_bytes));
-            EVZ_CUDA_CHECK(h, cudaFuncSetAttribute(evz::match_top2_vkernel_t<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, evz::VCfgT<2>::smem_bytes));
-            EVZ_CUDA_CHECK(h, cudaFuncSetAttribute(evz::match_top2_wkernel, cudaFuncAttributeMaxDynamicSharedMemorySize, evz::VCfg::smem_bytes));
-            EVZ_CUDA_CHECK(h, cudaFuncSetAttribute(evz::match_top2_xkernel, cudaFuncAttributeMaxDynamicSharedMemorySize, evz::XCfg::smem_bytes));
-            h->attr_match |= 8u;
+        if (!(h->attr_match & 2u)) {
+            EVZ_CUDA_CHECK(h, cudaFuncSetAttribute(evz::match_top2_vkernel, cudaFuncAttributeMaxDynamicSharedMemorySize, evz::VCfg::smem_bytes));
+            h->attr_match |= 2u;
         }
         cudaEvent_t* tev = nullptr;
         if (h->opt_time_match) {
@@ -2330,52 +1078,25 @@ extern "C" int evz_match_top2_d(evz_handle* h, const uint8_t* desc, int desc_byt
             tev = h->match_ev[h->match_calls++ & 15];
             EVZ_CUDA_CHECK(h, cudaEventRecord(tev[0], st));
         }
-        if (vpair) {
-            a.pair_mode = 1;
-            cudaLaunchConfig_t cfg = {};
-            cfg.gridDim = dim3(static_cast<unsigned>(h->sm_count / 2 * 2));
-            cfg.blockDim = dim3(evz::VCfgT<2>::threads);
-            cfg.dynamicSmemBytes = evz::VCfgT<2>::smem_bytes;
-            cfg.stream = st;
-            cudaLaunchAttribute at[1];
-            at[0].id = cudaLaunchAttributeClusterDimension;
-            at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-            cfg.attrs = at;
-            cfg.numAttrs = 1;
-            EVZ_CUDA_CHECK(h, cudaLaunchKernelEx(&cfg, evz::match_top2_vkernel_t<2>, h->tmap, h->tmap_half, a));
-        } else if (variant == 9) {
-            evz::match_top2_xkernel<<<h->sm_count, evz::XCfg::threads, evz::XCfg::smem_bytes, st>>>(h->tmap, a);
-        } else if (variant == 8) {
-            evz::match_top2_wkernel<<<h->sm_count, evz::VCfg::threads, evz::VCfg::smem_bytes, st>>>(h->tmap, a);
-        } else if (h->opt_match_debug == 1) {
-            evz::match_top2_vkernel<1><<<h->sm_count, evz::VCfg::threads, evz::VCfg::smem_bytes, st>>>(h->tmap, a);
-        } else if (h->opt_match_debug == 2) {
-            evz::match_top2_vkernel<2><<<h->sm_count, evz::VCfg::threads, evz::VCfg::smem_bytes, st>>>(h->tmap, a);
-        } else if (h->opt_match_debug == 3) {
-            evz::match_top2_vkernel<3><<<h->sm_count, evz::VCfg::threads, evz::VCfg::smem_bytes, st>>>(h->tmap, a);
-        } else {
-            evz::match_top2_vkernel<0><<<h->sm_count, evz::VCfg::threads, evz::VCfg::smem_bytes, st>>>(h->tmap, a);
-        }
+        evz::match_top2_vkernel<<<h->sm_count, evz::VCfg::threads, evz::VCfg::smem_bytes, st>>>(h->tmap, a);
         EVZ_LAUNCH_CHECK(h);
         if (tev) EVZ_CUDA_CHECK(h, cudaEventRecord(tev[1], st));
         evz::match_fixup_kernel<<<h->sm_count * 16, 128, 0, st>>>(desc, a);      // latency-bound (one row per CTA at a time): fill the SMs
         EVZ_LAUNCH_CHECK(h);
-        // pairs whose train frame has a norm range the fifth K block cannot encode: legacy kernel (normally no items)
+        // pairs whose train frame has a norm range the fifth K block cannot encode go to the key-space kernel
+        // below (normally no items)
         a.items = items_slow;
         a.n_items = n_items_slow;
         a.pair_hmax = nullptr;
-        a.pair_mode = 0;
-        EVZ_MATCH_LAUNCH(8, 8);
     } else {
-        evz::build_items_kernel<<<1, 1024, 0, st>>>(n_kp, pair_q, n_pairs, items, n_items, static_cast<int>(capacity), nullptr, 0, evz::kBlockQ);
+        evz::build_items_kernel<<<1, 1024, 0, st>>>(n_kp, pair_q, n_pairs, items, n_items, static_cast<int>(capacity), nullptr, 0);
         EVZ_LAUNCH_CHECK(h);
-        switch (variant) {
-            case 1:  EVZ_MATCH_LAUNCH(0, 8); break;
-            case 2:  EVZ_MATCH_LAUNCH(16, 8); break;
-            default: EVZ_MATCH_LAUNCH(8, 8); break;
-        }
     }
-#undef EVZ_MATCH_LAUNCH
+    if (!(h->attr_match & 1u)) {
+        EVZ_CUDA_CHECK(h, cudaFuncSetAttribute(evz::match_top2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, evz::MatchCfg::smem_bytes));
+        h->attr_match |= 1u;
+    }
+    evz::match_top2_kernel<<<h->sm_count, evz::MatchCfg::threads, evz::MatchCfg::smem_bytes, st>>>(h->tmap, a);
     EVZ_LAUNCH_CHECK(h);
     return EVZ_OK;
 }

@@ -5,7 +5,6 @@ hand-written CUDA behind the C ABI of include/evz.h.  All heavy results stay on 
 as torch tensors; `video_geometry` is the host-arrays-in / host-arrays-out call.
 """
 import ctypes as C
-import os
 from dataclasses import dataclass, field
 from typing import Optional
 
@@ -95,8 +94,6 @@ class GeometryEngine:
             raise _lib.EvzError(self.lib.evz_last_error(None).decode())
         self.h = h
         self.sm_count = self.lib.evz_sm_count(self.h)
-        if os.environ.get("EVZ_MATCH_VARIANT"):          # A/B of the match kernels (EVZ_OPT_MATCH_VARIANT), results identical
-            self.set_option(2, int(os.environ["EVZ_MATCH_VARIANT"]))
 
     def __del__(self):
         try:

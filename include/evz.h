@@ -84,27 +84,15 @@ int         evz_sm_count(const evz_handle* h);
 
 /* debugging / A-B options; results are identical for every setting, only the route differs */
 #define EVZ_OPT_RANSAC_EXACT   1  /* 1: score every hypothesis x match with the exactly-rounded formula (no fused fast path) */
-#define EVZ_OPT_MATCH_VARIANT  2  /* match kernel: 0 default ("V-space": the train norm enters the accumulator through a
-                                     fifth K block, max-tree epilogue, exact resolution from two saved chunks + fix-up);
-                                     key-space kernel (distance/index keys formed per element): 5 chunk-8 minima + saved
-                                     best chunk, 1 exact top-2 per element, 2 chunk-16 minima;
-                                     7: the V-space kernel on CTA pairs (tcgen05 cta_group::2: a 2-CTA cluster shares every
-                                     train tile, each CTA stages half of it and drains its own 256 query rows) -- bit-identical,
-                                     5 % slower than 0 on B200 (DESIGN.md K1), kept for A/B;
-                                     8: two-pass drain (chunk maxima first, then only the row's two best chunks of the tile are
-                                     re-read from tensor memory in the 16x256b shape and saved by a quad of threads): a quarter of
-                                     the shared-memory store cycles, but 2.4x slower -- the second pass is a serial chain of
-                                     ballot / load / store steps per warp; 9: sixteen drain warps (eight per accumulator, column
-                                     halves, per-half save slots, two-stage tile ring): 19 % slower.  Both bit-identical, kept as
-                                     measured negative results (DESIGN.md K1, round 2) */
+#define EVZ_OPT_MATCH_VARIANT  2  /* match route: 0 (default) = the "V-space" kernel (the train norm enters the accumulator
+                                     through a fifth K block, max-tree epilogue, exact resolution from two saved chunks +
+                                     fix-up) for every pair whose train frame it can encode, the key-space kernel for the rest;
+                                     5 = the key-space kernel (distance/index keys formed per element, chunk-8 minima + saved
+                                     best chunk) for every pair.  Any other value returns EVZ_E_ARG */
 #define EVZ_OPT_RANSAC_NO_PRUNE 3  /* 1: score every valid hypothesis even after one of them counted all matches as inliers
                                      (default 0: hypotheses that can no longer win the (count desc, index asc) arg-max are skipped) */
 #define EVZ_OPT_TIME_MATCH     4  /* 1: evz_match_top2 brackets its main kernel with CUDA events on the caller's stream (a ring of
                                      16 pairs, one per call); read them with evz_match_kernel_ms after synchronising */
-#define EVZ_OPT_MATCH_DEBUG    5  /* measurement only, NOT result-preserving (outputs are undefined): 1 = the V-space epilogue releases
-                                     every accumulator without draining it (times the TMA / tcgen05 front end alone); 2 = it loads
-                                     every accumulator column from TMEM but does no arithmetic and no saves; 3 = all eight drain warps work on
-                                     one accumulator at a time (column halves sharing their save slots): the timing of an eight-warp drain */
 int         evz_set_option(evz_handle* h, int option, int value);
 /* elapsed time of the main match kernel of the k-th most recent evz_match_top2 call (k = 0: the last one), for the
  * roofline line of bench.py.  The stream must have been synchronised; returns EVZ_E_ARG when no such record exists. */

@@ -1,4 +1,4 @@
-"""Micro-benchmark of the match kernel alone: bench_match.py [pairs] [keypoints] [variants, e.g. 0,5,7] [EVZ_OPT_MATCH_DEBUG] [descriptor bytes: 128 | 32]."""
+"""Micro-benchmark of the match kernel alone: bench_match.py [pairs] [keypoints] [EVZ_OPT_MATCH_VARIANT values, default 0,5] [descriptor bytes: 128 | 32]."""
 import sys, os
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -8,9 +8,7 @@ P = int(sys.argv[1]) if len(sys.argv) > 1 else 2000
 N = int(sys.argv[2]) if len(sys.argv) > 2 else 2048
 variants = [int(v) for v in sys.argv[3].split(",")] if len(sys.argv) > 3 else [0, 5]
 eng = evz.GeometryEngine(0)
-D = int(sys.argv[5]) if len(sys.argv) > 5 else 128
-if len(sys.argv) > 4:
-    eng.set_option(5, int(sys.argv[4]))      # EVZ_OPT_MATCH_DEBUG: 1 = front end alone (results undefined)
+D = int(sys.argv[4]) if len(sys.argv) > 4 else 128
 ch = synth.make_chain(P + 1, N, d=D, seed=0, device="cuda")
 st = eng.ingest(ch["desc"], ch["coords"])
 pq = torch.arange(1, P + 1, dtype=torch.int32, device="cuda"); pt = torch.arange(0, P, dtype=torch.int32, device="cuda")
@@ -29,7 +27,7 @@ for v in variants:
     e1.record(); e1.synchronize()
     ms = e0.elapsed_time(e1) / 5
     line = f"variant {v}: {ms:.3f} ms  {2.0*N*N*D*P/ms/1e9:.1f} TOP/s (whole call)"
-    if v in (0, 7, 8, 9): # V-space kernels: duration of the main kernel alone (EVZ_OPT_TIME_MATCH)
+    if v == 0:            # V-space kernel: duration of the main kernel alone (EVZ_OPT_TIME_MATCH)
         eng.set_option(4, 1)
         for _ in range(5): call()
         torch.cuda.synchronize()

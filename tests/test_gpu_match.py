@@ -235,8 +235,8 @@ def test_match_full_size_properties(engine):
 
 
 def test_match_epilogue_variants_agree(engine):
-    """Default epilogue (chunk minima + saved best chunk) vs the straightforward exact top-2 per element,
-    for every epilogue variant of EVZ_OPT_MATCH_VARIANT."""
+    """Default route (V-space kernel) vs the key-space kernel for every pair (EVZ_OPT_MATCH_VARIANT = 5) on tie-heavy
+    data, and both against the oracle."""
     from evenvizion_b200 import synth
     ch = synth.make_chain(6, 2048, seed=8, device="cuda")
     d = ch["desc"].clone()
@@ -245,14 +245,13 @@ def test_match_epilogue_variants_agree(engine):
     d[4, :] = d[4, 0:1]                   # a whole frame of identical descriptors
     st = engine.ingest(d, ch["coords"])
     outs = {}
-    for v in (0, 1, 2, 5, 7, 8, 9):
+    for v in (0, 5):
         engine.set_option(2, v)
         outs[v] = engine.match(st, list(range(1, 6)), list(range(0, 5)))
     engine.set_option(2, 0)
     q0 = int(st.row_off_h[1])
-    for v in (1, 2, 5, 7, 8, 9):
-        assert torch.equal(outs[0].top2_idx[q0:], outs[v].top2_idx[q0:]), v
-        assert torch.equal(outs[0].top2_d2[q0:], outs[v].top2_d2[q0:]), v
+    assert torch.equal(outs[0].top2_idx[q0:], outs[5].top2_idx[q0:])
+    assert torch.equal(outs[0].top2_d2[q0:], outs[5].top2_d2[q0:])
     # and both equal the oracle on the tie-heavy pairs
     dn = d.cpu().numpy()
     for p in (2, 3, 4):
@@ -262,9 +261,25 @@ def test_match_epilogue_variants_agree(engine):
         assert np.array_equal(outs[0].top2_d2[o:o + 2048].cpu().numpy().astype(np.int64), d2)
 
 
+def test_match_options_reject_unknown_routes(engine):
+    """EVZ_OPT_MATCH_VARIANT takes 0 or 5 only and option 5 does not exist: both are EVZ_E_ARG, and the rejected
+    values leave the default route in place."""
+    from evenvizion_b200 import EvzError
+    for v in (1, 2, 7, 8, 9):
+        with pytest.raises(EvzError):
+            engine.set_option(2, v)
+    with pytest.raises(EvzError):
+        engine.set_option(5, 1)
+    frames = _ragged_frames([300, 520], seed=4)
+    st = _ingest(engine, frames)
+    r = engine.match(st, [1], [0])
+    torch.cuda.synchronize()
+    _check_pair(engine, st, r, 0, frames, 1, 0)
+
+
 def _check_launch_against_gemm(engine, st, pq, pt, counts, dd, offs):
     outs = {}
-    for v in (0, 1, 2, 5, 7, 8, 9):
+    for v in (0, 5):
         engine.set_option(2, v)
         outs[v] = [engine.match(st, pq, pt) for _ in range(2 if v == 0 else 1)]
     engine.set_option(2, 0)
@@ -293,8 +308,8 @@ def _check_launch_against_gemm(engine, st, pq, pt, counts, dd, offs):
 
 def test_match_ragged_stress_against_device_reference(engine):
     """Many ragged items through the persistent kernel (item ring, merge double-buffering, sentinel across
-    tiles, ckey ring wrap-around): every pair against an exact f32 GEMM on the device, for all epilogue
-    variants, and bit-identical across repeated runs."""
+    tiles, ckey ring wrap-around): every pair against an exact f32 GEMM on the device, for both match routes
+    (EVZ_OPT_MATCH_VARIANT 0 and 5), and bit-identical across repeated runs."""
     rng = np.random.default_rng(123)
     sizes = [0, 1, 2, 7, 8, 9, 127, 128, 129, 255, 256, 257, 511, 512, 513, 700, 1023, 1024, 1025, 1500, 2047, 2048, 2049, 2600]
     counts = [int(rng.choice(sizes)) for _ in range(90)]
@@ -321,7 +336,7 @@ def test_match_ragged_stress_against_device_reference(engine):
 
 def test_match_wide_norm_range_falls_back(engine):
     """A train frame whose norm range exceeds what the fifth K block of the V-space kernel can encode
-    (hmax - hmin >= 1 951 004) goes through the legacy kernel, in the same launch as ordinary pairs."""
+    (hmax - hmin >= 1 951 004) goes through the key-space kernel, in the same launch as ordinary pairs."""
     frames = _ragged_frames([300, 280, 310, 290, 520], seed=11)
     frames[1][1][3] = 0
     frames[1][1][7] = 255            # ||t||^2 from 0 to 8 323 200 inside frame 1
@@ -348,7 +363,7 @@ def test_match_largest_frames(engine):
     offs = np.r_[0, np.cumsum(counts)]
     outs = {}
     pq, pt = [1, 2, 3], [0, 1, 2]
-    for v in (0, 5, 7, 8, 9):
+    for v in (0, 5):
         engine.set_option(2, v)
         outs[v] = engine.match(st, pq, pt)
     engine.set_option(2, 0)
@@ -361,6 +376,6 @@ def test_match_largest_frames(engine):
         key = d2.double() * 16384 + torch.arange(nt, device="cuda", dtype=torch.float64)[None, :]
         top = torch.topk(key, 2, dim=1, largest=False).values
         idx = (top % 16384).long(); val = torch.div(top, 16384, rounding_mode="floor").long()
-        for v in (0, 5, 7, 8, 9):
+        for v in (0, 5):
             assert torch.equal(outs[v].top2_idx[ro:ro + nq].long(), idx), (v, p)
             assert torch.equal(outs[v].top2_d2[ro:ro + nq].long(), val), (v, p)
