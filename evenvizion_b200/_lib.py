@@ -33,9 +33,13 @@ SIGNATURES = {
     "evz_filter_matches": [_p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _i, _i, _d, _i, _p, _p, _p, _p, _p, _p, _p],
     "evz_find_homography": [_p, _p, _p, _p, _i, _i, _p, _i, C.c_uint32, _i64, _i, _d, _d, _i,
                             _p, _p, _p, _p, _p, _p, _p, _p, _p],
+    "evz_find_homography_ids": [_p, _p, _p, _p, _i, _i, _p, _i, C.c_uint32, _p, _i, _d, _d, _i,
+                                _p, _p, _p, _p, _p, _p, _p, _p, _p],
     "evz_static_filter": [_p, _p, _p, _p, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p],
     "evz_concat_dedup": [_p, _i, C.POINTER(_p), C.POINTER(_p), C.POINTER(_p), _i, _p, _i, _p, _p, _p, _p],
     "evz_chain_scan": [_p, _p, _p, _i, _i, _p, _p, _p, _p, _p, _p],
+    "evz_chain_scan_segments": [_p, _p, _p, _i, _p, _i, _i, _p, _p, _p],
+    "evz_chain_ref_step": [_p, _p, _p, _i, _i, _i, _p, _p, _p, _p],
     "evz_chain_seed_apply": [_p, _p, _i, _i, _i, _i, _p, _p, _p, _p],
     "evz_remap": [_p, _p, _p, _i64, _p, _i, _d, _d, _i, _p, _p],
     "evz_max_movement": [_p, _p, _i, _i, _i, _p, _p],

@@ -186,14 +186,59 @@ __device__ __forceinline__ M3 m3_shfl_up(const M3& a, int d) {
 
 constexpr int kScanBlock = 256;
 
+// The scan kernels run over one chain (seg_blk = null: block b covers pairs [256 b, 256 b + 256) of n) or over several
+// independent chains (evz_chain_scan_segments): segment s holds pairs [seg_off[s], seg_off[s+1]) and owns the block slots
+// [seg_blk[s], seg_blk[s+1]), one per 256 pairs counted from the segment's own start, so that every block of a segment
+// computes exactly what the one-chain scan of that segment alone computes in the same block.  Indices inside a segment
+// (k, src[]) are segment-relative; `base` turns them into rows of G / S / H_fixed.
+struct ScanBlock { int base, n, blk, slot; };
+// false: a surplus block of the segmented grid (the grid is sized by a host-known bound)
+__device__ __forceinline__ bool scan_block(const int32_t* seg_off, const int32_t* seg_blk, int n_segs, int n, ScanBlock& sb) {
+    const int g = blockIdx.x;
+    if (!seg_blk) { sb.base = 0; sb.n = n; sb.blk = g; sb.slot = g; return true; }
+    if (g >= seg_blk[n_segs]) return false;
+    int lo = 0, hi = n_segs - 1;                                  // last s with seg_blk[s] <= g (a non-empty segment)
+    while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (seg_blk[mid] <= g) lo = mid; else hi = mid - 1; }
+    sb.base = seg_off[lo]; sb.n = seg_off[lo + 1] - seg_off[lo]; sb.blk = g - seg_blk[lo]; sb.slot = g;
+    return true;
+}
+// segmented scan set-up (single CTA): seg_blk[s] = sum over s' < s of ceil(len(s') / 256)
+__global__ void __launch_bounds__(kScanBlock)
+seg_blocks_kernel(const int32_t* __restrict__ seg_off, int n_segs, int32_t* __restrict__ seg_blk) {
+    __shared__ int ws[kScanBlock / 32];
+    __shared__ int carry_s;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    int carry = 0;
+    for (int s0 = 0; s0 < n_segs; s0 += kScanBlock) {
+        const int s = s0 + threadIdx.x;
+        const int nb = s < n_segs ? (seg_off[s + 1] - seg_off[s] + kScanBlock - 1) / kScanBlock : 0;
+        int v = nb;
+#pragma unroll
+        for (int d = 1; d < 32; d <<= 1) { const int t = __shfl_up_sync(0xffffffff, v, d); if (lane >= d) v += t; }
+        if (lane == 31) ws[warp] = v;
+        __syncthreads();
+        int c = carry;
+        for (int w = 0; w < warp; ++w) c += ws[w];
+        if (s < n_segs) seg_blk[s] = c + v - nb;
+        if (threadIdx.x == kScanBlock - 1) carry_s = c + v;
+        __syncthreads();
+        carry = carry_s;
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) seg_blk[n_segs] = carry;
+}
+
 // phase A1: src[k] = index of the last valid pair at or before k within the block (or -1);
 // block_last[b] = last valid index of block b (or -1)
 __global__ void __launch_bounds__(kScanBlock)
-fill_local_kernel(const int32_t* __restrict__ status, int n, int32_t* __restrict__ src, int32_t* __restrict__ block_last) {
+fill_local_kernel(const int32_t* __restrict__ status, int n, int32_t* __restrict__ src, int32_t* __restrict__ block_last,
+                  const int32_t* __restrict__ seg_off, const int32_t* __restrict__ seg_blk, int n_segs) {
     __shared__ int ws[kScanBlock / 32];
-    const int k = blockIdx.x * kScanBlock + threadIdx.x;
+    ScanBlock sb;
+    if (!scan_block(seg_off, seg_blk, n_segs, n, sb)) return;
+    const int k = sb.blk * kScanBlock + threadIdx.x;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    int v = (k < n && status[k] == EVZ_ST_OK) ? k : -1;
+    int v = (k < sb.n && status[sb.base + k] == EVZ_ST_OK) ? k : -1;
 #pragma unroll
     for (int d = 1; d < 32; d <<= 1) { const int t = __shfl_up_sync(0xffffffff, v, d); if (lane >= d) v = max(v, t); }
     if (lane == 31) ws[warp] = v;
@@ -201,35 +246,43 @@ fill_local_kernel(const int32_t* __restrict__ status, int n, int32_t* __restrict
     int carry = -1;
     for (int w = 0; w < warp; ++w) carry = max(carry, ws[w]);
     v = max(v, carry);
-    if (k < n) src[k] = v;
-    if (threadIdx.x == kScanBlock - 1) block_last[blockIdx.x] = v;
+    if (k < sb.n) src[sb.base + k] = v;
+    if (threadIdx.x == kScanBlock - 1) block_last[sb.slot] = v;
 }
-// phase A2 (single CTA): running max over block_last -> block_carry[b] = last valid before block b
-__global__ void fill_carry_kernel(const int32_t* __restrict__ block_last, int nb, int32_t* __restrict__ block_carry) {
+// phase A2 (one CTA per segment): running max over block_last -> block_carry[b] = last valid before block b
+__global__ void fill_carry_kernel(const int32_t* __restrict__ block_last, int nb, int32_t* __restrict__ block_carry,
+                                  const int32_t* __restrict__ seg_blk) {
     if (threadIdx.x == 0) {
+        const int b0 = seg_blk ? seg_blk[blockIdx.x] : 0, b1 = seg_blk ? seg_blk[blockIdx.x + 1] : nb;
         int c = -1;
-        for (int b = 0; b < nb; ++b) { block_carry[b] = c; c = max(c, block_last[b]); }
+        for (int b = b0; b < b1; ++b) { block_carry[b] = c; c = max(c, block_last[b]); }
     }
 }
 // phase A3: fold the cross-block carry into src
 __global__ void __launch_bounds__(kScanBlock)
-fill_apply_kernel(int32_t* __restrict__ src, const int32_t* __restrict__ block_carry, int n) {
-    const int k = blockIdx.x * kScanBlock + threadIdx.x;
-    if (k < n) src[k] = max(src[k], block_carry[blockIdx.x]);
+fill_apply_kernel(int32_t* __restrict__ src, const int32_t* __restrict__ block_carry, int n,
+                  const int32_t* __restrict__ seg_off, const int32_t* __restrict__ seg_blk, int n_segs) {
+    ScanBlock sb;
+    if (!scan_block(seg_off, seg_blk, n_segs, n, sb)) return;
+    const int k = sb.blk * kScanBlock + threadIdx.x;
+    if (k < sb.n) src[sb.base + k] = max(src[sb.base + k], block_carry[sb.slot]);
 }
 // phase B1: Gf[k] = filled step matrix; local inclusive product scan; block totals
 __global__ void __launch_bounds__(kScanBlock)
 prod_local_kernel(const double* __restrict__ G, const int32_t* __restrict__ src,
                   int n, int policy, const double* __restrict__ seed_G,
-                  double* __restrict__ S, double* __restrict__ block_tot) {
+                  double* __restrict__ S, double* __restrict__ block_tot,
+                  const int32_t* __restrict__ seg_off, const int32_t* __restrict__ seg_blk, int n_segs) {
     __shared__ double wt[kScanBlock / 32][9];
-    const int k = blockIdx.x * kScanBlock + threadIdx.x;
+    ScanBlock sb;
+    if (!scan_block(seg_off, seg_blk, n_segs, n, sb)) return;
+    const int k = sb.blk * kScanBlock + threadIdx.x;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     M3 v = m3_identity();
-    if (k < n) {
-        int s = src[k];
+    if (k < sb.n) {
+        int s = src[sb.base + k];
         if (policy == 0 && s != k) s = -2;                       // identity step for an invalid pair
-        if (s >= 0) v = m3_load(G + static_cast<size_t>(s) * 9);
+        if (s >= 0) v = m3_load(G + static_cast<size_t>(sb.base + s) * 9);
         else if (s == -1 && policy != 0 && seed_G) v = m3_load(seed_G);
     }
 #pragma unroll
@@ -244,17 +297,23 @@ prod_local_kernel(const double* __restrict__ G, const int32_t* __restrict__ src,
         for (int w = 1; w < warp; ++w) c = m3_mul_scaled(c, m3_load(wt[w]));
         v = m3_mul_scaled(c, v);
     }
-    if (k < n) m3_store(S + static_cast<size_t>(k) * 9, m3_norm22(v));         // a true prefix of the (shard's) chain
-    if (threadIdx.x == kScanBlock - 1) m3_store(block_tot + static_cast<size_t>(blockIdx.x) * 9, v);
+    if (k < sb.n) m3_store(S + static_cast<size_t>(sb.base + k) * 9, m3_norm22(v));   // a true prefix of the (shard's) chain
+    if (threadIdx.x == kScanBlock - 1) m3_store(block_tot + static_cast<size_t>(sb.slot) * 9, v);
 }
-// phase B2 (single CTA): exclusive prefix of the block totals, seeded.  Block-wide shuffle scan over
+// phase B2 (one CTA per segment): exclusive prefix of the block totals, seeded.  Block-wide shuffle scan over
 // chunks of kScanBlock totals (a serial loop over blocks costs ~1 us per block: L2 latency + f64 divides)
 __global__ void __launch_bounds__(kScanBlock)
 prod_carry_kernel(const double* __restrict__ block_tot, int nb, const double* __restrict__ seed_S,
-                  double* __restrict__ block_pre) {
+                  double* __restrict__ block_pre, const int32_t* __restrict__ seg_blk) {
     __shared__ double wt[kScanBlock / 32][9];
     __shared__ double carry_s[9];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (seg_blk) {
+        const int b0 = seg_blk[blockIdx.x];
+        nb = seg_blk[blockIdx.x + 1] - b0;
+        block_tot += static_cast<size_t>(b0) * 9;
+        block_pre += static_cast<size_t>(b0) * 9;
+    }
     M3 carry = seed_S ? m3_load(seed_S) : m3_identity();
     for (int b0 = 0; b0 < nb; b0 += kScanBlock) {
         const int b = b0 + threadIdx.x;
@@ -281,19 +340,57 @@ prod_carry_kernel(const double* __restrict__ block_tot, int nb, const double* __
 }
 // phase B3: S[k] = block_pre[b] . S_local[k]
 __global__ void __launch_bounds__(kScanBlock)
-prod_apply_kernel(double* __restrict__ S, const double* __restrict__ block_pre, int n, int has_seed) {
-    const int k = blockIdx.x * kScanBlock + threadIdx.x;
-    if (k >= n || (blockIdx.x == 0 && !has_seed)) return;
-    const M3 r = m3_mul_norm(m3_load(block_pre + static_cast<size_t>(blockIdx.x) * 9), m3_load(S + static_cast<size_t>(k) * 9));
-    m3_store(S + static_cast<size_t>(k) * 9, r);
+prod_apply_kernel(double* __restrict__ S, const double* __restrict__ block_pre, int n, int has_seed,
+                  const int32_t* __restrict__ seg_off, const int32_t* __restrict__ seg_blk, int n_segs) {
+    ScanBlock sb;
+    if (!scan_block(seg_off, seg_blk, n_segs, n, sb)) return;
+    const int k = sb.blk * kScanBlock + threadIdx.x;
+    if (k >= sb.n || (sb.blk == 0 && !has_seed)) return;
+    double* Sk = S + static_cast<size_t>(sb.base + k) * 9;
+    m3_store(Sk, m3_mul_norm(m3_load(block_pre + static_cast<size_t>(sb.slot) * 9), m3_load(Sk)));
 }
 // H_fixed[k] = normalise(S[k] . S[k-1]^-1)
 __global__ void __launch_bounds__(kScanBlock)
-fixed_plane_kernel(const double* __restrict__ S, const double* __restrict__ seed_S, int n, double* __restrict__ Hf) {
-    const int k = blockIdx.x * kScanBlock + threadIdx.x;
-    if (k >= n) return;
-    const M3 prev = k > 0 ? m3_load(S + static_cast<size_t>(k - 1) * 9) : (seed_S ? m3_load(seed_S) : m3_identity());
-    m3_store(Hf + static_cast<size_t>(k) * 9, m3_mul_norm(m3_load(S + static_cast<size_t>(k) * 9), m3_inverse(prev)));
+fixed_plane_kernel(const double* __restrict__ S, const double* __restrict__ seed_S, int n, double* __restrict__ Hf,
+                   const int32_t* __restrict__ seg_off, const int32_t* __restrict__ seg_blk, int n_segs) {
+    ScanBlock sb;
+    if (!scan_block(seg_off, seg_blk, n_segs, n, sb)) return;
+    const int k = sb.blk * kScanBlock + threadIdx.x;
+    if (k >= sb.n) return;
+    const double* Sk = S + static_cast<size_t>(sb.base + k) * 9;
+    const M3 prev = k > 0 ? m3_load(Sk - 9) : (seed_S ? m3_load(seed_S) : m3_identity());
+    m3_store(Hf + static_cast<size_t>(sb.base + k) * 9, m3_mul_norm(m3_load(Sk), m3_inverse(prev)));
+}
+
+// Reference-exact chain step (video_processing.py:119-149 on the device), one thread per chain c:
+//   H = H2[c] if status[c] == EVZ_ST_OK, else H_prev[c] if policy and not first, else the identity;  H_out[c] = H;
+//   S_state[c] = H if first, else C / C[2][2] with C = H . S_state[c].
+// The product uses one fixed operation order, fma(H[i][2], S[2][j], fma(H[i][1], S[1][j], H[i][0] * S[0][j])), followed by
+// an IEEE division: the order in which NumPy's np.dot (OpenBLAS dgemm) forms a 3x3 f64 product, so the device chain
+// follows the host loop bit for bit wherever the host's BLAS does the same.  H_prev may alias H_out (each thread reads
+// its own row before it writes it).
+__global__ void __launch_bounds__(kScanBlock)
+chain_ref_step_kernel(const double* __restrict__ H2, const int32_t* __restrict__ status, int n, int first, int policy,
+                      double* __restrict__ S_state, const double* H_prev, double* H_out) {
+    const int c = blockIdx.x * kScanBlock + threadIdx.x;
+    if (c >= n) return;
+    M3 H;
+    if (status[c] == EVZ_ST_OK) H = m3_load(H2 + static_cast<size_t>(c) * 9);
+    else if (policy && !first) H = m3_load(H_prev + static_cast<size_t>(c) * 9);
+    else H = m3_identity();
+    m3_store(H_out + static_cast<size_t>(c) * 9, H);
+    double* Sc = S_state + static_cast<size_t>(c) * 9;
+    if (first) { m3_store(Sc, H); return; }
+    const M3 S = m3_load(Sc);
+    M3 R;
+#pragma unroll
+    for (int i = 0; i < 3; ++i)
+#pragma unroll
+        for (int j = 0; j < 3; ++j)
+            R.m[3 * i + j] = __fma_rn(H.m[3 * i + 2], S.m[6 + j], __fma_rn(H.m[3 * i + 1], S.m[3 + j], __dmul_rn(H.m[3 * i], S.m[j])));
+    const double d = R.m[8];
+#pragma unroll
+    for (int i = 0; i < 9; ++i) Sc[i] = __ddiv_rn(R.m[i], d);
 }
 // shard summary for the cross-GPU all-gather (see evz.h)
 __global__ void summary_kernel(const double* __restrict__ G, const int32_t* __restrict__ src, const double* __restrict__ S_noseed_tot,
@@ -450,20 +547,20 @@ extern "C" int evz_chain_scan(evz_handle* h, const double* G, const int32_t* sta
     double* block_pre = reinterpret_cast<double*>(b); b += evz_align_up(static_cast<size_t>(nb) * 72, 256);
     double* S_work = S ? S : reinterpret_cast<double*>(b);
 
-    evz::fill_local_kernel<<<nb, evz::kScanBlock, 0, st>>>(status, n_pairs, src, block_last);
+    evz::fill_local_kernel<<<nb, evz::kScanBlock, 0, st>>>(status, n_pairs, src, block_last, nullptr, nullptr, 0);
     EVZ_LAUNCH_CHECK(h);
-    evz::fill_carry_kernel<<<1, 32, 0, st>>>(block_last, nb, block_carry);
+    evz::fill_carry_kernel<<<1, 32, 0, st>>>(block_last, nb, block_carry, nullptr);
     EVZ_LAUNCH_CHECK(h);
-    evz::fill_apply_kernel<<<nb, evz::kScanBlock, 0, st>>>(src, block_carry, n_pairs);
+    evz::fill_apply_kernel<<<nb, evz::kScanBlock, 0, st>>>(src, block_carry, n_pairs, nullptr, nullptr, 0);
     EVZ_LAUNCH_CHECK(h);
     const bool seeded = seed_S != nullptr || seed_G != nullptr;
     if (summary || (S && !seeded)) {
         // unseeded pass: leading invalid pairs are identity steps, so the total is R
-        evz::prod_local_kernel<<<nb, evz::kScanBlock, 0, st>>>(G, src, n_pairs, policy, nullptr, S_work, block_tot);
+        evz::prod_local_kernel<<<nb, evz::kScanBlock, 0, st>>>(G, src, n_pairs, policy, nullptr, S_work, block_tot, nullptr, nullptr, 0);
         EVZ_LAUNCH_CHECK(h);
-        evz::prod_carry_kernel<<<1, evz::kScanBlock, 0, st>>>(block_tot, nb, nullptr, block_pre);
+        evz::prod_carry_kernel<<<1, evz::kScanBlock, 0, st>>>(block_tot, nb, nullptr, block_pre, nullptr);
         EVZ_LAUNCH_CHECK(h);
-        evz::prod_apply_kernel<<<nb, evz::kScanBlock, 0, st>>>(S_work, block_pre, n_pairs, 0);
+        evz::prod_apply_kernel<<<nb, evz::kScanBlock, 0, st>>>(S_work, block_pre, n_pairs, 0, nullptr, nullptr, 0);
         EVZ_LAUNCH_CHECK(h);
         if (summary) {
             evz::summary_kernel<<<1, 32, 0, st>>>(G, src, S_work + static_cast<size_t>(n_pairs - 1) * 9, n_pairs, summary);
@@ -471,17 +568,76 @@ extern "C" int evz_chain_scan(evz_handle* h, const double* G, const int32_t* sta
         }
     }
     if (S && seeded) {
-        evz::prod_local_kernel<<<nb, evz::kScanBlock, 0, st>>>(G, src, n_pairs, policy, seed_G, S, block_tot);
+        evz::prod_local_kernel<<<nb, evz::kScanBlock, 0, st>>>(G, src, n_pairs, policy, seed_G, S, block_tot, nullptr, nullptr, 0);
         EVZ_LAUNCH_CHECK(h);
-        evz::prod_carry_kernel<<<1, evz::kScanBlock, 0, st>>>(block_tot, nb, seed_S, block_pre);
+        evz::prod_carry_kernel<<<1, evz::kScanBlock, 0, st>>>(block_tot, nb, seed_S, block_pre, nullptr);
         EVZ_LAUNCH_CHECK(h);
-        evz::prod_apply_kernel<<<nb, evz::kScanBlock, 0, st>>>(S, block_pre, n_pairs, seed_S ? 1 : 0);
+        evz::prod_apply_kernel<<<nb, evz::kScanBlock, 0, st>>>(S, block_pre, n_pairs, seed_S ? 1 : 0, nullptr, nullptr, 0);
         EVZ_LAUNCH_CHECK(h);
     }
     if (S && H_fixed) {
-        evz::fixed_plane_kernel<<<nb, evz::kScanBlock, 0, st>>>(S, seed_S, n_pairs, H_fixed);
+        evz::fixed_plane_kernel<<<nb, evz::kScanBlock, 0, st>>>(S, seed_S, n_pairs, H_fixed, nullptr, nullptr, 0);
         EVZ_LAUNCH_CHECK(h);
     }
+    return EVZ_OK;
+}
+
+extern "C" int evz_chain_scan_segments(evz_handle* h, const double* G, const int32_t* status, int n_pairs,
+                                       const int32_t* seg_off, int n_segs, int policy, double* S, double* H_fixed, void* stream) {
+    if (!h) return EVZ_E_ARG;
+    EVZ_ENTER(h);
+    EVZ_REQUIRE(h, G && status && seg_off && S, "null pointer");
+    EVZ_REQUIRE(h, n_segs >= 0, "n_segs must not be negative");
+    if (n_pairs <= 0 || n_segs == 0) return EVZ_OK;
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    // host-known bound of the block slots: sum over s of ceil(len(s) / 256) <= ceil(n_pairs / 256) + n_segs
+    const int nb = (n_pairs + evz::kScanBlock - 1) / evz::kScanBlock + n_segs;
+    // scratch: src[n] | block_last[nb] | block_carry[nb] | block_tot[nb*9] | block_pre[nb*9] | seg_blk[n_segs+1]
+    const size_t need = evz_align_up(static_cast<size_t>(n_pairs) * 4, 256) + 2 * evz_align_up(static_cast<size_t>(nb) * 4, 256) +
+                        2 * evz_align_up(static_cast<size_t>(nb) * 72, 256) + evz_align_up(static_cast<size_t>(n_segs + 1) * 4, 256) + 256;
+    void* scr = nullptr;
+    int rc = evz_scratch(h, need, &scr);
+    if (rc) return rc;
+    uint8_t* b = static_cast<uint8_t*>(scr);
+    int32_t* src = reinterpret_cast<int32_t*>(b); b += evz_align_up(static_cast<size_t>(n_pairs) * 4, 256);
+    int32_t* block_last = reinterpret_cast<int32_t*>(b); b += evz_align_up(static_cast<size_t>(nb) * 4, 256);
+    int32_t* block_carry = reinterpret_cast<int32_t*>(b); b += evz_align_up(static_cast<size_t>(nb) * 4, 256);
+    double* block_tot = reinterpret_cast<double*>(b); b += evz_align_up(static_cast<size_t>(nb) * 72, 256);
+    double* block_pre = reinterpret_cast<double*>(b); b += evz_align_up(static_cast<size_t>(nb) * 72, 256);
+    int32_t* seg_blk = reinterpret_cast<int32_t*>(b);
+
+    evz::seg_blocks_kernel<<<1, evz::kScanBlock, 0, st>>>(seg_off, n_segs, seg_blk);
+    EVZ_LAUNCH_CHECK(h);
+    evz::fill_local_kernel<<<nb, evz::kScanBlock, 0, st>>>(status, n_pairs, src, block_last, seg_off, seg_blk, n_segs);
+    EVZ_LAUNCH_CHECK(h);
+    evz::fill_carry_kernel<<<n_segs, 32, 0, st>>>(block_last, nb, block_carry, seg_blk);
+    EVZ_LAUNCH_CHECK(h);
+    evz::fill_apply_kernel<<<nb, evz::kScanBlock, 0, st>>>(src, block_carry, n_pairs, seg_off, seg_blk, n_segs);
+    EVZ_LAUNCH_CHECK(h);
+    evz::prod_local_kernel<<<nb, evz::kScanBlock, 0, st>>>(G, src, n_pairs, policy, nullptr, S, block_tot, seg_off, seg_blk, n_segs);
+    EVZ_LAUNCH_CHECK(h);
+    evz::prod_carry_kernel<<<n_segs, evz::kScanBlock, 0, st>>>(block_tot, nb, nullptr, block_pre, seg_blk);
+    EVZ_LAUNCH_CHECK(h);
+    evz::prod_apply_kernel<<<nb, evz::kScanBlock, 0, st>>>(S, block_pre, n_pairs, 0, seg_off, seg_blk, n_segs);
+    EVZ_LAUNCH_CHECK(h);
+    if (H_fixed) {
+        evz::fixed_plane_kernel<<<nb, evz::kScanBlock, 0, st>>>(S, nullptr, n_pairs, H_fixed, seg_off, seg_blk, n_segs);
+        EVZ_LAUNCH_CHECK(h);
+    }
+    return EVZ_OK;
+}
+
+extern "C" int evz_chain_ref_step(evz_handle* h, const double* H2, const int32_t* status, int n_chains, int first, int policy,
+                                  double* S_state, const double* H_prev, double* H_out, void* stream) {
+    if (!h) return EVZ_E_ARG;
+    EVZ_ENTER(h);
+    EVZ_REQUIRE(h, H2 && status && S_state && H_out, "null pointer");
+    EVZ_REQUIRE(h, first || !policy || H_prev, "null pointer (H_prev is required after the first step when policy = 1)");
+    if (n_chains <= 0) return EVZ_OK;
+    const int nb = (n_chains + evz::kScanBlock - 1) / evz::kScanBlock;
+    evz::chain_ref_step_kernel<<<nb, evz::kScanBlock, 0, static_cast<cudaStream_t>(stream)>>>(H2, status, n_chains, first ? 1 : 0,
+                                                                                             policy ? 1 : 0, S_state, H_prev, H_out);
+    EVZ_LAUNCH_CHECK(h);
     return EVZ_OK;
 }
 
@@ -499,7 +655,7 @@ extern "C" int evz_chain_seed_apply(evz_handle* h, const double* summaries, int 
     evz::seed_apply_kernel<<<nb, evz::kScanBlock, 0, st>>>(S, summaries, rank, seeds_out, n_pairs);
     EVZ_LAUNCH_CHECK(h);
     if (H_fixed) {
-        evz::fixed_plane_kernel<<<nb, evz::kScanBlock, 0, st>>>(S, seeds_out, n_pairs, H_fixed);
+        evz::fixed_plane_kernel<<<nb, evz::kScanBlock, 0, st>>>(S, seeds_out, n_pairs, H_fixed, nullptr, nullptr, 0);
         EVZ_LAUNCH_CHECK(h);
     }
     return EVZ_OK;

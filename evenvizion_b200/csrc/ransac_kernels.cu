@@ -141,6 +141,7 @@ struct FhArgs {
     int exact_only;
     int no_prune;
     float4* hcache;     // [n_pairs][n_hyp][2] f32 models of the hypotheses that passed pass 0 (null: solved again where needed)
+    const int64_t* pair_ids;   // [n_pairs] sampler id of every pair (null: pair_id_base + p)
 };
 
 // 8x8 symmetric positive-definite system through an LDL^T factorisation held in registers
@@ -737,7 +738,7 @@ ransac_score_kernel(const FhArgs a, double* __restrict__ Hbest_out, int32_t* __r
 #pragma unroll
     for (int w = 0; w < kRsThreads / 32; ++w) cmax = fmaxf(cmax, cmax_s[w]);
 
-    const uint32_t pair_level = static_cast<uint32_t>((a.pair_id_base + p) * 2 + a.level);
+    const uint32_t pair_level = static_cast<uint32_t>((a.pair_ids ? a.pair_ids[p] : a.pair_id_base + p) * 2 + a.level);
     if (m == 4) {
         // findHomography: npoints == 4 -> exact model through the 4 points, mask = ones, no LM
         if (tid == 0) {
@@ -1210,19 +1211,20 @@ ransac_refit_kernel(const FhArgs a, const double* __restrict__ Hbest_in, const i
 
 }  // namespace evz
 
-extern "C" int evz_find_homography(evz_handle* h, const float* pts, const int32_t* off, const int32_t* cnt, int n_pairs,
-                                   int max_cnt, const double* pre_H, int n_hyp, uint32_t seed, int64_t pair_id_base, int level,
-                                   double thresh, double min_inlier_frac, int fail_status,
-                                   int32_t* status, double* H, uint8_t* mask, int32_t* inl_cnt,
-                                   int32_t* best_hyp, int32_t* best_cnt, uint8_t* mask_best, double* H_best,
-                                   void* stream) {
-    if (!h) return EVZ_E_ARG;
-    EVZ_ENTER(h);
-    EVZ_REQUIRE(h, pts && off && cnt && status && H, "null pointer");
-    EVZ_REQUIRE(h, n_hyp > 0, "n_hyp must be positive");
-    EVZ_REQUIRE(h, (reinterpret_cast<uintptr_t>(pts) & 15) == 0, "pts must be 16-byte aligned");
+// evz_find_homography (pair_ids = null) and evz_find_homography_ids (pair_ids set): the kernels are shared, the only
+// difference is the sampler id of pair p (FhArgs::pair_ids).  `fn` names the entry point in the error text.
+#define FH_REQUIRE(cond, msg) do { if (!(cond)) { EVZ_SET_ERR(h, "%s: %s", fn, msg); return EVZ_E_ARG; } } while (0)
+static int find_homography(const char* fn, evz_handle* h, const float* pts, const int32_t* off, const int32_t* cnt, int n_pairs,
+                           int max_cnt, const double* pre_H, int n_hyp, uint32_t seed, int64_t pair_id_base,
+                           const int64_t* pair_ids, int level, double thresh, double min_inlier_frac, int fail_status,
+                           int32_t* status, double* H, uint8_t* mask, int32_t* inl_cnt,
+                           int32_t* best_hyp, int32_t* best_cnt, uint8_t* mask_best, double* H_best,
+                           void* stream) {
+    FH_REQUIRE(pts && off && cnt && status && H, "null pointer");
+    FH_REQUIRE(n_hyp > 0, "n_hyp must be positive");
+    FH_REQUIRE((reinterpret_cast<uintptr_t>(pts) & 15) == 0, "pts must be 16-byte aligned");
     if (max_cnt > EVZ_MAX_KP) {
-        EVZ_SET_ERR(h, "evz_find_homography: max_cnt %d exceeds the supported %d points per pair", max_cnt, EVZ_MAX_KP);
+        EVZ_SET_ERR(h, "%s: max_cnt %d exceeds the supported %d points per pair", fn, max_cnt, EVZ_MAX_KP);
         return EVZ_E_UNSUPPORTED;
     }
     if (n_pairs <= 0) return EVZ_OK;
@@ -1240,7 +1242,7 @@ extern "C" int evz_find_homography(evz_handle* h, const float* pts, const int32_
     int32_t* phase = static_cast<int32_t*>(scr);
     double* hb = H_best ? H_best : reinterpret_cast<double*>(static_cast<uint8_t*>(scr) + ph_bytes);
     float4* hcache = hc_bytes ? reinterpret_cast<float4*>(static_cast<uint8_t*>(scr) + ph_bytes + hb_bytes) : nullptr;
-    EVZ_REQUIRE(h, n_hyp <= 65535, "n_hyp must be below 65536");
+    FH_REQUIRE(n_hyp <= 65535, "n_hyp must be below 65536");
     const int smem_score = max_cnt * 16 + ((max_cnt + 7) & ~7) * 2 + 8 * n_hyp + 16;
     const int smem_refit = max_cnt * 17 + 16;
     if (smem_score > h->attr_score) {
@@ -1253,10 +1255,37 @@ extern "C" int evz_find_homography(evz_handle* h, const float* pts, const int32_
     }
     const float t = static_cast<float>(thresh * thresh);
     evz::FhArgs a{pts, off, cnt, pre_H, n_hyp, seed, pair_id_base, level, t, min_inlier_frac, fail_status,
-                  status, H, mask, inl_cnt, best_hyp, best_cnt, mask_best, H_best, max_cnt, h->opt_ransac_exact, h->opt_ransac_no_prune, hcache};
+                  status, H, mask, inl_cnt, best_hyp, best_cnt, mask_best, H_best, max_cnt, h->opt_ransac_exact, h->opt_ransac_no_prune, hcache,
+                  pair_ids};
     evz::ransac_score_kernel<<<n_pairs, evz::kRsThreads, smem_score, st>>>(a, hb, phase);
     EVZ_LAUNCH_CHECK(h);
     evz::ransac_refit_kernel<<<n_pairs, evz::kRfThreads, smem_refit, st>>>(a, hb, phase);
     EVZ_LAUNCH_CHECK(h);
     return EVZ_OK;
+}
+#undef FH_REQUIRE
+
+extern "C" int evz_find_homography(evz_handle* h, const float* pts, const int32_t* off, const int32_t* cnt, int n_pairs,
+                                   int max_cnt, const double* pre_H, int n_hyp, uint32_t seed, int64_t pair_id_base, int level,
+                                   double thresh, double min_inlier_frac, int fail_status,
+                                   int32_t* status, double* H, uint8_t* mask, int32_t* inl_cnt,
+                                   int32_t* best_hyp, int32_t* best_cnt, uint8_t* mask_best, double* H_best,
+                                   void* stream) {
+    if (!h) return EVZ_E_ARG;
+    EVZ_ENTER(h);
+    return find_homography(__func__, h, pts, off, cnt, n_pairs, max_cnt, pre_H, n_hyp, seed, pair_id_base, nullptr, level, thresh,
+                           min_inlier_frac, fail_status, status, H, mask, inl_cnt, best_hyp, best_cnt, mask_best, H_best, stream);
+}
+
+extern "C" int evz_find_homography_ids(evz_handle* h, const float* pts, const int32_t* off, const int32_t* cnt, int n_pairs,
+                                       int max_cnt, const double* pre_H, int n_hyp, uint32_t seed, const int64_t* pair_id,
+                                       int level, double thresh, double min_inlier_frac, int fail_status,
+                                       int32_t* status, double* H, uint8_t* mask, int32_t* inl_cnt,
+                                       int32_t* best_hyp, int32_t* best_cnt, uint8_t* mask_best, double* H_best,
+                                       void* stream) {
+    if (!h) return EVZ_E_ARG;
+    EVZ_ENTER(h);
+    EVZ_REQUIRE(h, pair_id, "null pointer");
+    return find_homography(__func__, h, pts, off, cnt, n_pairs, max_cnt, pre_H, n_hyp, seed, 0, pair_id, level, thresh,
+                           min_inlier_frac, fail_status, status, H, mask, inl_cnt, best_hyp, best_cnt, mask_best, H_best, stream);
 }

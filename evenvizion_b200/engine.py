@@ -220,10 +220,12 @@ class GeometryEngine:
 
     # ------------------------------------------------------------------ K3 / K4
     def find_homography(self, pts, off, cnt, status, max_cnt, n_hyp=1024, seed=0, pair_id_base=0, level=1,
-                        thresh=3.0, min_inlier_frac=0.0, fail_status=_lib.ST_NO_MODEL_1, pre_H=None, light=False):
+                        thresh=3.0, min_inlier_frac=0.0, fail_status=_lib.ST_NO_MODEL_1, pre_H=None, light=False,
+                        pair_ids=None):
         """Batched seeded RANSAC + LM refit over the point lists pts[off[p]:off[p]+cnt[p]].
         status is updated in place.  Returns dict(H, mask, inl_cnt, best_hyp, best_cnt, mask_best, H_best);
-        light=True skips the per-point masks and the diagnostics (H and inl_cnt only)."""
+        light=True skips the per-point masks and the diagnostics (H and inl_cnt only).
+        pair_ids: int64 [P] device tensor of sampler ids (pair p is seeded with pair_ids[p] instead of pair_id_base + p)."""
         P = int(cnt.numel())
         rows = int(pts.shape[0])
         z = lambda shape, dt: torch.zeros(shape, dtype=dt, device=self.device)
@@ -233,12 +235,16 @@ class GeometryEngine:
         else:
             out.update(mask=z((rows,), torch.uint8), best_hyp=torch.full((P,), -1, dtype=torch.int32, device=self.device),
                        best_cnt=z((P,), torch.int32), mask_best=z((rows,), torch.uint8), H_best=z((P, 9), torch.float64))
-        self._check(self.lib.evz_find_homography(self.h, _ptr(pts), _ptr(off), _ptr(cnt), P, int(max_cnt), _ptr(pre_H),
-                                                 int(n_hyp), int(seed) & 0xFFFFFFFF, int(pair_id_base), int(level),
-                                                 float(thresh), float(min_inlier_frac), int(fail_status),
-                                                 _ptr(status), _ptr(out["H"]), _ptr(out["mask"]), _ptr(out["inl_cnt"]),
-                                                 _ptr(out["best_hyp"]), _ptr(out["best_cnt"]), _ptr(out["mask_best"]),
-                                                 _ptr(out["H_best"]), self._stream()))
+        if pair_ids is not None:
+            fn, ids = self.lib.evz_find_homography_ids, _ptr(pair_ids)
+        else:
+            fn, ids = self.lib.evz_find_homography, int(pair_id_base)
+        self._check(fn(self.h, _ptr(pts), _ptr(off), _ptr(cnt), P, int(max_cnt), _ptr(pre_H),
+                       int(n_hyp), int(seed) & 0xFFFFFFFF, ids, int(level),
+                       float(thresh), float(min_inlier_frac), int(fail_status),
+                       _ptr(status), _ptr(out["H"]), _ptr(out["mask"]), _ptr(out["inl_cnt"]),
+                       _ptr(out["best_hyp"]), _ptr(out["best_cnt"]), _ptr(out["mask_best"]),
+                       _ptr(out["H_best"]), self._stream()))
         return out
 
     # ------------------------------------------------------------------ K5
@@ -309,6 +315,56 @@ class GeometryEngine:
         elif summ is not None:       # an empty shard: identity product, no valid pair
             summ.copy_(torch.tensor([1, 0, 0, 0, 1, 0, 0, 0, 1] * 2 + [0, 0], dtype=torch.float64))
         return S, Hf, summ
+
+    def chain_scan_segments(self, G, status, seg_off, policy=True):
+        """`chain_scan` (no seeds) restarted at every segment: segment s = pairs [seg_off[s], seg_off[s+1]) of G / status,
+        seg_off an int32 [n_segs+1] device tensor.  Returns (S, H_fixed), both [P,9]."""
+        G = G.reshape(-1, 9).contiguous()
+        P = G.shape[0]
+        S = self._empty((P, 9), torch.float64)
+        Hf = self._empty((P, 9), torch.float64)
+        self._check(self.lib.evz_chain_scan_segments(self.h, _ptr(G), _ptr(status), P, _ptr(seg_off), int(seg_off.numel()) - 1,
+                                                     1 if policy else 0, _ptr(S), _ptr(Hf), self._stream()))
+        return S, Hf
+
+    def chain_ref_step(self, H2, status, first, policy, S_state, H_prev, H_out):
+        """One reference-exact chain step for the first n = len(status) chains (include/evz.h, evz_chain_ref_step):
+        writes H_out[:n] and advances S_state[:n] in place.  H_prev: the previous step's H_out (None on the first step)."""
+        self._check(self.lib.evz_chain_ref_step(self.h, _ptr(H2), _ptr(status), int(status.numel()), 1 if first else 0,
+                                                1 if policy else 0, _ptr(S_state), _ptr(H_prev), _ptr(H_out), self._stream()))
+
+    def reference_chains(self, pts, off, cnt, status, max_cnt, step_off, n_hyp=1024, seed=0, policy=True, thresh=3.0,
+                         min_inlier_frac=0.7, fail_status=_lib.ST_NO_MODEL_2):
+        """RANSAC #2 of the reference-exact chain (video_processing.py:67-105) for several videos in lockstep.
+
+        The pairs are in step-major order: step k is pairs [step_off[k], step_off[k+1]) = pair k of chains 0 .. n_k - 1,
+        with n_0 >= n_1 >= ... (chains ordered by length, longest first), so the chains still running are a prefix.
+        Step k is one RANSAC launch over its pairs, seeded with id k and pre-transformed by every chain's running
+        superposition, then one evz_chain_ref_step.  The outputs are allocated before the loop and the loop neither
+        allocates nor synchronises with the host.  status is updated in place; returns H_out [P,9]: the matrix the
+        reference stores for every pair, after the None-H policy."""
+        step_off = np.asarray(step_off, np.int64)
+        K = len(step_off) - 1
+        P = int(cnt.numel())
+        H2 = torch.zeros((P, 9), dtype=torch.float64, device=self.device)
+        H_out = self._empty((P, 9), torch.float64)
+        inl = torch.zeros((P,), dtype=torch.int32, device=self.device)
+        S_state = self._empty((int(step_off[1] - step_off[0]) if K else 0, 9), torch.float64)
+        # pinned + non_blocking: the set-up does not synchronise with the host either
+        ids = torch.from_numpy(np.repeat(np.arange(K, dtype=np.int64), np.diff(step_off))).pin_memory()
+        ids = ids.to(self.device, non_blocking=True)
+        lib, h, strm = self.lib, self.h, self._stream()
+        at = lambda t, p0, k=1: C.c_void_p(t.data_ptr() + int(p0) * k * t.element_size())
+        for k in range(len(step_off) - 1):
+            a, b = int(step_off[k]), int(step_off[k + 1])
+            self._check(lib.evz_find_homography_ids(h, _ptr(pts), at(off, a), at(cnt, a), b - a, int(max_cnt),
+                                                    None if k == 0 else _ptr(S_state), int(n_hyp), int(seed) & 0xFFFFFFFF,
+                                                    at(ids, a), 2, float(thresh), float(min_inlier_frac), int(fail_status),
+                                                    at(status, a), at(H2, a, 9), None, at(inl, a), None, None, None, None, strm))
+            self._check(lib.evz_chain_ref_step(h, at(H2, a, 9), at(status, a), b - a, 1 if k == 0 else 0, 1 if policy else 0,
+                                               _ptr(S_state), None if k == 0 else at(H_out, step_off[k - 1], 9), at(H_out, a, 9),
+                                               strm))
+        return H_out
 
     def chain_seed_apply(self, summaries, rank, S, policy=True, want_fixed=True):
         """Turn this rank's unseeded local scan S ([P,9], in place) into its slice of the global scan, given the

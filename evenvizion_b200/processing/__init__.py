@@ -10,5 +10,6 @@ from .utils import (HomographyException, remove_double_matching, homography_tran
                     inverse_homography_transformation, matrix_superposition, read_homography_dict,
                     superposition_dict, are_infinity_coordinates, read_json_with_coordinates,
                     get_largest_group_points, find_point_displacement, compute_homography)
-from .video_processing import get_homography_dict, geometry_from_features, read_and_describe       # noqa: F401
+from .video_processing import (get_homography_dict, get_homography_dicts, geometry_from_features,      # noqa: F401
+                               geometry_from_features_batch, read_and_describe)
 from .formats import dump_homography_dict, load_homography_arrays, dump_coordinates, load_coordinates_arrays   # noqa: F401

@@ -61,15 +61,7 @@ def geometry_from_features(feats, none_H_processing=True, mode="reference", n_hy
     status = torch.zeros(P, dtype=torch.int32, device=dev)
     per_type = []
     for t in types:
-        frames = feats[t]
-        if any(d is None for _, d in frames):
-            # a frame without descriptors fails every pair it belongs to (matching.py:104-107)
-            frames = [(c if d is not None else np.zeros((0, 2), np.float32),
-                       d if d is not None else np.zeros((0, frames_d(frames)), np.uint8)) for c, d in frames]
-        dtype = np.uint8 if all(d.dtype == np.uint8 for _, d in frames) else np.float32
-        desc = np.concatenate([np.asarray(d, dtype).reshape(len(c), -1) for c, d in frames])
-        coords = np.concatenate([np.asarray(c, np.float32).reshape(-1, 2) for c, _ in frames])
-        st = eng.ingest(desc, coords, [len(c) for c, _ in frames])
+        st = _ingest_frames(eng, [feats[t]], frames_d(feats[t]))
         r = eng.match(st, np.arange(1, F), np.arange(0, F - 1))
         h1 = eng.find_homography(r.m_pts, r.out_off, r.m_cnt, r.status, st.max_kp, n_hyp, seed, 0, 1,
                                  THRESHOLD_FOR_FIND_HOMOGRAPHY, 0.0, _lib.ST_NO_MODEL_1)
@@ -150,6 +142,125 @@ def geometry_from_features(feats, none_H_processing=True, mode="reference", n_hy
     return H_list, st_out
 
 
+class PairLayout:
+    """Where the pairs of several videos sit in one batched call.  Video v has n_pairs[v] pairs; pair (v, k) is frame
+    pair (k + 1, k) of video v.
+      video, k   int64 [P]  video and within-video pair index of every pair, in processing order
+      inverse    int64 [P]  processing position of every pair in input order (video-major, videos in input order), so that
+                            per_pair_result[inverse] lists video 0's pairs, then video 1's, ...
+      seg_off    int64 [V+1] first input-order position of every video's pairs (the split of per_pair_result[inverse])
+      step_off   int64 [K+1] step-major only: step k = pairs [step_off[k], step_off[k+1]) = pair k of the n_k longest videos
+    Step-major order (the lockstep reference chain) sorts the videos by pair count, longest first (ties in input order),
+    so the chains still running at step k are a prefix; otherwise the order is video-major in input order, which is what
+    the segmented scan wants."""
+
+    def __init__(self, n_pairs, step_major):
+        n = np.asarray(n_pairs, np.int64).reshape(-1)
+        self.seg_off = np.zeros(len(n) + 1, np.int64)
+        np.cumsum(n, out=self.seg_off[1:])
+        video_in = np.repeat(np.arange(len(n), dtype=np.int64), n)        # input order
+        k_in = np.arange(int(self.seg_off[-1]), dtype=np.int64) - self.seg_off[video_in]
+        if step_major:
+            rank = np.empty(len(n), np.int64)
+            rank[np.argsort(-n, kind="stable")] = np.arange(len(n))
+            order = np.lexsort((rank[video_in], k_in))                    # by step, then by rank of the video
+            self.step_off = np.searchsorted(k_in[order], np.arange(int(n.max(initial=0)) + 1), side="left").astype(np.int64)
+        else:
+            order = np.arange(len(video_in), dtype=np.int64)
+            self.step_off = None
+        self.video, self.k = video_in[order], k_in[order]
+        self.inverse = np.empty(len(order), np.int64)
+        self.inverse[order] = np.arange(len(order), dtype=np.int64)
+
+    def split(self, per_pair):
+        """per-pair values in processing order -> list over videos (input order) of their pairs in order."""
+        x = np.asarray(per_pair)[self.inverse]
+        return [x[a:b] for a, b in zip(self.seg_off[:-1], self.seg_off[1:])]
+
+
+def _ingest_frames(eng, frames_per_video, d):
+    """One frame store over the frames of every video, concatenated; d = descriptor width of the feature type.  A frame
+    without descriptors becomes an empty frame: it fails every pair it belongs to (matching.py:104-107)."""
+    frames = [(c if dd is not None else np.zeros((0, 2), np.float32), dd if dd is not None else np.zeros((0, d), np.uint8))
+              for fr in frames_per_video for c, dd in fr]
+    dtype = np.uint8 if all(dd.dtype == np.uint8 for _, dd in frames) else np.float32
+    desc = np.concatenate([np.asarray(dd, dtype).reshape(len(c), d) for c, dd in frames])
+    coords = np.concatenate([np.asarray(c, np.float32).reshape(-1, 2) for c, _ in frames])
+    return eng.ingest(desc, coords, [len(c) for c, _ in frames])
+
+
+def geometry_from_features_batch(feats_list, none_H_processing=True, mode="reference", n_hyp=None, seed=None, engine=None):
+    """`geometry_from_features` for many videos in one call: returns [(H_list, status)] in input order, entry i equal to
+    geometry_from_features(feats_list[i], ...).  All videos share one frame store per feature type and one launch of
+    every per-pair stage; pair k of every video keeps RANSAC id k.  mode="parallel" ends in one segmented scan;
+    mode="reference" runs the reference-exact chains of all videos in lockstep on the device (one RANSAC #2 launch and
+    one chain-step launch per step, no host round trip inside the loop)."""
+    from .. import default_engine
+    eng = engine or default_engine()
+    n_hyp = RANSAC_HYPOTHESES if n_hyp is None else n_hyp
+    seed = RANSAC_SEED if seed is None else seed
+    if mode not in ("reference", "parallel"):
+        raise ValueError("mode must be 'reference' or 'parallel'")
+    if not feats_list:
+        return []
+    types = list(feats_list[0])
+    if any(list(f) != types for f in feats_list):
+        raise ValueError("every video must list the same feature types")
+    F = np.array([len(f[types[0]]) for f in feats_list], np.int64)
+    n_pairs = np.maximum(F - 1, 0)
+    lay = PairLayout(n_pairs, step_major=(mode == "reference"))
+    P = len(lay.k)
+    if P == 0:
+        return [([], np.zeros(0, np.int32)) for _ in feats_list]
+    dev = eng.device
+    f0 = np.zeros(len(F), np.int64)
+    np.cumsum(F[:-1], out=f0[1:])
+    pq = f0[lay.video] + lay.k + 1
+    pt = f0[lay.video] + lay.k
+    ids = torch.from_numpy(lay.k).to(dev)
+    status = torch.zeros(P, dtype=torch.int32, device=dev)
+    per_type, video_kp = [], []
+    for t in types:
+        d = next((dd.shape[1] for f in feats_list for _, dd in f[t] if dd is not None), 128)
+        st = _ingest_frames(eng, [f[t] for f in feats_list], d)
+        kp = st.n_kp_h.astype(np.int64)
+        video_kp.append([int(kp[a:b].max(initial=0)) for a, b, n in zip(f0, f0 + F, n_pairs) if n])   # each video's store max_kp
+        r = eng.match(st, pq, pt)
+        h1 = eng.find_homography(r.m_pts, r.out_off, r.m_cnt, r.status, st.max_kp, n_hyp, seed, 0, 1,
+                                 THRESHOLD_FOR_FIND_HOMOGRAPHY, 0.0, _lib.ST_NO_MODEL_1, pair_ids=ids)
+        sp, sc, _, _ = eng.static_filter(r.m_pts, r.out_off, r.m_cnt, h1["H"], r.status, max_cnt=st.max_kp)
+        status = torch.where(status == 0, r.status, status)
+        per_type.append((st, r, sp, sc))
+    # level-2 input, as geometry_from_features builds it; max_cnt = the largest of the per-video bounds it would use
+    if len(types) == 1:
+        st, r, pts2, cnt2 = per_type[0]
+        off2 = r.out_off
+        max_cnt = max(video_kp[0])
+        cnt2 = torch.where(status == 0, cnt2, torch.zeros_like(cnt2))
+    else:
+        cap = np.zeros(P, np.int64)
+        for st, _, _, _ in per_type:
+            cap += st.n_kp_h[pq].astype(np.int64)
+        cap = (cap + 3) // 4 * 4 + 4
+        off_h = np.zeros(P, np.int64)
+        np.cumsum(cap[:-1], out=off_h[1:])
+        max_cnt = max(max(sum(v), 4) for v in zip(*video_kp))
+        off2 = torch.from_numpy(off_h.astype(np.int32)).to(dev)
+        pts2, cnt2 = eng.concat_dedup([(sp, r.out_off, sc) for _, r, sp, sc in per_type], status, off2,
+                                      int(cap.sum()), max_cnt)
+    if mode == "parallel":
+        h2 = eng.find_homography(pts2, off2, cnt2, status, max_cnt, n_hyp, seed, 0, 2, THRESHOLD_FOR_FIND_HOMOGRAPHY,
+                                 LENGTH_ACCOUNTED_POINTS, _lib.ST_NO_MODEL_2, pair_ids=ids)
+        seg_off = torch.from_numpy(lay.seg_off.astype(np.int32)).to(dev)
+        _, H = eng.chain_scan_segments(h2["H"], status, seg_off, none_H_processing)
+    else:
+        H = eng.reference_chains(pts2, off2, cnt2, status, max_cnt, lay.step_off, n_hyp, seed, none_H_processing,
+                                 THRESHOLD_FOR_FIND_HOMOGRAPHY, LENGTH_ACCOUNTED_POINTS, _lib.ST_NO_MODEL_2)
+    H = H.cpu().numpy().reshape(P, 3, 3)
+    st_h = status.cpu().numpy()
+    return [([Hv[k] for k in range(len(Hv))], sv) for Hv, sv in zip(lay.split(H), lay.split(st_h))]
+
+
 def frames_d(frames):
     for _, d in frames:
         if d is not None:
@@ -168,3 +279,17 @@ def get_homography_dict(capture, resize_width=400, matching_path=None, none_H_pr
         homography_dict[k + 2] = {"H": np.asarray(H, np.float64).tolist()}
     homography_dict["resize_info"] = {"h": int(shape[0]), "w": int(shape[1])}
     return homography_dict
+
+
+def get_homography_dicts(captures, resize_width=400, matching_path=None, none_H_processing=True,
+                         features_type_list=None, mode="reference", n_hyp=None, seed=None):
+    """`get_homography_dict` for several captures: every capture is decoded and described as there, then the geometry
+    of all of them runs in one `geometry_from_features_batch` call.  Returns one dict per capture, in order."""
+    described = [read_and_describe(c, resize_width, features_type_list) for c in captures]
+    results = geometry_from_features_batch([f for f, _ in described], none_H_processing, mode, n_hyp, seed)
+    out = []
+    for (_, shape), (H_list, _) in zip(described, results):
+        homography_dict = {k + 2: {"H": np.asarray(H, np.float64).tolist()} for k, H in enumerate(H_list)}
+        homography_dict["resize_info"] = {"h": int(shape[0]), "w": int(shape[1])}
+        out.append(homography_dict)
+    return out

@@ -190,6 +190,19 @@ int evz_find_homography(evz_handle* h, const float* pts, const int32_t* off, con
                         int32_t* status, double* H, uint8_t* mask, int32_t* inl_cnt,
                         int32_t* best_hyp, int32_t* best_cnt, uint8_t* mask_best, double* H_best,
                         void* stream);
+/* The same with a sampler id per pair instead of pair_id_base + p: pair p is seeded with pair_id[p].  Replaces the same
+ * call sites; used to run the pairs of several videos in one launch while pair k of every video keeps id k, so that each
+ * pair gets the result of a call on its video alone (video_processing.py:67-105 runs one video per call).
+ *   pair_id    DEV int64 [P] (required)
+ * Every other argument and result is that of evz_find_homography; with pair_id[p] = pair_id_base + p the results are
+ * identical to it.
+ */
+int evz_find_homography_ids(evz_handle* h, const float* pts, const int32_t* off, const int32_t* cnt, int n_pairs,
+                            int max_cnt, const double* pre_H, int n_hyp, uint32_t seed, const int64_t* pair_id, int level,
+                            double thresh, double min_inlier_frac, int fail_status,
+                            int32_t* status, double* H, uint8_t* mask, int32_t* inl_cnt,
+                            int32_t* best_hyp, int32_t* best_cnt, uint8_t* mask_best, double* H_best,
+                            void* stream);
 
 /* ---- K5: displacement-mode static-point filter.  Replaces find_point_displacement
  * (utils.py:289-325) + get_largest_group_points (utils.py:258-286).
@@ -238,6 +251,34 @@ int evz_concat_dedup(evz_handle* h, int n_types, const float* const* pts, const 
 int evz_chain_scan(evz_handle* h, const double* G, const int32_t* status, int n_pairs, int policy,
                    const double* seed_S, const double* seed_G,
                    double* S, double* H_fixed, double* summary, void* stream);
+
+/* ---- K6, many chains in one call: evz_chain_scan (no seeds, no summary) over every segment of the pair list.
+ * Replaces video_processing.py:94-103 and superposition_dict (utils.py:184-211) for several videos at once: segment s is
+ * one video's chain, pairs [seg_off[s], seg_off[s+1]); the None-H fill and the product restart at its first pair.
+ *   seg_off DEV int32 [n_segs+1], non-decreasing, seg_off[0] = 0, seg_off[n_segs] = n_pairs; empty segments are allowed
+ *   S       DEV double [P][9] (required), H_fixed DEV double [P][9] or NULL
+ * The rows of every segment are bit-identical to what evz_chain_scan writes for that segment alone (same policy): the
+ * segment is cut into 256-pair blocks counted from its own start and scanned by the same kernels.  A fixed number of
+ * launches, whatever n_segs; handle scratch of about 4 B per pair + 160 B per (256 pairs + 1 segment).
+ */
+int evz_chain_scan_segments(evz_handle* h, const double* G, const int32_t* status, int n_pairs,
+                            const int32_t* seg_off, int n_segs, int policy, double* S, double* H_fixed, void* stream);
+
+/* ---- K6c: one step of the reference-exact chain for n_chains independent chains.  Replaces the host loop body of
+ * video_processing.py:94-105 (None-H policy, matrix_superposition utils.py:118-145) so that a chain advances without a
+ * host round trip; the next step's RANSAC #2 reads S_state as its pre_H.  Chain c:
+ *   H = H2[c]        if status[c] == EVZ_ST_OK
+ *     = H_prev[c]    elif policy and not first              (video_processing.py:95-96)
+ *     = identity     otherwise                              (the reference crashes here; DESIGN.md deviation 4)
+ *   H_out[c] = H;  S_state[c] = H if first (un-normalised, as the reference), else C / C[2][2] with C = H . S_state[c]
+ *   C[i][j] = fma(H[i][2], S[2][j], fma(H[i][1], S[1][j], H[i][0] * S[0][j])), each operation rounded once (the order of
+ *   NumPy's np.dot on 3x3 f64 through OpenBLAS), then an IEEE division of every element by C[2][2].
+ *   H2, H_out DEV double [n_chains][9]; status DEV int32 [n_chains]; S_state DEV double [n_chains][9] (in/out)
+ *   H_prev DEV double [n_chains][9]: the previous step's H_out (may alias H_out); NULL allowed when first or policy = 0
+ * n_chains = 0 is a no-op.  Chains that end early are dropped from the end: order chains by length, longest first.
+ */
+int evz_chain_ref_step(evz_handle* h, const double* H2, const int32_t* status, int n_chains, int first, int policy,
+                       double* S_state, const double* H_prev, double* H_out, void* stream);
 
 /* ---- K6b: cross-GPU seeding of the scan, on the device (no host round trip).  Every rank calls evz_chain_scan with
  * S and summary (no seeds: an UNSEEDED local scan), all-gathers the 20-double summaries into `summaries`
