@@ -267,10 +267,12 @@ fill_apply_kernel(int32_t* __restrict__ src, const int32_t* __restrict__ block_c
     const int k = sb.blk * kScanBlock + threadIdx.x;
     if (k < sb.n) src[sb.base + k] = max(src[sb.base + k], block_carry[sb.slot]);
 }
-// phase B1: Gf[k] = filled step matrix; local inclusive product scan; block totals
+// phase B1: Gf[k] = filled step matrix; local inclusive product scan; block totals.  Only block 0 of an unseeded scan holds
+// true prefixes, which are normalised here; every other block stores its block-local prefix (a partial product, whose
+// [2][2] may be 0) with its power-of-two scale, and prod_apply_kernel normalises it once the carry is applied.
 __global__ void __launch_bounds__(kScanBlock)
 prod_local_kernel(const double* __restrict__ G, const int32_t* __restrict__ src,
-                  int n, int policy, const double* __restrict__ seed_G,
+                  int n, int policy, const double* __restrict__ seed_G, int has_seed,
                   double* __restrict__ S, double* __restrict__ block_tot,
                   const int32_t* __restrict__ seg_off, const int32_t* __restrict__ seg_blk, int n_segs) {
     __shared__ double wt[kScanBlock / 32][9];
@@ -297,7 +299,7 @@ prod_local_kernel(const double* __restrict__ G, const int32_t* __restrict__ src,
         for (int w = 1; w < warp; ++w) c = m3_mul_scaled(c, m3_load(wt[w]));
         v = m3_mul_scaled(c, v);
     }
-    if (k < sb.n) m3_store(S + static_cast<size_t>(sb.base + k) * 9, m3_norm22(v));   // a true prefix of the (shard's) chain
+    if (k < sb.n) m3_store(S + static_cast<size_t>(sb.base + k) * 9, (sb.blk == 0 && !has_seed) ? m3_norm22(v) : v);
     if (threadIdx.x == kScanBlock - 1) m3_store(block_tot + static_cast<size_t>(sb.slot) * 9, v);
 }
 // phase B2 (one CTA per segment): exclusive prefix of the block totals, seeded.  Block-wide shuffle scan over
@@ -461,20 +463,22 @@ remap_kernel(const double* __restrict__ pin, const int32_t* __restrict__ frame_i
     reinterpret_cast<double2*>(pout)[i] = r;
 }
 
-// dense max-movement: max over frames and pixels of max(x', y')
+// dense max-movement: max over frames and pixels of max(x', y').  gridDim.y is at most 65 535, so y-block b covers
+// frames b, b + gridDim.y, ...; one partial per (y-block, x-block).
 __global__ void __launch_bounds__(256)
 max_movement_kernel(const double* __restrict__ S, int n_frames, int height, int width, double* __restrict__ partial) {
     __shared__ double ws[8];
-    const int f = blockIdx.y;
-    const M3 T = m3_load(S + static_cast<size_t>(f) * 9);
     double best = -1.0 / 0.0;
     const int npix = height * width;
-    for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < npix; i += gridDim.x * blockDim.x) {
-        const double x = static_cast<double>(i % width), y = static_cast<double>(i / width);
-        const double X = (T.m[0] * x + T.m[1] * y) + T.m[2];
-        const double Y = (T.m[3] * x + T.m[4] * y) + T.m[5];
-        const double W = (T.m[6] * x + T.m[7] * y) + T.m[8];
-        best = fmax(best, fmax(X / W, Y / W));
+    for (int f = blockIdx.y; f < n_frames; f += gridDim.y) {
+        const M3 T = m3_load(S + static_cast<size_t>(f) * 9);
+        for (int i = blockIdx.x * blockDim.x + threadIdx.x; i < npix; i += gridDim.x * blockDim.x) {
+            const double x = static_cast<double>(i % width), y = static_cast<double>(i / width);
+            const double X = (T.m[0] * x + T.m[1] * y) + T.m[2];
+            const double Y = (T.m[3] * x + T.m[4] * y) + T.m[5];
+            const double W = (T.m[6] * x + T.m[7] * y) + T.m[8];
+            best = fmax(best, fmax(X / W, Y / W));
+        }
     }
 #pragma unroll
     for (int of = 16; of > 0; of >>= 1) best = fmax(best, __shfl_xor_sync(0xffffffff, best, of));
@@ -482,7 +486,7 @@ max_movement_kernel(const double* __restrict__ S, int n_frames, int height, int 
     __syncthreads();
     if (threadIdx.x == 0) {
         for (int w = 1; w < 8; ++w) best = fmax(best, ws[w]);
-        partial[static_cast<size_t>(f) * gridDim.x + blockIdx.x] = best;
+        partial[static_cast<size_t>(blockIdx.y) * gridDim.x + blockIdx.x] = best;
     }
 }
 __global__ void max_reduce_kernel(const double* __restrict__ partial, int n, double* __restrict__ out) {
@@ -556,7 +560,7 @@ extern "C" int evz_chain_scan(evz_handle* h, const double* G, const int32_t* sta
     const bool seeded = seed_S != nullptr || seed_G != nullptr;
     if (summary || (S && !seeded)) {
         // unseeded pass: leading invalid pairs are identity steps, so the total is R
-        evz::prod_local_kernel<<<nb, evz::kScanBlock, 0, st>>>(G, src, n_pairs, policy, nullptr, S_work, block_tot, nullptr, nullptr, 0);
+        evz::prod_local_kernel<<<nb, evz::kScanBlock, 0, st>>>(G, src, n_pairs, policy, nullptr, 0, S_work, block_tot, nullptr, nullptr, 0);
         EVZ_LAUNCH_CHECK(h);
         evz::prod_carry_kernel<<<1, evz::kScanBlock, 0, st>>>(block_tot, nb, nullptr, block_pre, nullptr);
         EVZ_LAUNCH_CHECK(h);
@@ -568,7 +572,7 @@ extern "C" int evz_chain_scan(evz_handle* h, const double* G, const int32_t* sta
         }
     }
     if (S && seeded) {
-        evz::prod_local_kernel<<<nb, evz::kScanBlock, 0, st>>>(G, src, n_pairs, policy, seed_G, S, block_tot, nullptr, nullptr, 0);
+        evz::prod_local_kernel<<<nb, evz::kScanBlock, 0, st>>>(G, src, n_pairs, policy, seed_G, seed_S ? 1 : 0, S, block_tot, nullptr, nullptr, 0);
         EVZ_LAUNCH_CHECK(h);
         evz::prod_carry_kernel<<<1, evz::kScanBlock, 0, st>>>(block_tot, nb, seed_S, block_pre, nullptr);
         EVZ_LAUNCH_CHECK(h);
@@ -614,7 +618,7 @@ extern "C" int evz_chain_scan_segments(evz_handle* h, const double* G, const int
     EVZ_LAUNCH_CHECK(h);
     evz::fill_apply_kernel<<<nb, evz::kScanBlock, 0, st>>>(src, block_carry, n_pairs, seg_off, seg_blk, n_segs);
     EVZ_LAUNCH_CHECK(h);
-    evz::prod_local_kernel<<<nb, evz::kScanBlock, 0, st>>>(G, src, n_pairs, policy, nullptr, S, block_tot, seg_off, seg_blk, n_segs);
+    evz::prod_local_kernel<<<nb, evz::kScanBlock, 0, st>>>(G, src, n_pairs, policy, nullptr, 0, S, block_tot, seg_off, seg_blk, n_segs);
     EVZ_LAUNCH_CHECK(h);
     evz::prod_carry_kernel<<<n_segs, evz::kScanBlock, 0, st>>>(block_tot, nb, nullptr, block_pre, seg_blk);
     EVZ_LAUNCH_CHECK(h);
@@ -683,13 +687,14 @@ extern "C" int evz_max_movement(evz_handle* h, const double* S, int n_frames, in
     int bx = (height * width + 256 * 8 - 1) / (256 * 8);
     if (bx < 1) bx = 1;
     if (bx > 64) bx = 64;
+    const int by = n_frames < 65535 ? n_frames : 65535;         // the limit of gridDim.y; the kernel loops over the rest
     void* scr = nullptr;
-    int rc = evz_scratch(h, static_cast<size_t>(n_frames) * bx * 8 + 256, &scr);
+    int rc = evz_scratch(h, static_cast<size_t>(by) * bx * 8 + 256, &scr);
     if (rc) return rc;
-    dim3 grid(bx, n_frames);
+    dim3 grid(bx, by);
     evz::max_movement_kernel<<<grid, 256, 0, st>>>(S, n_frames, height, width, static_cast<double*>(scr));
     EVZ_LAUNCH_CHECK(h);
-    evz::max_reduce_kernel<<<1, 1024, 0, st>>>(static_cast<const double*>(scr), n_frames * bx, out_max);
+    evz::max_reduce_kernel<<<1, 1024, 0, st>>>(static_cast<const double*>(scr), by * bx, out_max);
     EVZ_LAUNCH_CHECK(h);
     return EVZ_OK;
 }

@@ -195,10 +195,14 @@ def _ref_step_host(H2, ok, sizes, policy):
     return out, S
 
 
-@pytest.mark.parametrize("policy", [True, False])
-def test_chain_ref_step_against_host_loop(engine, policy):
+@pytest.mark.parametrize("policy,sizes", [
+    pytest.param(True, [9, 9, 7, 7, 7, 4, 2, 2, 1, 1, 1, 1], id="True"),
+    pytest.param(False, [9, 9, 7, 7, 7, 4, 2, 2, 1, 1, 1, 1], id="False"),
+    pytest.param(True, [1000, 1000, 999, 700, 257, 256, 1], id="1000-chains-True"),      # four CTAs
+    pytest.param(False, [1000, 1000, 999, 700, 257, 256, 1], id="1000-chains-False"),
+])
+def test_chain_ref_step_against_host_loop(engine, policy, sizes):
     rng = np.random.default_rng(5)
-    sizes = [9, 9, 7, 7, 7, 4, 2, 2, 1, 1, 1, 1]
     P = sum(sizes)
     H2, ok = _random_steps(P, rng, 0.15)
     ok[:2] = False                                             # first pairs that fail: identity
