@@ -19,8 +19,9 @@
 //            Counts and the (count desc, hypothesis asc) arg-max are identical to evaluating the exact formula for every
 //            hypothesis (EVZ_OPT_RANSAC_EXACT / EVZ_OPT_RANSAC_NO_PRUNE force that, for the tests).
 // ransac_refit_kernel (64 threads, one CTA per pair that found a model)
-//   phase 3  inlier mask of the winner (exact formula) inside the first pass of an LM refit on the 8 free parameters in
-//            f64 with OpenCV's damping schedule, started undamped from the winning model;
+//   phase 3  inlier mask of the winner (exact formula, pixel coordinates) and the bounding boxes of its inliers, then an
+//            LM refit on the 8 free parameters in f64 with OpenCV's damping schedule, started undamped from the winning
+//            model and run in coordinates normalised by those boxes (see LmNorm);
 //   phase 4  final mask = f32 error of the refined H <= thresh^2, inlier count, 70 % gate.
 //
 // This file is compiled with --fmad=false: the f64 solver must round exactly like the NumPy
@@ -206,13 +207,21 @@ __device__ __forceinline__ double refit_rcp(double x) {
     r = fma(fma(-x, r, 1.0), r, r);
     return r;
 }
-__device__ __forceinline__ void lm_point(const double* h, const float4 pt, double* s) {
-    const double Mx = pt.x, My = pt.y;
+// The LM runs in normalised coordinates: a' = (a - ca) / sa, b' = (b - cb) / sb with ca, cb the centres of the bounding
+// boxes of the winner's inliers and sa, sb powers of two that bound their half-extents, so |a'|, |b'| <= 1 over the
+// inliers and both maps are exact in f64.  In pixel coordinates far from the origin J^T J is close to singular in f64
+// (a 96 x 54 px patch at (1500, 800): the LM stalled up to 1.66 px from the optimum); in these it stays well
+// conditioned.  The residuals are those
+// in pixels of b divided by sb, so the minimiser is the same.
+struct LmNorm { double cax, cay, ia, cbx, cby, ib; };
+__device__ __forceinline__ void lm_point(const double* h, const LmNorm& nm, const float4 pt, double* s) {
+    const double Mx = (pt.x - nm.cax) * nm.ia, My = (pt.y - nm.cay) * nm.ia;
+    const double bx = (pt.z - nm.cbx) * nm.ib, by = (pt.w - nm.cby) * nm.ib;
     double ww = fma(h[6], Mx, fma(h[7], My, 1.0));
     ww = fabs(ww) > DBL_EPSILON ? refit_rcp(ww) : 0.0;
     const double xi = fma(h[0], Mx, fma(h[1], My, h[2])) * ww;
     const double yi = fma(h[3], Mx, fma(h[4], My, h[5])) * ww;
-    const double rx = xi - pt.z, ry = yi - pt.w;
+    const double rx = xi - bx, ry = yi - by;
     const double p0 = Mx * ww, p1 = My * ww, p2 = ww;
     const double p00 = p0 * p0, p01 = p0 * p1, p02 = p0 * p2, p11 = p1 * p1, p12 = p1 * p2, p22 = p2 * p2;
     s[0] += p00; s[1] += p01; s[2] += p02; s[3] += p11; s[4] += p12; s[5] += p22;
@@ -246,37 +255,62 @@ __device__ void lm_expand(const double* s, double* A, double* v) {
     v[6] = s[27]; v[7] = s[28];
 }
 
+// G = T_b H T_a^-1 with T(p) = (p - c) / s, scaled to g22 = 1; x receives the 8 free entries
+__device__ void lm_to_normalised(const double* H, const LmNorm& nm, double sa, double* x) {
+    double M[9];                                              // H T_a^-1
+    for (int r = 0; r < 3; ++r) {
+        M[3 * r] = H[3 * r] * sa;
+        M[3 * r + 1] = H[3 * r + 1] * sa;
+        M[3 * r + 2] = (H[3 * r] * nm.cax + H[3 * r + 1] * nm.cay) + H[3 * r + 2];
+    }
+    double G[9];
+    for (int j = 0; j < 3; ++j) {
+        G[j] = (M[j] - nm.cbx * M[6 + j]) * nm.ib;
+        G[3 + j] = (M[3 + j] - nm.cby * M[6 + j]) * nm.ib;
+        G[6 + j] = M[6 + j];
+    }
+    const double inv = 1.0 / G[8];
+    for (int i = 0; i < 8; ++i) x[i] = G[i] * inv;
+}
+// H = T_b^-1 G T_a, scaled to h22 = 1 (all 9 entries written)
+__device__ void lm_from_normalised(const double* x, const LmNorm& nm, double sb, double* H) {
+    double N[9];                                              // G T_a
+    for (int r = 0; r < 3; ++r) {
+        const double g0 = x[3 * r], g1 = x[3 * r + 1], g2 = r == 2 ? 1.0 : x[3 * r + 2];
+        N[3 * r] = g0 * nm.ia;
+        N[3 * r + 1] = g1 * nm.ia;
+        N[3 * r + 2] = g2 - (g0 * nm.cax + g1 * nm.cay) * nm.ia;
+    }
+    double K[9];
+    for (int j = 0; j < 3; ++j) {
+        K[j] = N[j] * sb + nm.cbx * N[6 + j];
+        K[3 + j] = N[3 + j] * sb + nm.cby * N[6 + j];
+        K[6 + j] = N[6 + j];
+    }
+    const double inv = 1.0 / K[8];
+    for (int i = 0; i < 8; ++i) H[i] = K[i] * inv;
+    H[8] = 1.0;
+}
+
 struct LmShared {
-    double x[8], A[64], v[8], D[8];
+    double x[8], A[64], v[8], D[8];     // x: parameters in normalised coordinates (g22 = 1)
+    double H[9];                        // the model in pixel coordinates (h22 = 1)
     double S, lam, lc;
+    double px_prev;                     // pixels moved by the last evaluated step if it was undamped and accepted, else inf
     double sums[kNSums];
     double wsum[kRfThreads / 32][kNSums];
-    float cmax_w[kRfThreads / 32];
+    float box_w[kRfThreads / 32][8];    // per warp: min and -max of ax, ay, bx, by
+    LmNorm nm;
     int iter, go;
 };
 
 // all threads: accumulate the packed sums at parameters h over the inliers flagged in msk
-// kMakeMask: the first pass also classifies every point with the winner's f32 model (hb, thresh2) and writes the mask
-template <bool kMakeMask>
-__device__ void lm_accumulate(const double* h, const float4* pts, uint8_t* msk, int m, LmShared& L,
-                              const float* hb = nullptr, float thresh2 = 0.f, uint8_t* mask_out = nullptr) {
+__device__ void lm_accumulate(const double* h, const float4* pts, const uint8_t* msk, int m, LmShared& L) {
     double s[kNSums];
 #pragma unroll
     for (int i = 0; i < kNSums; ++i) s[i] = 0.0;
-    if (kMakeMask) {
-        float hf[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) hf[i] = hb[i];
-        for (int i = threadIdx.x; i < m; i += blockDim.x) {
-            const float4 pt = pts[i];
-            const uint8_t in = reproj_err32(hf, pt) <= thresh2 ? 1 : 0;
-            msk[i] = in;
-            if (mask_out) mask_out[i] = in;
-            if (in) lm_point(h, pt, s);
-        }
-    } else {
-        for (int i = threadIdx.x; i < m; i += blockDim.x) if (msk[i]) lm_point(h, pts[i], s);
-    }
+    const LmNorm nm = L.nm;
+    for (int i = threadIdx.x; i < m; i += blockDim.x) if (msk[i]) lm_point(h, nm, pts[i], s);
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     // warp reduction of the 30 sums as a transposing butterfly: at every step a lane keeps one half of its values
     // and trades the other half, so that lane i ends up with the warp total of sum i (31 exchanges instead of
@@ -1051,16 +1085,13 @@ ransac_refit_kernel(const FhArgs a, const double* __restrict__ Hbest_in, const i
     const int64_t o = a.off[p];
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
     const double* T = a.pre_H ? a.pre_H + static_cast<size_t>(p) * 9 : nullptr;
-    float cmax = 0.f;
     if (T) {
         for (int i = tid; i < m; i += blockDim.x) {
             float4 v = reinterpret_cast<const float4*>(a.pts)[o + i];
             const float2 pa = pre_map(T, v.x, v.y), pb = pre_map(T, v.z, v.w);
-            v = make_float4(pa.x, pa.y, pb.x, pb.y);
-            pts[i] = v;
-            cmax = fmaxf(cmax, fmaxf(fabsf(v.x), fabsf(v.y)));
+            pts[i] = make_float4(pa.x, pa.y, pb.x, pb.y);
         }
-        if (tid < 8) L.x[tid] = Hbest_in[static_cast<size_t>(p) * 9 + tid];
+        if (tid < 9) L.H[tid] = Hbest_in[static_cast<size_t>(p) * 9 + tid];
     } else {
         // one bulk copy (TMA, 16 bytes per point) instead of a latency-bound loop of 64-thread loads: the point list of a
         // pair is contiguous and 16-byte aligned
@@ -1070,41 +1101,82 @@ ransac_refit_kernel(const FhArgs a, const double* __restrict__ Hbest_in, const i
             mbar_arrive_expect_tx(&stage_bar, static_cast<uint32_t>(m) * 16u);
             bulk_load_1d(pts, reinterpret_cast<const float4*>(a.pts) + o, static_cast<uint32_t>(m) * 16u, &stage_bar);
         }
-        if (tid < 8) L.x[tid] = Hbest_in[static_cast<size_t>(p) * 9 + tid];
+        if (tid < 9) L.H[tid] = Hbest_in[static_cast<size_t>(p) * 9 + tid];
         mbar_wait(&stage_bar, 0);
-        for (int i = tid; i < m; i += blockDim.x) {
-            const float4 v = pts[i];
-            cmax = fmaxf(cmax, fmaxf(fabsf(v.x), fabsf(v.y)));
-        }
     }
-#pragma unroll
-    for (int of = 16; of > 0; of >>= 1) cmax = fmaxf(cmax, __shfl_xor_sync(0xffffffff, cmax, of));
-    if (lane == 0) L.cmax_w[warp] = cmax;
     __syncthreads();
-#pragma unroll
-    for (int w = 0; w < kRfThreads / 32; ++w) cmax = fmaxf(cmax, L.cmax_w[w]);
-    const double cm = static_cast<double>(fmaxf(cmax, 1.f));
 
-    // ---------------- phase 3: winner's inlier mask and the first LM pass over it, in one sweep
+    // ---------------- phase 3: winner's inlier mask (pixel coordinates, f32 formula) and the bounding boxes of its
+    // inliers in a and b, as (min, -max) so that one fminf reduction serves both.  The boxes of the inliers, not of all
+    // points: outliers spread over the frame would leave inliers clustered in a corner ill-conditioned again.
+    float box[8];
+#pragma unroll
+    for (int k = 0; k < 8; ++k) box[k] = INFINITY;
     {
         float hb[8];
 #pragma unroll
-        for (int i = 0; i < 8; ++i) hb[i] = static_cast<float>(L.x[i]);
-        lm_accumulate<true>(L.x, pts, msk, m, L, hb, a.thresh2, a.mask_best ? a.mask_best + o : nullptr);
+        for (int i = 0; i < 8; ++i) hb[i] = static_cast<float>(L.H[i]);
+        uint8_t* mask_out = a.mask_best ? a.mask_best + o : nullptr;
+        for (int i = tid; i < m; i += blockDim.x) {
+            const float4 v = pts[i];
+            const uint8_t in = reproj_err32(hb, v) <= a.thresh2 ? 1 : 0;
+            msk[i] = in;
+            if (mask_out) mask_out[i] = in;
+            if (in) {
+                box[0] = fminf(box[0], v.x); box[1] = fminf(box[1], v.y); box[2] = fminf(box[2], v.z); box[3] = fminf(box[3], v.w);
+                box[4] = fminf(box[4], -v.x); box[5] = fminf(box[5], -v.y); box[6] = fminf(box[6], -v.z); box[7] = fminf(box[7], -v.w);
+            }
+        }
     }
+#pragma unroll
+    for (int k = 0; k < 8; ++k) {
+#pragma unroll
+        for (int of = 16; of > 0; of >>= 1) box[k] = fminf(box[k], __shfl_xor_sync(0xffffffff, box[k], of));
+    }
+    if (lane == 0) {
+#pragma unroll
+        for (int k = 0; k < 8; ++k) L.box_w[warp][k] = box[k];
+    }
+    __syncthreads();
+    if (tid == 0) {
+        // (the winner counts at least 4 inliers, so the boxes are finite)
+        for (int w = 1; w < kRfThreads / 32; ++w)
+            for (int k = 0; k < 8; ++k) box[k] = fminf(box[k], L.box_w[w][k]);
+        // centre: an f32 value, so that x - c is exact in f64; scale: a power of two >= the half-extent (at least 1 px)
+        LmNorm nm;
+        double sc[2];
+        for (int q = 0; q < 2; ++q) {
+            const float lx = box[2 * q], ly = box[2 * q + 1], hx = -box[4 + 2 * q], hy = -box[5 + 2 * q];
+            const float cx = 0.5f * lx + 0.5f * hx, cy = 0.5f * ly + 0.5f * hy;
+            const double ext = fmax(1.0, fmax(fmax(static_cast<double>(hx) - cx, static_cast<double>(cx) - lx),
+                                              fmax(static_cast<double>(hy) - cy, static_cast<double>(cy) - ly)));
+            int e;
+            frexp(ext, &e);
+            sc[q] = ldexp(1.0, e);
+            if (q == 0) { nm.cax = cx; nm.cay = cy; } else { nm.cbx = cx; nm.cby = cy; }
+        }
+        nm.ia = 1.0 / sc[0]; nm.ib = 1.0 / sc[1];
+        L.nm = nm;
+        lm_to_normalised(L.H, nm, sc[0], L.x);
+    }
+    __syncthreads();
+    const double sb = 1.0 / L.nm.ib;                       // pixels of b per normalised unit
+    const double s_eps = DBL_EPSILON * L.nm.ib * L.nm.ib;  // OpenCV's DBL_EPSILON guards, in px^2, in units of S
+    // first LM pass over the inliers
+    lm_accumulate(L.x, pts, msk, m, L);
     if (tid == 0) {
         lm_expand(L.sums, L.A, L.v);
         for (int i = 0; i < 8; ++i) L.D[i] = L.A[i * 8 + i];
         L.S = L.sums[29];
         // (OpenCV starts at lambda = 1 from a DLT estimate; from the winning 4-point model an undamped first step saves
-        // one pass over the inliers and reaches the same optimum -- a step that does not reduce S is damped as usual)
-        L.lam = 0.0; L.lc = 0.75; L.iter = 0;
-        L.go = L.sums[30] >= static_cast<double>(FLT_EPSILON);
+        // one pass over the inliers -- a step that does not reduce S is damped as usual)
+        L.lam = 0.0; L.lc = 0.75; L.iter = 0; L.px_prev = INFINITY;
+        L.go = L.sums[30] * sb >= static_cast<double>(FLT_EPSILON);
     }
     __syncthreads();
     while (L.go) {
         // every thread solves (A + lambda diag(D)) d = v redundantly in registers: no serial section
-        double d[8], xd[8];
+        double d[8], xd[8], px;
         {
             Ldl8 f;
             ldl8_factor(L.A, L.D, L.lam, f);
@@ -1114,38 +1186,43 @@ ransac_refit_kernel(const FhArgs a, const double* __restrict__ Hbest_in, const i
             ldl8_solve(f, vv, d);
 #pragma unroll
             for (int i = 0; i < 8; ++i) { if (!f.ok) d[i] = 0.0; xd[i] = L.x[i] - d[i]; }
-            // a step that moves no point of the data range by more than kPxTol pixels is not worth a pass over the
-            // inliers: converged (every thread holds the same d, so the exit is uniform)
-            const double px = fmax(fmax(fabs(d[0]), fabs(d[1])), fmax(fabs(d[3]), fabs(d[4]))) * cm + fmax(fabs(d[2]), fabs(d[5])) +
-                              fmax(fabs(d[6]), fabs(d[7])) * cm * cm;
+            // a step that moves no inlier by more than kPxTol pixels of b is not worth a pass over the inliers: converged
+            // (every thread holds the same d, so the exit is uniform).  px estimates that movement from the entries of d:
+            // |a'|, |b'| <= 1 over the inliers and den ~ 1, so a point moves by about |d0| x' + |d1| y' + |d2| +
+            // (|d6| x' + |d7| y') |xi'| normalised units; the largest entries stand in for the sums (within a factor of
+            // ~2 either way), and sb converts to pixels.
+            px = f.ok ? (fmax(fmax(fabs(d[0]), fabs(d[1])), fmax(fabs(d[3]), fabs(d[4]))) + fmax(fabs(d[2]), fabs(d[5])) +
+                         fmax(fabs(d[6]), fabs(d[7]))) * sb : 0.0;
             if (f.ok && px < kPxTol) break;
-            // an undamped step below kPxApply pixels is taken without the pass that would only confirm it: the step
-            // after it is smaller by the contraction factor of Gauss-Newton near the optimum (~1e-3 on these problems),
-            // i.e. far below kPxTol, so x - d is the point the full iteration stops at as well
-            if (f.ok && px < kPxApply && L.lam == 0.0) {
+            // an undamped step below kPxApply pixels is taken without the pass that would only confirm it when the step
+            // after it, px times the contraction px / px_prev of the last two Gauss-Newton steps, is below kPxTol: x - d
+            // is then the point the full iteration stops at as well.  Without a previous undamped step the contraction
+            // is taken to be small (the first step from the 4-point model).  The contraction is ~1e-3 on full-frame sets
+            // but 1e-2 and more on small noisy patches, where a fixed assumption left the result 1e-5 px short.
+            if (f.ok && px < kPxApply && L.lam == 0.0 && px * px < kPxTol * L.px_prev) {
                 __syncthreads();
                 if (tid < 8) L.x[tid] = xd[tid];
                 __syncthreads();
                 break;
             }
         }
-        lm_accumulate<false>(xd, pts, msk, m, L);
+        lm_accumulate(xd, pts, msk, m, L);
         if (tid == 0) {
             const double Sd = L.sums[29];
-            double dS = 0.0, tdv = 0.0, dmax = 0.0;
+            const double lam_step = L.lam;
+            double dS = 0.0, tdv = 0.0;
             for (int i = 0; i < 8; ++i) {
                 double Ad = 0.0;
                 for (int j = 0; j < 8; ++j) Ad += L.A[i * 8 + j] * d[j];
                 dS += d[i] * (2.0 * L.v[i] - Ad);
                 tdv += d[i] * L.v[i];
-                dmax = fmax(dmax, fabs(d[i]));
             }
-            const double R = (L.S - Sd) / (fabs(dS) > DBL_EPSILON ? dS : 1.0);
+            const double R = (L.S - Sd) / (fabs(dS) > s_eps ? dS : 1.0);
             if (R > 0.75) {
                 L.lam *= 0.5;
                 if (L.lam < L.lc) L.lam = 0.0;
             } else if (R < 0.25) {
-                double nu = (Sd - L.S) / (fabs(tdv) > DBL_EPSILON ? tdv : 1.0) + 2.0;
+                double nu = (Sd - L.S) / (fabs(tdv) > s_eps ? tdv : 1.0) + 2.0;
                 nu = fmin(fmax(nu, 2.0), 10.0);
                 if (L.lam == 0.0) {
                     // lambda = lc = 1 / max |diag(A^-1)|
@@ -1170,7 +1247,9 @@ ransac_refit_kernel(const FhArgs a, const double* __restrict__ Hbest_in, const i
                 L.lam *= nu;
             }
             double rmax = 0.0;
+            L.px_prev = INFINITY;
             if (Sd < L.S) {
+                if (lam_step == 0.0) L.px_prev = px;
                 L.S = Sd;
                 for (int i = 0; i < 8; ++i) L.x[i] = xd[i];
                 lm_expand(L.sums, L.A, L.v);
@@ -1179,15 +1258,19 @@ ransac_refit_kernel(const FhArgs a, const double* __restrict__ Hbest_in, const i
                 rmax = 1.0;     // residual at the kept x is unchanged and was >= eps
             }
             L.iter++;
-            L.go = L.iter < kLmMaxIters && dmax >= static_cast<double>(FLT_EPSILON) && rmax >= static_cast<double>(FLT_EPSILON);
+            // OpenCV also stops on a step below FLT_EPSILON in parameter units; here every step that reaches this point
+            // moves some point by kPxTol or more, except the zero step of a failed factorisation, which ends the loop
+            L.go = L.iter < kLmMaxIters && px > 0.0 && rmax * sb >= static_cast<double>(FLT_EPSILON);
         }
         __syncthreads();
     }
 
-    // ---------------- phase 4: final mask under the refined H, count, gate
+    // ---------------- phase 4: final mask under the refined H (pixel coordinates), count, gate
+    if (tid == 0) lm_from_normalised(L.x, L.nm, sb, L.H);
+    __syncthreads();
     float hfin[8];
 #pragma unroll
-    for (int i = 0; i < 8; ++i) hfin[i] = static_cast<float>(L.x[i]);
+    for (int i = 0; i < 8; ++i) hfin[i] = static_cast<float>(L.H[i]);
     int c = 0;
     for (int i = tid; i < m; i += blockDim.x) {
         const int in = reproj_err32(hfin, pts[i]) <= a.thresh2 ? 1 : 0;
@@ -1202,8 +1285,7 @@ ransac_refit_kernel(const FhArgs a, const double* __restrict__ Hbest_in, const i
         int tot = 0;
         for (int w = 0; w < kRfThreads / 32; ++w) tot += red[w];
         if (a.inl_cnt) a.inl_cnt[p] = tot;
-        for (int i = 0; i < 8; ++i) a.H[static_cast<size_t>(p) * 9 + i] = L.x[i];
-        a.H[static_cast<size_t>(p) * 9 + 8] = 1.0;
+        for (int i = 0; i < 9; ++i) a.H[static_cast<size_t>(p) * 9 + i] = L.H[i];
         if (a.min_inlier_frac > 0.0 && static_cast<double>(tot) < a.min_inlier_frac * static_cast<double>(m))
             a.status[p] = EVZ_ST_FEW_INLIERS;
     }

@@ -247,6 +247,138 @@ def refit(a, b):
     return H
 
 
+# ----------------------------------------------------------------------------- least-squares optimum
+def _project(H, p):
+    """pi(H p) for (N,2) points in the dtype of p (H is cast to it)."""
+    H = np.asarray(H).reshape(3, 3).astype(p.dtype)
+    w = H[2, 0] * p[:, 0] + H[2, 1] * p[:, 1] + H[2, 2]
+    return np.stack([(H[0, 0] * p[:, 0] + H[0, 1] * p[:, 1] + H[0, 2]) / w,
+                     (H[1, 0] * p[:, 0] + H[1, 1] * p[:, 1] + H[1, 2]) / w], 1)
+
+
+def probe_points(a):
+    """The points of a set plus the four corners of its bounding box (f64)."""
+    a = np.asarray(a, np.float64).reshape(-1, 2)
+    lo, hi = a.min(0), a.max(0)
+    corners = np.array([[lo[0], lo[1]], [hi[0], lo[1]], [lo[0], hi[1]], [hi[0], hi[1]]])
+    return np.concatenate([a, corners])
+
+
+def max_px_dist(H1, H2, a):
+    """Largest distance in pixels between pi(H1 p) and pi(H2 p) over the points of `a` and the corners of their
+    bounding box, evaluated in long double."""
+    p = probe_points(a).astype(np.longdouble)
+    return float(np.sqrt(((_project(H1, p) - _project(H2, p)) ** 2).sum(1)).max())
+
+
+def sum_sq(H, a, b):
+    """S(H) = sum |pi(H a) - b|^2 in long double (a, b as given, usually f32)."""
+    a = np.asarray(a).astype(np.longdouble).reshape(-1, 2)
+    b = np.asarray(b).astype(np.longdouble).reshape(-1, 2)
+    return float(((_project(H, a) - b) ** 2).sum())
+
+
+def _normalise(p):
+    """(T, p') for the similarity T that moves the centroid of p to the origin and scales the mean distance from it
+    to 1, and p' = T p."""
+    c = p.mean(0)
+    s = np.sqrt(((p - c) ** 2).sum(1)).mean()
+    s = s if s > 0 else 1.0
+    return np.array([[1 / s, 0, -c[0] / s], [0, 1 / s, -c[1] / s], [0, 0, 1.0]]), (p - c) / s
+
+
+def _gauss_newton(g, an, bn, probe, sb, max_iters=200, tol_px=1e-12):
+    """Gauss-Newton on the 8 free entries of g (g22 = 1) in normalised coordinates.  Far from the optimum a step is
+    halved until S does not grow; a step that moves no probe point by more than 1e-6 px of b is taken as it is (S cannot
+    resolve such steps in f64; Gauss-Newton converges there).  Stops when a step moves no probe point by more than
+    tol_px pixels of b.  Returns (g (9,), converged)."""
+    x = np.asarray(g, np.float64).ravel()[:8] / g.ravel()[8]
+    def move_px(x1, x0):
+        return sb * np.sqrt(((_project(np.append(x1, 1.0), probe) - _project(np.append(x0, 1.0), probe)) ** 2).sum(1)).max()
+    for _ in range(max_iters):
+        r, J = _lm_residual_jac(x, an, bn)
+        S = float(r @ r)
+        d = np.linalg.lstsq(J, r, rcond=None)[0]
+        t = 1.0
+        while True:
+            xt = x - t * d
+            mv = move_px(xt, x)
+            if mv <= 1e-6:
+                break
+            rt, _ = _lm_residual_jac(xt, an, bn, want_j=False)
+            if float(rt @ rt) <= S:
+                break
+            t *= 0.5
+        x = xt
+        if t == 1.0 and mv <= tol_px:
+            return np.append(x, 1.0), True
+    return np.append(x, 1.0), False
+
+
+def ls_optimum(a, b, H0):
+    """Minimiser of S(H) = sum |pi(H a) - b|^2 over the point set (a, b), h22 = 1.
+
+    Solved by Gauss-Newton with a backtracking line search in coordinates where a and b are moved to their centroids and
+    scaled by a similarity to unit mean distance: the residuals are those in pixels of b divided by one constant, so the
+    minimiser is unchanged, and J^T J is well conditioned even for a small patch far from the origin.  Iterates until a
+    step moves no point of a (nor a corner of its bounding box) by more than 1e-12 px.
+
+    Runs from H0 (the winning 4-point model), from the normalised DLT and from `refit` and keeps the lowest S.
+    Returns (H (9,) f64 with H[8] == 1, cert) where cert holds
+      grad_rel   max |J^T r| / (||J||_F (||r|| + ||J||_F ||x||)) at the optimum x in normalised coordinates, J^T r
+                 evaluated in long double (rounding x to f64 alone leaves ~1e-16 here; the ||J|| ||x|| term keeps the
+                 measure meaningful for exact fits, where r is rounding noise);
+      cond       condition number of the normalised J^T J (positive definite when finite and min_eig > 0);
+      min_eig    its smallest eigenvalue;
+      spread_px  largest max_px_dist between the optima reached from the different starts;
+      converged  every start met the 1e-12 px stop rule;
+      S          S at the optimum (long double, pixels)."""
+    a = np.asarray(a, np.float32).reshape(-1, 2)
+    b = np.asarray(b, np.float32).reshape(-1, 2)
+    a64, b64 = a.astype(np.float64), b.astype(np.float64)
+    Ta, an = _normalise(a64)
+    Tb, bn = _normalise(b64)
+    sb = 1.0 / Tb[0, 0]                 # pixels of b per normalised unit
+    Tb_inv = np.linalg.inv(Tb)
+    probe = probe_points(an)
+    starts = [np.asarray(H0, np.float64).reshape(3, 3)]
+    for H in (dlt_normalised(a, b), refit(a, b)):
+        if H is not None and np.isfinite(H).all():
+            starts.append(H.reshape(3, 3))
+    sols, conv = [], True
+    for H in starts:
+        g = Tb @ H @ np.linalg.inv(Ta)
+        g, ok = _gauss_newton(g / g[2, 2], an, bn, probe, sb)
+        conv = conv and ok
+        Hp = Tb_inv @ g.reshape(3, 3) @ Ta
+        Hp = Hp / Hp[2, 2]
+        sols.append((sum_sq(Hp, a, b), Hp.ravel(), g))
+    S, H, g = min(sols, key=lambda s: s[0])
+    spread = max(max_px_dist(H, s[1], a) for s in sols)
+    # certificate in the normalised parametrisation: gradient in long double, curvature of the normal equations
+    an_l, bn_l = an.astype(np.longdouble), bn.astype(np.longdouble)
+    gl = np.asarray(g, np.float64).astype(np.longdouble)
+    w = gl[6] * an_l[:, 0] + gl[7] * an_l[:, 1] + 1
+    xi = (gl[0] * an_l[:, 0] + gl[1] * an_l[:, 1] + gl[2]) / w
+    yi = (gl[3] * an_l[:, 0] + gl[4] * an_l[:, 1] + gl[5]) / w
+    r = np.empty(2 * len(a), np.longdouble)
+    r[0::2] = xi - bn_l[:, 0]
+    r[1::2] = yi - bn_l[:, 1]
+    J = np.zeros((2 * len(a), 8), np.longdouble)
+    J[0::2, 0] = an_l[:, 0] / w; J[0::2, 1] = an_l[:, 1] / w; J[0::2, 2] = 1 / w
+    J[1::2, 3] = an_l[:, 0] / w; J[1::2, 4] = an_l[:, 1] / w; J[1::2, 5] = 1 / w
+    J[0::2, 6] = -an_l[:, 0] * xi / w; J[0::2, 7] = -an_l[:, 1] * xi / w
+    J[1::2, 6] = -an_l[:, 0] * yi / w; J[1::2, 7] = -an_l[:, 1] * yi / w
+    grad = J.T @ r
+    nJ = np.sqrt(float((J.astype(np.float64) ** 2).sum()))
+    scale = nJ * (np.sqrt(float(r @ r)) + nJ * np.linalg.norm(np.asarray(g, np.float64)[:8]))
+    eig = np.linalg.eigvalsh((J.T @ J).astype(np.float64))
+    cert = dict(grad_rel=float(np.abs(grad).max()) / scale, min_eig=float(eig[0]),
+                cond=float(eig[-1] / eig[0]) if eig[0] > 0 else float("inf"),
+                spread_px=spread, converged=conv, S=S)
+    return H, cert
+
+
 # ----------------------------------------------------------------------------- driver
 ST_OK = 0
 ST_TOO_FEW = 3        # < 4 points: cv2.error in the reference (uncaught)
