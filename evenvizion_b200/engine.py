@@ -5,7 +5,7 @@ hand-written CUDA behind the C ABI of include/evz.h.  All heavy results stay on 
 as torch tensors; `video_geometry` is the host-arrays-in / host-arrays-out call.
 """
 import ctypes as C
-from dataclasses import dataclass, field
+from dataclasses import dataclass, field, fields
 from typing import Optional
 
 import numpy as np
@@ -79,6 +79,18 @@ class PairResults:
     inl2: Optional[torch.Tensor] = None
     extra: dict = field(default_factory=dict)
 
+    _PER_ROW = ("top2_idx", "top2_d2", "surv", "m_idx", "m_pts", "mask1", "mask1_best", "static_pts", "mask2", "mask2_best")
+
+    def pairs(self, p0, p1) -> "PairResults":
+        """Pairs [p0, p1) as views into this workspace: per-pair tensors (and `extra`) sliced, per-row tensors shared
+        (they are addressed through out_off), so engine calls given the view write into this workspace."""
+        v = {f.name: getattr(self, f.name) for f in fields(self)}
+        for k, t in v.items():
+            if k not in self._PER_ROW and isinstance(t, torch.Tensor):
+                v[k] = t[p0:p1]
+        v["extra"] = {k: t[p0:p1] for k, t in self.extra.items()}
+        return PairResults(**v)
+
 
 class GeometryEngine:
     def __init__(self, device: int = 0):
@@ -137,10 +149,10 @@ class GeometryEngine:
         return row_off.astype(np.int32)
 
     # ------------------------------------------------------------------ ingest
-    def ingest(self, desc, coords, n_kp=None, check=True) -> FrameStore:
-        """desc: [sum n_kp, d] uint8 or float32 (integer-valued, <= 255), frames concatenated (a
-        uniform [F, N, d] array is accepted too); coords: matching [.., 2] float32; n_kp: per-frame
-        counts.  Arrays may be numpy, pinned/CPU torch or CUDA torch tensors."""
+    @staticmethod
+    def _frames_input(desc, coords, n_kp):
+        """The frame input of `ingest` / `video_geometry`, normalised and checked: returns (desc [rows, d],
+        coords [rows, 2], n_kp int64 [F], d, is_f32), desc and coords as torch tensors where they were given."""
         desc_t = torch.as_tensor(desc)
         coords_t = torch.as_tensor(coords)
         if desc_t.dim() == 3:
@@ -165,76 +177,102 @@ class GeometryEngine:
             is_f32 = 1
         else:
             raise TypeError("descriptors must be uint8 or float32 (SIFT/ORB); SURF's non-integer floats are not supported")
-        desc_d = desc_t.to(self.device, non_blocking=True).contiguous()
-        coords_d = coords_t.to(torch.float32).to(self.device, non_blocking=True).contiguous()
+        return desc_t, coords_t, n_kp_h, d, is_f32
+
+    def _new_store(self, n_kp_h, d):
+        """An unfilled FrameStore for frames of n_kp_h keypoints.  Returns (store, raw_off_h, raw_off, bad): the host and
+        device offsets of every frame's first input row and the device count of non-integer descriptor values, which
+        `_ingest_frames` takes.  store.keep holds the device tensors until the stream has consumed them."""
+        dev = self.device
         row_off_h = self.layout(n_kp_h)
         raw_off_h = np.zeros(len(n_kp_h) + 1, np.int64)
         np.cumsum(n_kp_h, out=raw_off_h[1:])
         rows = int(row_off_h[-1])
-        raw_off = torch.from_numpy(raw_off_h).to(self.device, non_blocking=True)
-        row_off = torch.from_numpy(row_off_h).to(self.device, non_blocking=True)
-        n_kp_d = torch.from_numpy(n_kp_h.astype(np.int32)).to(self.device, non_blocking=True)
-        bad = torch.zeros(1, dtype=torch.int32, device=self.device)
+        raw_off = torch.from_numpy(raw_off_h).to(dev, non_blocking=True)
+        row_off = torch.from_numpy(row_off_h).to(dev, non_blocking=True)
+        n_kp_d = torch.from_numpy(n_kp_h.astype(np.int32)).to(dev, non_blocking=True)
+        bad = torch.zeros(1, dtype=torch.int32, device=dev)
         st = FrameStore(desc=self._empty((rows, EVZ_DESC_BYTES), torch.uint8), ckey=self._empty((rows,), torch.int32),
                         coords=self._empty((rows, 2), torch.float32), canon=self._empty((rows,), torch.int32),
                         row_off=row_off, n_kp=n_kp_d, row_off_h=row_off_h, n_kp_h=n_kp_h.astype(np.int32), d=d,
-                        keep=(desc_d, coords_d, raw_off, bad))
-        if rows and desc_d.shape[0]:
-            self._check(self.lib.evz_ingest(self.h, _ptr(desc_d), is_f32, d, _ptr(coords_d), _ptr(raw_off), _ptr(row_off),
-                                            len(n_kp_h), _ptr(st.desc), _ptr(st.ckey), _ptr(st.coords), _ptr(st.canon),
-                                            _ptr(bad), self._stream()))
-        elif rows:
-            st.desc.zero_(); st.ckey.fill_(2 ** 31 - 1); st.coords.zero_(); st.canon.fill_(-1)
-        if is_f32 and check and int(bad.item()):
-            raise ValueError(f"{int(bad.item())} descriptor values are not integers in [0,255]; "
+                        keep=(raw_off, bad))
+        return st, raw_off_h, raw_off, bad
+
+    def _ingest_frames(self, st, desc, coords, raw_off, is_f32, bad, f0, f1):
+        """Frames [f0, f1) of st from the device input rows desc / coords (frame f starts at row raw_off[f])."""
+        self._check(self.lib.evz_ingest(self.h, _ptr(desc), is_f32, st.d, _ptr(coords), _ptr(raw_off[f0:]),
+                                        _ptr(st.row_off[f0:]), f1 - f0, _ptr(st.desc), _ptr(st.ckey), _ptr(st.coords),
+                                        _ptr(st.canon), _ptr(bad), self._stream()))
+
+    @staticmethod
+    def _check_integer_descriptors(bad):
+        n = int(bad.item())
+        if n:
+            raise ValueError(f"{n} descriptor values are not integers in [0,255]; "
                              "the int8 tensor-core matcher is exact only for SIFT/ORB-style descriptors")
+
+    def ingest(self, desc, coords, n_kp=None, check=True) -> FrameStore:
+        """desc: [sum n_kp, d] uint8 or float32 (integer-valued, <= 255), frames concatenated (a
+        uniform [F, N, d] array is accepted too); coords: matching [.., 2] float32; n_kp: per-frame
+        counts.  Arrays may be numpy, pinned/CPU torch or CUDA torch tensors."""
+        desc_t, coords_t, n_kp_h, d, is_f32 = self._frames_input(desc, coords, n_kp)
+        desc_d = desc_t.to(self.device, non_blocking=True).contiguous()
+        coords_d = coords_t.to(torch.float32).to(self.device, non_blocking=True).contiguous()
+        st, _, raw_off, bad = self._new_store(n_kp_h, d)
+        st.keep += (desc_d, coords_d)
+        if st.rows and desc_d.shape[0]:
+            self._ingest_frames(st, desc_d, coords_d, raw_off, is_f32, bad, 0, st.n_frames)
+        elif st.rows:
+            st.desc.zero_(); st.ckey.fill_(2 ** 31 - 1); st.coords.zero_(); st.canon.fill_(-1)
+        if is_f32 and check:
+            self._check_integer_descriptors(bad)
         return st
 
     # ------------------------------------------------------------------ K1 / K1b / K2
-    def match(self, st: FrameStore, pair_q, pair_t, ratio=0.5, min_matching_pts=4) -> PairResults:
-        """K1 + K1b/K2 for the pairs (pair_q[p], pair_t[p]).  Per-row outputs of pair p start at
-        out_off[p] = row_off[pair_q[p]], so one call must not list the same query frame twice (the C ABI
-        takes out_off as an argument and has no such restriction)."""
+    def _match_results(self, st: FrameStore, pair_q, pair_t) -> PairResults:
+        """The outputs of `match` for the pairs (pair_q[p], pair_t[p]), allocated."""
         pq = torch.as_tensor(pair_q, dtype=torch.int32).to(self.device)
         pt = torch.as_tensor(pair_t, dtype=torch.int32).to(self.device)
-        P = int(pq.numel())
-        out_off = st.row_off[:-1][pq.long()].contiguous()
-        rows = st.rows
-        top2_idx = self._empty((rows, 2), torch.int32)
-        top2_d2 = self._empty((rows, 2), torch.int32)
-        self._check(self.lib.evz_match_top2_d(self.h, _ptr(st.desc), int(st.d), _ptr(st.ckey), rows, _ptr(st.row_off), _ptr(st.n_kp),
-                                              _ptr(pq), _ptr(pt), _ptr(out_off), P, _ptr(top2_idx), _ptr(top2_d2), self._stream()))
-        surv = self._empty((rows,), torch.uint8)
-        m_idx = self._empty((rows, 2), torch.int32)
-        m_pts = self._empty((rows, 4), torch.float32)
-        m_cnt = self._empty((P,), torch.int32)
-        n_filtered = self._empty((P,), torch.int32)
-        status = self._empty((P,), torch.int32)
-        self._check(self.lib.evz_filter_matches(self.h, _ptr(top2_idx), _ptr(top2_d2), _ptr(st.coords), _ptr(st.canon),
-                                                _ptr(st.row_off), _ptr(st.n_kp), _ptr(pq), _ptr(pt), _ptr(out_off), P,
-                                                st.max_kp, float(ratio), int(min_matching_pts),
-                                                _ptr(surv), _ptr(m_idx), _ptr(m_pts), _ptr(m_cnt), _ptr(n_filtered),
-                                                _ptr(status), self._stream()))
-        return PairResults(pair_q=pq, pair_t=pt, out_off=out_off, top2_idx=top2_idx, top2_d2=top2_d2, surv=surv,
-                           m_idx=m_idx, m_pts=m_pts, m_cnt=m_cnt, n_filtered=n_filtered, status=status)
+        P, rows, e, i32 = int(pq.numel()), st.rows, self._empty, torch.int32
+        return PairResults(pair_q=pq, pair_t=pt, out_off=st.row_off[:-1][pq.long()].contiguous(),
+                           top2_idx=e((rows, 2), i32), top2_d2=e((rows, 2), i32), surv=e((rows,), torch.uint8),
+                           m_idx=e((rows, 2), i32), m_pts=e((rows, 4), torch.float32), m_cnt=e((P,), i32),
+                           n_filtered=e((P,), i32), status=e((P,), i32))
+
+    def match(self, st: FrameStore, pair_q=None, pair_t=None, ratio=0.5, min_matching_pts=4, out=None) -> PairResults:
+        """K1 + K1b/K2 for the pairs (pair_q[p], pair_t[p]).  Per-row outputs of pair p start at
+        out_off[p] = row_off[pair_q[p]], so one call must not list the same query frame twice (the C ABI
+        takes out_off as an argument and has no such restriction).
+        out: a PairResults to write into instead of allocating (from `alloc_results`, or a `pairs` view of one); the pairs
+        and out_off are then its own, and pair_q / pair_t are not used."""
+        r = self._match_results(st, pair_q, pair_t) if out is None else out
+        P = int(r.pair_q.numel())
+        self._check(self.lib.evz_match_top2_d(self.h, _ptr(st.desc), int(st.d), _ptr(st.ckey), st.rows, _ptr(st.row_off),
+                                              _ptr(st.n_kp), _ptr(r.pair_q), _ptr(r.pair_t), _ptr(r.out_off), P,
+                                              _ptr(r.top2_idx), _ptr(r.top2_d2), self._stream()))
+        self._check(self.lib.evz_filter_matches(self.h, _ptr(r.top2_idx), _ptr(r.top2_d2), _ptr(st.coords), _ptr(st.canon),
+                                                _ptr(st.row_off), _ptr(st.n_kp), _ptr(r.pair_q), _ptr(r.pair_t), _ptr(r.out_off),
+                                                P, st.max_kp, float(ratio), int(min_matching_pts),
+                                                _ptr(r.surv), _ptr(r.m_idx), _ptr(r.m_pts), _ptr(r.m_cnt), _ptr(r.n_filtered),
+                                                _ptr(r.status), self._stream()))
+        return r
 
     # ------------------------------------------------------------------ K3 / K4
     def find_homography(self, pts, off, cnt, status, max_cnt, n_hyp=1024, seed=0, pair_id_base=0, level=1,
-                        thresh=3.0, min_inlier_frac=0.0, fail_status=_lib.ST_NO_MODEL_1, pre_H=None, light=False,
-                        pair_ids=None):
+                        thresh=3.0, min_inlier_frac=0.0, fail_status=_lib.ST_NO_MODEL_1, pre_H=None, pair_ids=None,
+                        out=None):
         """Batched seeded RANSAC + LM refit over the point lists pts[off[p]:off[p]+cnt[p]].
-        status is updated in place.  Returns dict(H, mask, inl_cnt, best_hyp, best_cnt, mask_best, H_best);
-        light=True skips the per-point masks and the diagnostics (H and inl_cnt only).
-        pair_ids: int64 [P] device tensor of sampler ids (pair p is seeded with pair_ids[p] instead of pair_id_base + p)."""
+        status is updated in place.  Returns dict(H, mask, inl_cnt, best_hyp, best_cnt, mask_best, H_best).
+        pair_ids: int64 [P] device tensor of sampler ids (pair p is seeded with pair_ids[p] instead of pair_id_base + p).
+        out: a dict of those tensors to write instead of allocating them; H and inl_cnt are required, an output left
+        out is not computed."""
         P = int(cnt.numel())
-        rows = int(pts.shape[0])
-        z = lambda shape, dt: torch.zeros(shape, dtype=dt, device=self.device)
-        out = dict(H=z((P, 9), torch.float64), inl_cnt=z((P,), torch.int32))
-        if light:
-            out.update(mask=None, best_hyp=None, best_cnt=None, mask_best=None, H_best=None)
-        else:
-            out.update(mask=z((rows,), torch.uint8), best_hyp=torch.full((P,), -1, dtype=torch.int32, device=self.device),
-                       best_cnt=z((P,), torch.int32), mask_best=z((rows,), torch.uint8), H_best=z((P, 9), torch.float64))
+        if out is None:
+            rows = int(pts.shape[0])
+            z = lambda shape, dt: torch.zeros(shape, dtype=dt, device=self.device)
+            out = dict(H=z((P, 9), torch.float64), inl_cnt=z((P,), torch.int32), mask=z((rows,), torch.uint8),
+                       best_hyp=torch.full((P,), -1, dtype=torch.int32, device=self.device), best_cnt=z((P,), torch.int32),
+                       mask_best=z((rows,), torch.uint8), H_best=z((P, 9), torch.float64))
         if pair_ids is not None:
             fn, ids = self.lib.evz_find_homography_ids, _ptr(pair_ids)
         else:
@@ -242,22 +280,23 @@ class GeometryEngine:
         self._check(fn(self.h, _ptr(pts), _ptr(off), _ptr(cnt), P, int(max_cnt), _ptr(pre_H),
                        int(n_hyp), int(seed) & 0xFFFFFFFF, ids, int(level),
                        float(thresh), float(min_inlier_frac), int(fail_status),
-                       _ptr(status), _ptr(out["H"]), _ptr(out["mask"]), _ptr(out["inl_cnt"]),
-                       _ptr(out["best_hyp"]), _ptr(out["best_cnt"]), _ptr(out["mask_best"]),
-                       _ptr(out["H_best"]), self._stream()))
+                       _ptr(status), _ptr(out["H"]), _ptr(out.get("mask")), _ptr(out["inl_cnt"]),
+                       _ptr(out.get("best_hyp")), _ptr(out.get("best_cnt")), _ptr(out.get("mask_best")),
+                       _ptr(out.get("H_best")), self._stream()))
         return out
 
     # ------------------------------------------------------------------ K5
-    def static_filter(self, pts, off, cnt, H, status, want_r=False, max_cnt=None):
-        """K5.  max_cnt: host-known upper bound of cnt (read back from the device when omitted)."""
+    def static_filter(self, pts, off, cnt, H, status, want_r=False, max_cnt=None, out=None):
+        """K5.  max_cnt: host-known upper bound of cnt (read back from the device when omitted).
+        out: (out_pts, out_cnt, best_r, flags) to write instead of allocating them."""
         P = int(cnt.numel())
         if max_cnt is None:
             max_cnt = int(cnt.max().item()) if P else 0
         r_out = self._empty((int(pts.shape[0]),), torch.int32) if want_r else None
-        out_pts = self._empty(tuple(pts.shape), torch.float32)
-        out_cnt = self._empty((P,), torch.int32)
-        best_r = self._empty((P,), torch.int32)
-        flags = self._empty((P,), torch.int32)
+        if out is None:
+            out = (self._empty(tuple(pts.shape), torch.float32), self._empty((P,), torch.int32),
+                   self._empty((P,), torch.int32), self._empty((P,), torch.int32))
+        out_pts, out_cnt, best_r, flags = out
         self._check(self.lib.evz_static_filter(self.h, _ptr(pts), _ptr(off), _ptr(cnt), P, int(max_cnt), _ptr(H), _ptr(status),
                                                _ptr(out_pts), _ptr(out_cnt), _ptr(best_r), _ptr(flags), _ptr(r_out),
                                                self._stream()))
@@ -282,22 +321,11 @@ class GeometryEngine:
 
     # ------------------------------------------------------------------ whole per-pair path
     def process_pairs(self, st: FrameStore, pair_q, pair_t, n_hyp=1024, seed=0, pair_id_base=0,
-                      ratio=0.5, thresh=3.0, min_matching_pts=4, pre_H=None) -> PairResults:
+                      ratio=0.5, thresh=3.0, min_matching_pts=4) -> PairResults:
         """match_static_kps + compute_homography for every pair (reference matching.py:131-163,
         utils.py:328-363), all on the device."""
-        r = self.match(st, pair_q, pair_t, ratio, min_matching_pts)
-        mk = st.max_kp
-        h1 = self.find_homography(r.m_pts, r.out_off, r.m_cnt, r.status, mk, n_hyp, seed, pair_id_base, 1, thresh,
-                                  0.0, _lib.ST_NO_MODEL_1)
-        r.H1, r.mask1, r.mask1_best, r.best_hyp1, r.best_cnt1, r.inl1 = (h1["H"], h1["mask"], h1["mask_best"],
-                                                                      h1["best_hyp"], h1["best_cnt"], h1["inl_cnt"])
-        r.extra["H1_best"] = h1["H_best"]
-        r.static_pts, r.static_cnt, r.static_r, r.flags = self.static_filter(r.m_pts, r.out_off, r.m_cnt, r.H1, r.status, max_cnt=mk)
-        h2 = self.find_homography(r.static_pts, r.out_off, r.static_cnt, r.status, mk, n_hyp, seed, pair_id_base, 2,
-                                  thresh, 0.7, _lib.ST_NO_MODEL_2, pre_H=pre_H)
-        r.H, r.mask2, r.mask2_best, r.best_hyp2, r.best_cnt2, r.inl2 = (h2["H"], h2["mask"], h2["mask_best"],
-                                                                     h2["best_hyp"], h2["best_cnt"], h2["inl_cnt"])
-        r.extra["H2_best"] = h2["H_best"]
+        r = self.alloc_results(st, pair_q, pair_t)
+        self._pairs_range(st, r, 0, int(r.pair_q.numel()), n_hyp, seed, pair_id_base, ratio, thresh, min_matching_pts)
         return r
 
     # ------------------------------------------------------------------ K6 / K7
@@ -353,17 +381,13 @@ class GeometryEngine:
         # pinned + non_blocking: the set-up does not synchronise with the host either
         ids = torch.from_numpy(np.repeat(np.arange(K, dtype=np.int64), np.diff(step_off))).pin_memory()
         ids = ids.to(self.device, non_blocking=True)
-        lib, h, strm = self.lib, self.h, self._stream()
-        at = lambda t, p0, k=1: C.c_void_p(t.data_ptr() + int(p0) * k * t.element_size())
-        for k in range(len(step_off) - 1):
+        for k in range(K):
             a, b = int(step_off[k]), int(step_off[k + 1])
-            self._check(lib.evz_find_homography_ids(h, _ptr(pts), at(off, a), at(cnt, a), b - a, int(max_cnt),
-                                                    None if k == 0 else _ptr(S_state), int(n_hyp), int(seed) & 0xFFFFFFFF,
-                                                    at(ids, a), 2, float(thresh), float(min_inlier_frac), int(fail_status),
-                                                    at(status, a), at(H2, a, 9), None, at(inl, a), None, None, None, None, strm))
-            self._check(lib.evz_chain_ref_step(h, at(H2, a, 9), at(status, a), b - a, 1 if k == 0 else 0, 1 if policy else 0,
-                                               _ptr(S_state), None if k == 0 else at(H_out, step_off[k - 1], 9), at(H_out, a, 9),
-                                               strm))
+            H2_k, status_k, prev = H2[a:b], status[a:b], int(step_off[k - 1]) if k else 0
+            self.find_homography(pts, off[a:b], cnt[a:b], status_k, max_cnt, n_hyp, seed, 0, 2, thresh, min_inlier_frac,
+                                 fail_status, pre_H=S_state if k else None, pair_ids=ids[a:b],
+                                 out=dict(H=H2_k, inl_cnt=inl[a:b]))
+            self.chain_ref_step(H2_k, status_k, k == 0, policy, S_state, H_out[prev:prev + b - a] if k else None, H_out[a:b])
         return H_out
 
     def chain_seed_apply(self, summaries, rank, S, policy=True, want_fixed=True):
@@ -396,54 +420,28 @@ class GeometryEngine:
     # ------------------------------------------------------------------ video-level driver
     def _pairs_range(self, st: FrameStore, r: PairResults, p0: int, p1: int, n_hyp, seed, pair_id_base, ratio, thresh,
                      min_matching_pts=4, after_match=None):
-        """match_static_kps + compute_homography for pairs [p0, p1) of an already allocated PairResults
-        (device pointers offset into the per-pair arrays; per-row arrays are addressed through out_off)."""
-        n = p1 - p0
-        if n <= 0:
+        """match_static_kps + compute_homography for pairs [p0, p1) of an already allocated PairResults, written through a
+        `pairs` view of it."""
+        if p1 <= p0:
             return
-        lib, h, strm = self.lib, self.h, self._stream()
-        mk = st.max_kp
-        at = lambda t, k=1: C.c_void_p(t.data_ptr() + p0 * k * t.element_size())
-        self._check(lib.evz_match_top2_d(h, _ptr(st.desc), int(st.d), _ptr(st.ckey), st.rows, _ptr(st.row_off), _ptr(st.n_kp),
-                                         at(r.pair_q), at(r.pair_t), at(r.out_off), n, _ptr(r.top2_idx), _ptr(r.top2_d2), strm))
-        self._check(lib.evz_filter_matches(h, _ptr(r.top2_idx), _ptr(r.top2_d2), _ptr(st.coords), _ptr(st.canon),
-                                           _ptr(st.row_off), _ptr(st.n_kp), at(r.pair_q), at(r.pair_t), at(r.out_off), n,
-                                           mk, float(ratio), int(min_matching_pts), _ptr(r.surv), _ptr(r.m_idx), _ptr(r.m_pts),
-                                           at(r.m_cnt), at(r.n_filtered), at(r.status), strm))
+        v, mk = r.pairs(p0, p1), st.max_kp
+        self.match(st, ratio=ratio, min_matching_pts=min_matching_pts, out=v)
         if after_match is not None:
             after_match()
-        self._check(lib.evz_find_homography(h, _ptr(r.m_pts), at(r.out_off), at(r.m_cnt), n, mk, None, int(n_hyp),
-                                            int(seed) & 0xFFFFFFFF, int(pair_id_base) + p0, 1, float(thresh), 0.0,
-                                            _lib.ST_NO_MODEL_1, at(r.status), at(r.H1, 9), _ptr(r.mask1), at(r.inl1),
-                                            at(r.best_hyp1), at(r.best_cnt1), _ptr(r.mask1_best), at(r.extra["H1_best"], 9), strm))
-        self._check(lib.evz_static_filter(h, _ptr(r.m_pts), at(r.out_off), at(r.m_cnt), n, mk, at(r.H1, 9), at(r.status),
-                                          _ptr(r.static_pts), at(r.static_cnt), at(r.static_r), at(r.flags), None, strm))
-        self._check(lib.evz_find_homography(h, _ptr(r.static_pts), at(r.out_off), at(r.static_cnt), n, mk, None, int(n_hyp),
-                                            int(seed) & 0xFFFFFFFF, int(pair_id_base) + p0, 2, float(thresh), 0.7,
-                                            _lib.ST_NO_MODEL_2, at(r.status), at(r.H, 9), _ptr(r.mask2), at(r.inl2),
-                                            at(r.best_hyp2), at(r.best_cnt2), _ptr(r.mask2_best), at(r.extra["H2_best"], 9), strm))
+        self.find_homography(v.m_pts, v.out_off, v.m_cnt, v.status, mk, n_hyp, seed, int(pair_id_base) + p0, 1, thresh, 0.0,
+                             _lib.ST_NO_MODEL_1, out=dict(H=v.H1, mask=v.mask1, inl_cnt=v.inl1, best_hyp=v.best_hyp1,
+                                                          best_cnt=v.best_cnt1, mask_best=v.mask1_best, H_best=v.extra["H1_best"]))
+        self.static_filter(v.m_pts, v.out_off, v.m_cnt, v.H1, v.status, max_cnt=mk, out=(v.static_pts, v.static_cnt, v.static_r, v.flags))
+        self.find_homography(v.static_pts, v.out_off, v.static_cnt, v.status, mk, n_hyp, seed, int(pair_id_base) + p0, 2, thresh,
+                             0.7, _lib.ST_NO_MODEL_2, out=dict(H=v.H, mask=v.mask2, inl_cnt=v.inl2, best_hyp=v.best_hyp2,
+                                                               best_cnt=v.best_cnt2, mask_best=v.mask2_best, H_best=v.extra["H2_best"]))
 
     def alloc_results(self, st: FrameStore, pair_q, pair_t) -> PairResults:
         """Workspace for `process_pairs_into`: every per-pair / per-row output of the path, allocated once."""
-        pq = torch.as_tensor(pair_q, dtype=torch.int32).to(self.device)
-        pt = torch.as_tensor(pair_t, dtype=torch.int32).to(self.device)
-        return self._alloc_results(st, pq, pt)
-
-    def process_pairs_into(self, st: FrameStore, r: PairResults, n_hyp=1024, seed=0, pair_id_base=0, ratio=0.5, thresh=3.0,
-                           after_match=None) -> PairResults:
-        """`process_pairs` into a workspace from `alloc_results`: no allocation, no memset, nothing but the kernels of the
-        path on the current stream (what a steady-state caller -- and bench.py's timed region -- runs per batch).
-        after_match: optional callable invoked between the match stage and the first RANSAC (event recording)."""
-        self._pairs_range(st, r, 0, int(r.pair_q.numel()), n_hyp, seed, pair_id_base, ratio, thresh, after_match=after_match)
-        return r
-
-    def _alloc_results(self, st: FrameStore, pq, pt) -> PairResults:
-        P, rows = int(pq.numel()), st.rows
+        r = self._match_results(st, pair_q, pair_t)
+        P, rows = int(r.pair_q.numel()), st.rows
         e, z = self._empty, lambda shape, dt: torch.zeros(shape, dtype=dt, device=self.device)
         i32, u8, f64 = torch.int32, torch.uint8, torch.float64
-        r = PairResults(pair_q=pq, pair_t=pt, out_off=st.row_off[:-1][pq.long()].contiguous(),
-                        top2_idx=e((rows, 2), i32), top2_d2=e((rows, 2), i32), surv=e((rows,), u8), m_idx=e((rows, 2), i32),
-                        m_pts=e((rows, 4), torch.float32), m_cnt=e((P,), i32), n_filtered=e((P,), i32), status=e((P,), i32))
         r.H1, r.H = z((P, 9), f64), z((P, 9), f64)
         r.mask1, r.mask1_best, r.mask2, r.mask2_best = z((rows,), u8), z((rows,), u8), z((rows,), u8), z((rows,), u8)
         r.inl1, r.inl2, r.best_cnt1, r.best_cnt2 = z((P,), i32), z((P,), i32), z((P,), i32), z((P,), i32)
@@ -454,6 +452,14 @@ class GeometryEngine:
         r.static_r, r.flags = e((P,), i32), e((P,), i32)
         return r
 
+    def process_pairs_into(self, st: FrameStore, r: PairResults, n_hyp=1024, seed=0, pair_id_base=0, ratio=0.5, thresh=3.0,
+                           after_match=None) -> PairResults:
+        """`process_pairs` into a workspace from `alloc_results`: no allocation, no memset, nothing but the kernels of the
+        path on the current stream (what a steady-state caller -- and bench.py's timed region -- runs per batch).
+        after_match: optional callable invoked between the match stage and the first RANSAC (event recording)."""
+        self._pairs_range(st, r, 0, int(r.pair_q.numel()), n_hyp, seed, pair_id_base, ratio, thresh, after_match=after_match)
+        return r
+
     def video_geometry(self, desc, coords, n_kp=None, n_hyp=1024, seed=0, none_h_processing=True,
                        ratio=0.5, thresh=3.0, pair_id_base=0, chunk_frames=None):
         """Frame chain -> per-pair G, status, cumulative S and fixed-plane H (parallel formulation).
@@ -462,65 +468,37 @@ class GeometryEngine:
         Host input is streamed: frames are copied to the device in chunks on a copy stream while the
         compute stream ingests and processes the pairs of the chunks that have already landed, so the
         PCIe transfer (the end-to-end bound: 136 bytes per keypoint) overlaps the kernels."""
-        desc_t, coords_t = torch.as_tensor(desc), torch.as_tensor(coords)
-        if desc_t.dim() == 3:
-            f, n, d = desc_t.shape
-            if n_kp is None:
-                n_kp = np.full(f, n, np.int64)
-            desc_t, coords_t = desc_t.reshape(f * n, d), coords_t.reshape(f * n, 2)
-        if n_kp is None:
-            raise ValueError("n_kp is required for concatenated input")
-        n_kp_h = np.asarray(n_kp, np.int64)
+        desc_t, coords_t, n_kp_h, d, is_f32 = self._frames_input(desc, coords, n_kp)
         F = len(n_kp_h)
         if chunk_frames is None:
             chunk_frames = max(64, -(-F // 16))
-        if desc_t.is_cuda or F <= chunk_frames or desc_t.dtype not in (torch.uint8, torch.float32):
+        if desc_t.is_cuda or F <= chunk_frames:
             # small or device-resident input: one ingest, one batch
             st = self.ingest(desc_t, coords_t, n_kp_h)
-            pq = torch.arange(1, F, dtype=torch.int32)
-            pt = torch.arange(0, F - 1, dtype=torch.int32)
-            r = self.process_pairs(st, pq, pt, n_hyp, seed, pair_id_base, ratio, thresh)
+            r = self.process_pairs(st, torch.arange(1, F, dtype=torch.int32), torch.arange(0, F - 1, dtype=torch.int32),
+                                   n_hyp, seed, pair_id_base, ratio, thresh)
         else:
-            st, r = self._video_streamed(desc_t, coords_t, n_kp_h, chunk_frames, n_hyp, seed, pair_id_base, ratio, thresh)
+            st, r = self._video_streamed(desc_t, coords_t, n_kp_h, d, is_f32, chunk_frames, n_hyp, seed, pair_id_base,
+                                         ratio, thresh)
         S, Hf, _ = self.chain_scan(r.H, r.status, none_h_processing)
         return dict(G=r.H.cpu().numpy().reshape(-1, 3, 3), status=r.status.cpu().numpy(),
                     S=S.cpu().numpy().reshape(-1, 3, 3), H_fixed=Hf.cpu().numpy().reshape(-1, 3, 3), results=r, store=st)
 
-    def _video_streamed(self, desc_t, coords_t, n_kp_h, chunk_frames, n_hyp, seed, pair_id_base, ratio, thresh):
-        if int(n_kp_h.sum()) != desc_t.shape[0] or coords_t.shape[0] != desc_t.shape[0]:
-            raise ValueError("n_kp does not add up to the number of descriptor rows")
-        if int(n_kp_h.max()) > EVZ_MAX_KP:
-            raise ValueError(f"at most {EVZ_MAX_KP} keypoints per frame are supported")
-        d = int(desc_t.shape[1])
-        if d > EVZ_DESC_BYTES or d % 4:
-            raise ValueError("descriptor width must be a multiple of 4 and at most 128")
-        is_f32 = 1 if desc_t.dtype == torch.float32 else 0
+    def _video_streamed(self, desc_t, coords_t, n_kp_h, d, is_f32, chunk_frames, n_hyp, seed, pair_id_base, ratio, thresh):
         coords_t = coords_t.to(torch.float32)
         F = len(n_kp_h)
         dev = self.device
-        row_off_h = self.layout(n_kp_h)
-        raw_off_h = np.zeros(F + 1, np.int64)
-        np.cumsum(n_kp_h, out=raw_off_h[1:])
-        rows = int(row_off_h[-1])
         compute = torch.cuda.current_stream(dev)
         if getattr(self, "_copy_stream", None) is None:
             self._copy_stream = torch.cuda.Stream(dev)
         copy = self._copy_stream
-        raw_off = torch.from_numpy(raw_off_h).to(dev, non_blocking=True)
-        row_off = torch.from_numpy(row_off_h).to(dev, non_blocking=True)
-        n_kp_d = torch.from_numpy(n_kp_h.astype(np.int32)).to(dev, non_blocking=True)
-        bad = torch.zeros(1, dtype=torch.int32, device=dev)
+        st, raw_off_h, raw_off, bad = self._new_store(n_kp_h, d)
         desc_raw = torch.empty(desc_t.shape, dtype=desc_t.dtype, device=dev)
         coords_raw = torch.empty(coords_t.shape, dtype=torch.float32, device=dev)
-        st = FrameStore(desc=self._empty((rows, EVZ_DESC_BYTES), torch.uint8), ckey=self._empty((rows,), torch.int32),
-                        coords=self._empty((rows, 2), torch.float32), canon=self._empty((rows,), torch.int32),
-                        row_off=row_off, n_kp=n_kp_d, row_off_h=row_off_h, n_kp_h=n_kp_h.astype(np.int32), d=d,
-                        keep=(desc_raw, coords_raw, raw_off, bad))
-        pq = torch.arange(1, F, dtype=torch.int32, device=dev)
-        pt = torch.arange(0, F - 1, dtype=torch.int32, device=dev)
-        r = self._alloc_results(st, pq, pt)
+        st.keep += (desc_raw, coords_raw)
+        r = self.alloc_results(st, torch.arange(1, F, dtype=torch.int32, device=dev),
+                               torch.arange(0, F - 1, dtype=torch.int32, device=dev))
         copy.wait_stream(compute)            # the staging buffers were allocated on the compute stream
-        off8 = lambda t, k: C.c_void_p(t.data_ptr() + k * t.element_size())
         for f0 in range(0, F, chunk_frames):
             f1 = min(F, f0 + chunk_frames)
             a, b = int(raw_off_h[f0]), int(raw_off_h[f1])
@@ -530,15 +508,11 @@ class GeometryEngine:
                     coords_raw[a:b].copy_(coords_t[a:b], non_blocking=True)
                 landed = copy.record_event()
             compute.wait_event(landed)
-            if row_off_h[f1] > row_off_h[f0]:
-                self._check(self.lib.evz_ingest(self.h, _ptr(desc_raw), is_f32, d, _ptr(coords_raw), off8(raw_off, f0),
-                                                off8(row_off, f0), f1 - f0, _ptr(st.desc), _ptr(st.ckey), _ptr(st.coords),
-                                                _ptr(st.canon), _ptr(bad), self._stream()))
+            self._ingest_frames(st, desc_raw, coords_raw, raw_off, is_f32, bad, f0, f1)
             # pairs whose query frame is in this chunk (their train frame landed with this or an earlier chunk)
             self._pairs_range(st, r, max(f0, 1) - 1, f1 - 1, n_hyp, seed, pair_id_base, ratio, thresh)
         desc_raw.record_stream(copy); coords_raw.record_stream(copy)
         st.keep = (bad,)                     # every consumer of the raw staging copies is enqueued: let them go
-        if is_f32 and int(bad.item()):
-            raise ValueError(f"{int(bad.item())} descriptor values are not integers in [0,255]; "
-                             "the int8 tensor-core matcher is exact only for SIFT/ORB-style descriptors")
+        if is_f32:
+            self._check_integer_descriptors(bad)
         return st, r

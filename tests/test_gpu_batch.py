@@ -1,5 +1,6 @@
 """Many videos per call: evz_find_homography_ids, evz_chain_scan_segments, evz_chain_ref_step and
-geometry_from_features_batch / get_homography_dicts against the one-video calls.  Needs a B200."""
+geometry_from_features_batch / get_homography_dicts against the one-video calls and, in reference mode, against a
+host-loop chain.  Needs a B200."""
 import ctypes as C
 import os
 from fractions import Fraction
@@ -48,7 +49,7 @@ def _fma_dot(H, S):
 @pytest.fixture(scope="module")
 def blas_is_fma_order():
     """Does this host's np.dot on 3x3 f64 round like the device chain step?  Then the reference-mode chains must match
-    the single-video host loop bit for bit; otherwise only to the tolerance of the existing tests."""
+    the host loop (`_host_reference_chain`) bit for bit; otherwise only to the tolerance of the existing tests."""
     rng = np.random.default_rng(7)
     for _ in range(300):
         H, S = rng.normal(size=(3, 3)), rng.normal(size=(3, 3)) * 100
@@ -78,6 +79,46 @@ def _same(got, want, mode, bitwise_ref):
         assert all(np.array_equal(a, b) for a, b in zip(H_g, H_w))
     else:
         assert _chain_px(H_g, H_w) < 1e-2
+
+
+def _host_reference_chain(engine, feats, policy, n_hyp, seed):
+    """The reference chain of one video as a host loop (reference video_processing.py:67-105), independent of the device
+    chain step: RANSAC #2 of pair k alone (sampler id k) with pre_H = the running superposition S, the None-H policy,
+    then S = np.dot(H, S) / S[2][2] on the host.  The level-2 input is the driver's.  Returns (H_list, status)."""
+    from evenvizion_b200 import _lib
+    from evenvizion_b200.processing import video_processing as vp
+    from evenvizion_b200.processing.constants import LENGTH_ACCOUNTED_POINTS, THRESHOLD_FOR_FIND_HOMOGRAPHY
+    P = max(len(next(iter(feats.values()))) - 1, 0)
+    if P == 0:
+        return [], np.zeros(0, np.int32)
+    dev = engine.device
+    lay = vp.PairLayout([P], step_major=True)
+    pts2, off2, cnt2, status, max_cnt = vp._level2_input(engine, [feats], lay, torch.from_numpy(lay.k).to(dev), n_hyp, seed)
+    st_out = status.cpu().numpy().copy()
+    H_list, S, H_prev = [], None, None
+    for k in range(P):
+        H = None
+        if st_out[k] == 0:
+            s_k = torch.zeros(1, dtype=torch.int32, device=dev)
+            pre = None if S is None else torch.from_numpy(np.asarray(S, np.float64).reshape(1, 9)).to(dev)
+            out = dict(H=torch.zeros((1, 9), dtype=torch.float64, device=dev), inl_cnt=torch.zeros(1, dtype=torch.int32, device=dev))
+            engine.find_homography(pts2, off2[k:k + 1], cnt2[k:k + 1], s_k, max_cnt, n_hyp, seed, k, 2,
+                                   THRESHOLD_FOR_FIND_HOMOGRAPHY, LENGTH_ACCOUNTED_POINTS, _lib.ST_NO_MODEL_2, pre_H=pre, out=out)
+            st_out[k] = int(s_k[0])
+            if st_out[k] == 0:
+                H = out["H"][0].cpu().numpy().reshape(3, 3)
+        if H is None:
+            H = H_prev if policy else None                 # the reference reuses the previous pair's matrix (:95-96)
+            if H is None:
+                H = np.eye(3)                              # README.md:45: no transformation on this frame
+        H_list.append(H)
+        if k == 0:
+            S = H
+        else:
+            S = np.dot(H, S)
+            S = S / S[2][2]
+        H_prev = H
+    return H_list, st_out
 
 
 # ------------------------------------------------------------------------------------------------ C ABI / engine
@@ -177,7 +218,8 @@ def test_chain_scan_segments_bit_identical_per_segment(engine, policy):
 
 
 def _ref_step_host(H2, ok, sizes, policy):
-    """video_processing.py:119-149 restated per chain, with the product in the stated fma order."""
+    """The reference's host loop body (video_processing.py:84-105) restated per chain, with the product in the stated fma
+    order."""
     out = np.empty_like(H2)
     S, Hp = [None] * sizes[0], [None] * sizes[0]
     p = 0
@@ -291,12 +333,13 @@ def test_batch_parallel_bit_identical_to_single(proc, clip, types):
 
 @pytest.mark.parametrize("types", [("SIFT", "ORB"), ("SIFT",)])
 @pytest.mark.parametrize("policy", [True, False])
-def test_batch_reference_matches_single_and_oracle(proc, clip, types, policy, blas_is_fma_order):
+def test_batch_reference_matches_single_and_oracle(engine, proc, clip, types, policy, blas_is_fma_order):
     feats = [_clip_feats(clip, types, a, b) for a, b in SPLITS]
     got = proc.geometry_from_features_batch(feats, policy, "reference", n_hyp=1024, seed=0)
     for (a, b), f, g in zip(SPLITS, feats, got):
         single = proc.geometry_from_features(f, policy, "reference", n_hyp=1024, seed=0)
-        _same(g, single, "reference", blas_is_fma_order)
+        _same(g, single, "reference", True)                   # a batch of one: batching changes nothing
+        _same(g, _host_reference_chain(engine, f, policy, 1024, 0), "reference", blas_is_fma_order)
         if b - a < 2:
             continue
         ref = _oracle(clip, types, a, b, policy)
@@ -325,7 +368,7 @@ def _synth_feats(n_frames, n_kp, seed, unmatched_frac=0.0):
 
 
 @pytest.mark.parametrize("mode", ["parallel", "reference"])
-def test_batch_failures_stay_inside_their_video(proc, clip, mode, blas_is_fma_order):
+def test_batch_failures_stay_inside_their_video(engine, proc, clip, mode, blas_is_fma_order):
     a = _clip_feats(clip, ("SIFT", "ORB"), 0, 12)
     a["ORB"][5] = (a["ORB"][5][0], None)                      # a frame without descriptors
     b = _synth_feats(25, 600, 3, unmatched_frac=0.3)          # pairs without any correspondence
@@ -338,13 +381,15 @@ def test_batch_failures_stay_inside_their_video(proc, clip, mode, blas_is_fma_or
         gb = proc.geometry_from_features_batch([b2, b2], policy, mode, n_hyp=512, seed=2)
         for f, g in [(a, got[0]), (c, got[1]), (a, got[2]), (b2, gb[0])]:
             single = proc.geometry_from_features(f, policy, mode, n_hyp=512, seed=2)
-            _same(g, single, mode, blas_is_fma_order)
+            _same(g, single, mode, True)
+            if mode == "reference":
+                _same(g, _host_reference_chain(engine, f, policy, 512, 2), mode, blas_is_fma_order)
         assert got[1][1][0] != 0 and (gb[0][1] != 0).any()
         assert np.array_equal(got[1][0][0], np.eye(3))         # a failed first pair is an identity step
 
 
 @pytest.mark.parametrize("mode", ["parallel", "reference"])
-def test_batch_scale_64_videos(proc, mode, blas_is_fma_order):
+def test_batch_scale_64_videos(engine, proc, mode, blas_is_fma_order):
     from evenvizion_b200 import synth
     ch = synth.make_chain(64 * 30, 2048, seed=21, device="cuda", unmatched_frac=0.02)
     d, c = ch["desc"].cpu().numpy(), ch["coords"].cpu().numpy()
@@ -352,7 +397,9 @@ def test_batch_scale_64_videos(proc, mode, blas_is_fma_order):
     got = proc.geometry_from_features_batch(feats, True, mode, n_hyp=256, seed=4)
     assert len(got) == 64 and all(len(g[0]) == 29 for g in got)
     for v in (0, 17, 40, 63):
-        _same(got[v], proc.geometry_from_features(feats[v], True, mode, n_hyp=256, seed=4), mode, blas_is_fma_order)
+        _same(got[v], proc.geometry_from_features(feats[v], True, mode, n_hyp=256, seed=4), mode, True)
+        if mode == "reference":
+            _same(got[v], _host_reference_chain(engine, feats[v], True, 256, 4), mode, blas_is_fma_order)
 
 
 class _FakeCapture:
@@ -366,7 +413,7 @@ class _FakeCapture:
         return True, self.frames[self.i - 1].copy()
 
 
-def test_get_homography_dicts_equals_per_capture(proc, clip, blas_is_fma_order):
+def test_get_homography_dicts_equals_per_capture(engine, proc, clip, blas_is_fma_order):
     pytest.importorskip("cv2")
     fr = [[clip[f"frame{f}"] for f in range(6)], [clip[f"frame{f}"] for f in range(2, 5)]]
     got = proc.get_homography_dicts([_FakeCapture(x) for x in fr], n_hyp=1024, seed=0)
@@ -375,8 +422,10 @@ def test_get_homography_dicts_equals_per_capture(proc, clip, blas_is_fma_order):
         want = proc.get_homography_dict(_FakeCapture(x), n_hyp=1024, seed=0)
         assert list(g) == list(want) and g["resize_info"] == want["resize_info"]
         Hg = [g[k]["H"] for k in g if k != "resize_info"]
-        Hw = [want[k]["H"] for k in want if k != "resize_info"]
+        assert Hg == [want[k]["H"] for k in want if k != "resize_info"]
+        feats, _ = proc.read_and_describe(_FakeCapture(x))
+        Hh = [np.asarray(H, np.float64).tolist() for H in _host_reference_chain(engine, feats, True, 1024, 0)[0]]
         if blas_is_fma_order:
-            assert Hg == Hw
+            assert Hg == Hh
         else:
-            assert _chain_px(Hg, Hw) < 1e-2
+            assert _chain_px(Hg, Hh) < 1e-2
