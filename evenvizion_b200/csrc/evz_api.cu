@@ -84,6 +84,7 @@ int evz_scratch(evz_handle* h, size_t bytes, void** out) {
         const size_t want = evz_align_up(bytes + bytes / 4, size_t(1) << 20);
         cudaError_t e = cudaMalloc(&h->scratch, want);
         if (e != cudaSuccess) {
+            (void)cudaGetLastError();          // reported here, not again by the next launch check
             EVZ_SET_ERR(h, "scratch allocation of %zu bytes failed: %s", want, cudaGetErrorString(e));
             return EVZ_E_NOMEM;
         }

@@ -27,7 +27,8 @@ struct evz_handle {
     // cudaFuncSetAttribute(MaxDynamicSharedMemorySize) is per device: remembered per handle, not per process
     unsigned attr_match = 0;       // bit 0: key-space kernel, bit 1: V-space kernel
     bool attr_static = false, attr_canon = false, attr_concat = false;
-    int attr_filter = 0, attr_score = 0, attr_refit = 0;
+    int attr_filter = 0, attr_score = 0, attr_score_g = 0, attr_refit = 0;
+    int score_smem_room = -1;      // dynamic shared memory a scoring block may take (-1: not queried yet)
     // options (evz_set_option)
     int opt_ransac_exact = 0;
     int opt_ransac_no_prune = 0;
@@ -41,9 +42,11 @@ struct evz_handle {
 
 #define EVZ_SET_ERR(h, ...) do { if (h) snprintf((h)->err, sizeof((h)->err), __VA_ARGS__); } while (0)
 
+// A failure is reported once: the runtime's last-error state is cleared, so that the next cudaGetLastError() -- the
+// launch check of a later call, or PyTorch's -- does not report it again against unrelated work.
 #define EVZ_CUDA_CHECK(h, expr) do { cudaError_t e__ = (expr); if (e__ != cudaSuccess) {            \
         EVZ_SET_ERR(h, "%s:%d: %s -> %s", __FILE__, __LINE__, #expr, cudaGetErrorString(e__));        \
-        return EVZ_E_CUDA; } } while (0)
+        (void)cudaGetLastError(); return EVZ_E_CUDA; } } while (0)
 
 #define EVZ_LAUNCH_CHECK(h) EVZ_CUDA_CHECK(h, cudaGetLastError())
 

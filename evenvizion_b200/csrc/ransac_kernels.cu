@@ -704,13 +704,18 @@ __device__ __forceinline__ bool first_perfect_search(const FhArgs& a, const floa
 
 
 // dynamic shared memory of the scoring kernel: float4 pts[max_cnt] | u16 pos[max_cnt (rounded up to 8)] |
-// u16 vlist, slist, lo_s, hi_s [n_hyp] each
+// u16 vlist, slist, lo_s, hi_s [n_hyp] each.  kGlobalLists: the four hypothesis lists are the pair's slice
+// glists + 4 n_hyp p of handle scratch instead (chosen by the host when they do not fit in shared memory next to the
+// points: 12 288 points leave room for 944 hypotheses).  Only the block's own threads touch its slice, and every
+// cross-thread hand-over in this kernel already passes a __syncthreads, which orders global memory as well.
+template <bool kGlobalLists>
 __global__ void __launch_bounds__(kRsThreads, 4)
-ransac_score_kernel(const FhArgs a, double* __restrict__ Hbest_out, int32_t* __restrict__ phase) {
+ransac_score_kernel(const FhArgs a, double* __restrict__ Hbest_out, int32_t* __restrict__ phase, uint16_t* glists) {
     extern __shared__ __align__(16) uint8_t fh_smem[];
     float4* pts = reinterpret_cast<float4*>(fh_smem);
     uint16_t* pos = reinterpret_cast<uint16_t*>(fh_smem + static_cast<size_t>(a.max_cnt) * 16);      // sample index -> position in pts
-    uint16_t* vlist = pos + ((a.max_cnt + 7) & ~7);                                                   // valid hypotheses
+    uint16_t* vlist = kGlobalLists ? glists + static_cast<size_t>(blockIdx.x) * 4 * a.n_hyp           // valid hypotheses
+                                   : pos + ((a.max_cnt + 7) & ~7);
     uint16_t* slist = vlist + a.n_hyp;                                                                // survivors to rescore
     uint16_t* lo_s = slist + a.n_hyp;                                                                 // count bounds per valid slot
     uint16_t* hi_s = lo_s + a.n_hyp;
@@ -1304,6 +1309,7 @@ static int find_homography(const char* fn, evz_handle* h, const float* pts, cons
                            void* stream) {
     FH_REQUIRE(pts && off && cnt && status && H, "null pointer");
     FH_REQUIRE(n_hyp > 0, "n_hyp must be positive");
+    FH_REQUIRE(n_hyp <= 65535, "n_hyp must be below 65536");
     FH_REQUIRE((reinterpret_cast<uintptr_t>(pts) & 15) == 0, "pts must be 16-byte aligned");
     if (max_cnt > EVZ_MAX_KP) {
         EVZ_SET_ERR(h, "%s: max_cnt %d exceeds the supported %d points per pair", fn, max_cnt, EVZ_MAX_KP);
@@ -1312,24 +1318,39 @@ static int find_homography(const char* fn, evz_handle* h, const float* pts, cons
     if (n_pairs <= 0) return EVZ_OK;
     if (max_cnt < 4) max_cnt = 4;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    // scratch: phase[P] | H_best[P][9] when the caller does not want it
+    // the scoring kernel keeps its four u16 hypothesis lists (8 B per hypothesis) in shared memory when they fit next to
+    // the points, else in handle scratch; the room is the device's per-block opt-in limit less the kernel's static part
+    if (h->score_smem_room < 0) {
+        int optin = 0;
+        cudaFuncAttributes fa;
+        EVZ_CUDA_CHECK(h, cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, h->device));
+        EVZ_CUDA_CHECK(h, cudaFuncGetAttributes(&fa, evz::ransac_score_kernel<false>));
+        h->score_smem_room = optin - static_cast<int>(fa.sharedSizeBytes);
+    }
+    const int smem_pts = max_cnt * 16 + ((max_cnt + 7) & ~7) * 2 + 16;
+    const bool glists = smem_pts + 8 * n_hyp > h->score_smem_room;
+    const int smem_score = glists ? smem_pts : smem_pts + 8 * n_hyp;
+    // scratch: phase[P] | H_best[P][9] when the caller does not want it | hypothesis lists | model cache
     void* scr = nullptr;
     const size_t ph_bytes = evz_align_up(static_cast<size_t>(n_pairs) * 4, 256);
     const size_t hb_bytes = evz_align_up(H_best ? 0 : static_cast<size_t>(n_pairs) * 72, 256);
+    const size_t hl_bytes = glists ? evz_align_up(static_cast<size_t>(n_pairs) * static_cast<size_t>(n_hyp) * 8, 256) : 0;
     // model cache of the scoring kernel (hyp_model): 32 bytes per hypothesis, written and read by the pair's own CTA
     size_t hc_bytes = static_cast<size_t>(n_pairs) * static_cast<size_t>(n_hyp) * 32;
     if (hc_bytes > (size_t(4) << 30) || h->opt_ransac_exact) hc_bytes = 0;
-    int rc = evz_scratch(h, ph_bytes + hb_bytes + hc_bytes + 256, &scr);
+    int rc = evz_scratch(h, ph_bytes + hb_bytes + hl_bytes + hc_bytes + 256, &scr);
     if (rc) return rc;
+    uint8_t* scr8 = static_cast<uint8_t*>(scr);
     int32_t* phase = static_cast<int32_t*>(scr);
-    double* hb = H_best ? H_best : reinterpret_cast<double*>(static_cast<uint8_t*>(scr) + ph_bytes);
-    float4* hcache = hc_bytes ? reinterpret_cast<float4*>(static_cast<uint8_t*>(scr) + ph_bytes + hb_bytes) : nullptr;
-    FH_REQUIRE(n_hyp <= 65535, "n_hyp must be below 65536");
-    const int smem_score = max_cnt * 16 + ((max_cnt + 7) & ~7) * 2 + 8 * n_hyp + 16;
+    double* hb = H_best ? H_best : reinterpret_cast<double*>(scr8 + ph_bytes);
+    uint16_t* hlists = glists ? reinterpret_cast<uint16_t*>(scr8 + ph_bytes + hb_bytes) : nullptr;
+    float4* hcache = hc_bytes ? reinterpret_cast<float4*>(scr8 + ph_bytes + hb_bytes + hl_bytes) : nullptr;
     const int smem_refit = max_cnt * 17 + 16;
-    if (smem_score > h->attr_score) {
-        EVZ_CUDA_CHECK(h, cudaFuncSetAttribute(evz::ransac_score_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_score));
-        h->attr_score = smem_score;
+    int& attr_score = glists ? h->attr_score_g : h->attr_score;
+    if (smem_score > attr_score) {
+        EVZ_CUDA_CHECK(h, cudaFuncSetAttribute(glists ? evz::ransac_score_kernel<true> : evz::ransac_score_kernel<false>,
+                                               cudaFuncAttributeMaxDynamicSharedMemorySize, smem_score));
+        attr_score = smem_score;
     }
     if (smem_refit > h->attr_refit) {
         EVZ_CUDA_CHECK(h, cudaFuncSetAttribute(evz::ransac_refit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_refit));
@@ -1339,7 +1360,8 @@ static int find_homography(const char* fn, evz_handle* h, const float* pts, cons
     evz::FhArgs a{pts, off, cnt, pre_H, n_hyp, seed, pair_id_base, level, t, min_inlier_frac, fail_status,
                   status, H, mask, inl_cnt, best_hyp, best_cnt, mask_best, H_best, max_cnt, h->opt_ransac_exact, h->opt_ransac_no_prune, hcache,
                   pair_ids};
-    evz::ransac_score_kernel<<<n_pairs, evz::kRsThreads, smem_score, st>>>(a, hb, phase);
+    if (glists) evz::ransac_score_kernel<true><<<n_pairs, evz::kRsThreads, smem_score, st>>>(a, hb, phase, hlists);
+    else evz::ransac_score_kernel<false><<<n_pairs, evz::kRsThreads, smem_score, st>>>(a, hb, phase, nullptr);
     EVZ_LAUNCH_CHECK(h);
     evz::ransac_refit_kernel<<<n_pairs, evz::kRfThreads, smem_refit, st>>>(a, hb, phase);
     EVZ_LAUNCH_CHECK(h);

@@ -21,6 +21,7 @@ import numpy as np
 import torch
 
 from .. import _lib
+from .._lib import EVZ_MAX_KP
 from .constants import RANSAC_HYPOTHESES, RANSAC_SEED, THRESHOLD_FOR_FIND_HOMOGRAPHY, LENGTH_ACCOUNTED_POINTS
 from .frame_processing import FrameProcessing, resize, DEFAULT_FEATURES
 
@@ -97,26 +98,36 @@ def _ingest_frames(eng, frames_per_video, d):
     return eng.ingest(desc, coords, [len(c) for c, _ in frames])
 
 
+def _level2_bound(feats_list, types):
+    """Upper bound of the point count of a pair at RANSAC #2, known before anything is launched: over the videos with a
+    pair, the sum over the feature types of the video's largest frame (the static points of every type are concatenated,
+    frame_processing.py:91-104).  Raises ValueError when it exceeds EVZ_MAX_KP, the most that RANSAC and the de-dup take."""
+    kp = lambda frames: max((len(c) for c, dd in frames if dd is not None), default=0)
+    bound = max((sum(kp(f[t]) for t in types) for f in feats_list if len(f[types[0]]) > 1), default=0)
+    if bound > EVZ_MAX_KP:
+        raise ValueError(f"frames of {' + '.join(types)} features reach {bound} points per pair after concatenation; "
+                         f"at most EVZ_MAX_KP = {EVZ_MAX_KP} are supported")
+    return bound
+
+
 def _level2_input(eng, feats_list, lay, ids, n_hyp, seed):
     """Match, RANSAC #1 (pair p seeded with ids[p]) and the static filter of every pair of `lay`, for every feature type,
     then the input of RANSAC #2: the static points of all types concatenated and de-duplicated per pair
     (frame_processing.py:91-104).  Returns (pts, off, cnt, status, max_cnt); a pair that failed for any type has status
-    != 0, and max_cnt is the largest over the videos of each video's own bound."""
+    != 0, and max_cnt is `_level2_bound` (checked before anything is launched)."""
     types = list(feats_list[0])
+    max_cnt = _level2_bound(feats_list, types)
     F = np.array([len(f[types[0]]) for f in feats_list], np.int64)
-    n_pairs = np.maximum(F - 1, 0)
     P = len(lay.k)
     f0 = np.zeros(len(F), np.int64)
     np.cumsum(F[:-1], out=f0[1:])
     pq = f0[lay.video] + lay.k + 1
     pt = f0[lay.video] + lay.k
     status = torch.zeros(P, dtype=torch.int32, device=eng.device)
-    per_type, video_kp = [], []
+    per_type = []
     for t in types:
         d = next((dd.shape[1] for f in feats_list for _, dd in f[t] if dd is not None), 128)
         st = _ingest_frames(eng, [f[t] for f in feats_list], d)
-        kp = st.n_kp_h.astype(np.int64)
-        video_kp.append([int(kp[a:b].max(initial=0)) for a, b, n in zip(f0, f0 + F, n_pairs) if n])   # each video's store max_kp
         r = eng.match(st, pq, pt)
         h1 = eng.find_homography(r.m_pts, r.out_off, r.m_cnt, r.status, st.max_kp, n_hyp, seed, 0, 1,
                                  THRESHOLD_FOR_FIND_HOMOGRAPHY, 0.0, _lib.ST_NO_MODEL_1, pair_ids=ids)
@@ -125,7 +136,7 @@ def _level2_input(eng, feats_list, lay, ids, n_hyp, seed):
         per_type.append((st, r, sp, sc))
     if len(types) == 1:
         st, r, pts2, cnt2 = per_type[0]
-        return pts2, r.out_off, torch.where(status == 0, cnt2, torch.zeros_like(cnt2)), status, max(video_kp[0])
+        return pts2, r.out_off, torch.where(status == 0, cnt2, torch.zeros_like(cnt2)), status, max_cnt
     # evz_concat_dedup: pair p may hold up to the sum over the types of the query frame's keypoints -- known on the host,
     # so the layout needs no read-back
     cap = np.zeros(P, np.int64)
@@ -134,7 +145,6 @@ def _level2_input(eng, feats_list, lay, ids, n_hyp, seed):
     cap = (cap + 3) // 4 * 4 + 4
     off_h = np.zeros(P, np.int64)
     np.cumsum(cap[:-1], out=off_h[1:])
-    max_cnt = max(max(sum(v), 4) for v in zip(*video_kp))
     off2 = torch.from_numpy(off_h.astype(np.int32)).to(eng.device)
     pts2, cnt2 = eng.concat_dedup([(sp, r.out_off, sc) for _, r, sp, sc in per_type], status, off2, int(cap.sum()), max_cnt)
     return pts2, off2, cnt2, status, max_cnt
@@ -161,6 +171,7 @@ def geometry_from_features_batch(feats_list, none_H_processing=True, mode="refer
     P = len(lay.k)
     if P == 0:
         return [([], np.zeros(0, np.int32)) for _ in feats_list]
+    _level2_bound(feats_list, types)                 # an unsupported size is refused before the engine is used
     dev = eng.device
     ids = torch.from_numpy(lay.k).to(dev)
     pts2, off2, cnt2, status, max_cnt = _level2_input(eng, feats_list, lay, ids, n_hyp, seed)

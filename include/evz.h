@@ -161,10 +161,11 @@ int evz_filter_matches(evz_handle* h, const int32_t* top2_idx, const int32_t* to
  * utils.py:356-358 (level 2), including the 70 % inlier gate of utils.py:359-360 when
  * min_inlier_frac > 0.  Pairs whose status is non-zero on entry are skipped.
  *   pts        DEV float [rows][4]  point pairs of pair p at rows [off[p], off[p]+cnt[p])
- *   max_cnt    upper bound of cnt[p] (sizes shared memory; <= EVZ_MAX_KP); a pair with cnt[p] > max_cnt gets fail_status
+ *   max_cnt    upper bound of cnt[p] (sizes shared memory; <= EVZ_MAX_KP, else EVZ_E_UNSUPPORTED); a pair with
+ *              cnt[p] > max_cnt gets fail_status
  *   pre_H      DEV double [P][9] or NULL: both point sets are first mapped through this
  *              matrix in f64 and rounded to f32 (utils.py:351-355, matrix_H_prev)
- *   n_hyp      hypotheses per pair (counter-based sampler: seed, pair_id_base + p, level)
+ *   n_hyp      hypotheses per pair, 1 .. 65535 (else EVZ_E_ARG) (counter-based sampler: seed, pair_id_base + p, level)
  *   fail_status value written to status[p] when no model is found (EVZ_ST_NO_MODEL_1/2)
  * outputs (any may be NULL except H and status)
  *   H          DEV double [P][9]  refined homography, h22 = 1: Levenberg-Marquardt on the 8 free parameters over the
@@ -181,8 +182,13 @@ int evz_filter_matches(evz_handle* h, const int32_t* top2_idx, const int32_t* to
  *   best_cnt   DEV int32 [P]      its inlier count
  *   mask_best  DEV uint8 [rows]   its inlier mask (the refit set)
  *   H_best     DEV double [P][9]  its 4-point model
+ * Every max_cnt <= EVZ_MAX_KP and 1 <= n_hyp <= 65535 runs, with the same results whichever memory holds the tables.
  * Handle scratch used by this call: 4 B + 72 B per pair, plus a model cache of 32 B per (pair, hypothesis) when that stays
- * below 4 GB (without it every scoring stage solves its hypotheses again; the results are the same).
+ * below 4 GB (without it every scoring stage solves its hypotheses again; the results are the same).  The scoring kernel
+ * keeps 8 B per hypothesis of lists in shared memory next to 18 B per point of max_cnt; when both do not fit in the
+ * device's per-block shared memory (on a B200: n_hyp > 944 at max_cnt = EVZ_MAX_KP, n_hyp > 28 582 at any max_cnt) the
+ * lists take 8 B per (pair, hypothesis) of handle scratch instead, e.g. 8 MB for 1 000 pairs x 1 024 hypotheses or
+ * 5.2 GB for 10 000 pairs x 65 535; EVZ_E_NOMEM when that cannot be allocated.
  */
 int evz_find_homography(evz_handle* h, const float* pts, const int32_t* off, const int32_t* cnt, int n_pairs,
                         int max_cnt, const double* pre_H, int n_hyp, uint32_t seed, int64_t pair_id_base, int level,
