@@ -35,6 +35,8 @@ SIGNATURES = {
                             _p, _p, _p, _p, _p, _p, _p, _p, _p],
     "evz_find_homography_ids": [_p, _p, _p, _p, _i, _i, _p, _i, C.c_uint32, _p, _i, _d, _d, _i,
                                 _p, _p, _p, _p, _p, _p, _p, _p, _p],
+    "evz_find_homography_adaptive": [_p, _p, _p, _p, _i, _i, _p, _i, C.c_uint32, _i64, _p, _i, _d, _d, _i, _d,
+                                     _p, _p, _p, _p, _p, _p, _p, _p, _p, _p],
     "evz_static_filter": [_p, _p, _p, _p, _i, _i, _p, _p, _p, _p, _p, _p, _p, _p],
     "evz_concat_dedup": [_p, _i, C.POINTER(_p), C.POINTER(_p), C.POINTER(_p), _i, _p, _i, _p, _p, _p, _p],
     "evz_chain_scan": [_p, _p, _p, _i, _i, _p, _p, _p, _p, _p, _p],

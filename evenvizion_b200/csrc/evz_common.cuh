@@ -27,7 +27,7 @@ struct evz_handle {
     // cudaFuncSetAttribute(MaxDynamicSharedMemorySize) is per device: remembered per handle, not per process
     unsigned attr_match = 0;       // bit 0: key-space kernel, bit 1: V-space kernel
     bool attr_static = false, attr_canon = false, attr_concat = false;
-    int attr_filter = 0, attr_score = 0, attr_score_g = 0, attr_refit = 0;
+    int attr_filter = 0, attr_score = 0, attr_score_g = 0, attr_score_a = 0, attr_refit = 0;
     int score_smem_room = -1;      // dynamic shared memory a scoring block may take (-1: not queried yet)
     // options (evz_set_option)
     int opt_ransac_exact = 0;

@@ -260,12 +260,15 @@ class GeometryEngine:
     # ------------------------------------------------------------------ K3 / K4
     def find_homography(self, pts, off, cnt, status, max_cnt, n_hyp=1024, seed=0, pair_id_base=0, level=1,
                         thresh=3.0, min_inlier_frac=0.0, fail_status=_lib.ST_NO_MODEL_1, pre_H=None, pair_ids=None,
-                        out=None):
+                        out=None, confidence=None):
         """Batched seeded RANSAC + LM refit over the point lists pts[off[p]:off[p]+cnt[p]].
         status is updated in place.  Returns dict(H, mask, inl_cnt, best_hyp, best_cnt, mask_best, H_best).
         pair_ids: int64 [P] device tensor of sampler ids (pair p is seeded with pair_ids[p] instead of pair_id_base + p).
         out: a dict of those tensors to write instead of allocating them; H and inl_cnt are required, an output left
-        out is not computed."""
+        out is not computed.
+        confidence: None scores n_hyp hypotheses per pair.  A float in (0, 1) stops each pair's search where cv2's
+        RANSAC would at that confidence, with n_hyp as the iteration cap (evz_find_homography_adaptive); the result
+        dict then also holds n_used (int32 [P]: hypotheses consumed), allocated unless `out` leaves it out."""
         P = int(cnt.numel())
         if out is None:
             rows = int(pts.shape[0])
@@ -273,6 +276,16 @@ class GeometryEngine:
             out = dict(H=z((P, 9), torch.float64), inl_cnt=z((P,), torch.int32), mask=z((rows,), torch.uint8),
                        best_hyp=torch.full((P,), -1, dtype=torch.int32, device=self.device), best_cnt=z((P,), torch.int32),
                        mask_best=z((rows,), torch.uint8), H_best=z((P, 9), torch.float64))
+            if confidence is not None:
+                out["n_used"] = z((P,), torch.int32)
+        if confidence is not None:
+            self._check(self.lib.evz_find_homography_adaptive(
+                self.h, _ptr(pts), _ptr(off), _ptr(cnt), P, int(max_cnt), _ptr(pre_H), int(n_hyp), int(seed) & 0xFFFFFFFF,
+                int(pair_id_base), _ptr(pair_ids), int(level), float(thresh), float(min_inlier_frac), int(fail_status),
+                float(confidence), _ptr(status), _ptr(out["H"]), _ptr(out.get("mask")), _ptr(out["inl_cnt"]),
+                _ptr(out.get("best_hyp")), _ptr(out.get("best_cnt")), _ptr(out.get("mask_best")), _ptr(out.get("H_best")),
+                _ptr(out.get("n_used")), self._stream()))
+            return out
         if pair_ids is not None:
             fn, ids = self.lib.evz_find_homography_ids, _ptr(pair_ids)
         else:
@@ -321,11 +334,13 @@ class GeometryEngine:
 
     # ------------------------------------------------------------------ whole per-pair path
     def process_pairs(self, st: FrameStore, pair_q, pair_t, n_hyp=1024, seed=0, pair_id_base=0,
-                      ratio=0.5, thresh=3.0, min_matching_pts=4) -> PairResults:
+                      ratio=0.5, thresh=3.0, min_matching_pts=4, confidence=None) -> PairResults:
         """match_static_kps + compute_homography for every pair (reference matching.py:131-163,
-        utils.py:328-363), all on the device."""
-        r = self.alloc_results(st, pair_q, pair_t)
-        self._pairs_range(st, r, 0, int(r.pair_q.numel()), n_hyp, seed, pair_id_base, ratio, thresh, min_matching_pts)
+        utils.py:328-363), all on the device.  confidence: see `find_homography` (both RANSAC levels; the hypotheses
+        each pair consumed are in r.extra["n_used1"] / ["n_used2"])."""
+        r = self.alloc_results(st, pair_q, pair_t, confidence)
+        self._pairs_range(st, r, 0, int(r.pair_q.numel()), n_hyp, seed, pair_id_base, ratio, thresh, min_matching_pts,
+                          confidence=confidence)
         return r
 
     # ------------------------------------------------------------------ K6 / K7
@@ -362,14 +377,14 @@ class GeometryEngine:
                                                 1 if policy else 0, _ptr(S_state), _ptr(H_prev), _ptr(H_out), self._stream()))
 
     def reference_chains(self, pts, off, cnt, status, max_cnt, step_off, n_hyp=1024, seed=0, policy=True, thresh=3.0,
-                         min_inlier_frac=0.7, fail_status=_lib.ST_NO_MODEL_2):
+                         min_inlier_frac=0.7, fail_status=_lib.ST_NO_MODEL_2, confidence=None):
         """RANSAC #2 of the reference-exact chain (video_processing.py:67-105) for several videos in lockstep.
 
         The pairs are in step-major order: step k is pairs [step_off[k], step_off[k+1]) = pair k of chains 0 .. n_k - 1,
         with n_0 >= n_1 >= ... (chains ordered by length, longest first), so the chains still running are a prefix.
         Step k is one RANSAC launch over its pairs, seeded with id k and pre-transformed by every chain's running
         superposition, then one evz_chain_ref_step.  The outputs are allocated before the loop and the loop neither
-        allocates nor synchronises with the host.  status is updated in place; returns H_out [P,9]: the matrix the
+        allocates nor synchronises with the host.  confidence: see `find_homography`.  status is updated in place; returns H_out [P,9]: the matrix the
         reference stores for every pair, after the None-H policy."""
         step_off = np.asarray(step_off, np.int64)
         K = len(step_off) - 1
@@ -386,7 +401,7 @@ class GeometryEngine:
             H2_k, status_k, prev = H2[a:b], status[a:b], int(step_off[k - 1]) if k else 0
             self.find_homography(pts, off[a:b], cnt[a:b], status_k, max_cnt, n_hyp, seed, 0, 2, thresh, min_inlier_frac,
                                  fail_status, pre_H=S_state if k else None, pair_ids=ids[a:b],
-                                 out=dict(H=H2_k, inl_cnt=inl[a:b]))
+                                 out=dict(H=H2_k, inl_cnt=inl[a:b]), confidence=confidence)
             self.chain_ref_step(H2_k, status_k, k == 0, policy, S_state, H_out[prev:prev + b - a] if k else None, H_out[a:b])
         return H_out
 
@@ -419,7 +434,7 @@ class GeometryEngine:
 
     # ------------------------------------------------------------------ video-level driver
     def _pairs_range(self, st: FrameStore, r: PairResults, p0: int, p1: int, n_hyp, seed, pair_id_base, ratio, thresh,
-                     min_matching_pts=4, after_match=None):
+                     min_matching_pts=4, after_match=None, confidence=None):
         """match_static_kps + compute_homography for pairs [p0, p1) of an already allocated PairResults, written through a
         `pairs` view of it."""
         if p1 <= p0:
@@ -430,14 +445,17 @@ class GeometryEngine:
             after_match()
         self.find_homography(v.m_pts, v.out_off, v.m_cnt, v.status, mk, n_hyp, seed, int(pair_id_base) + p0, 1, thresh, 0.0,
                              _lib.ST_NO_MODEL_1, out=dict(H=v.H1, mask=v.mask1, inl_cnt=v.inl1, best_hyp=v.best_hyp1,
-                                                          best_cnt=v.best_cnt1, mask_best=v.mask1_best, H_best=v.extra["H1_best"]))
+                                                          best_cnt=v.best_cnt1, mask_best=v.mask1_best, H_best=v.extra["H1_best"],
+                                                          n_used=v.extra.get("n_used1")), confidence=confidence)
         self.static_filter(v.m_pts, v.out_off, v.m_cnt, v.H1, v.status, max_cnt=mk, out=(v.static_pts, v.static_cnt, v.static_r, v.flags))
         self.find_homography(v.static_pts, v.out_off, v.static_cnt, v.status, mk, n_hyp, seed, int(pair_id_base) + p0, 2, thresh,
                              0.7, _lib.ST_NO_MODEL_2, out=dict(H=v.H, mask=v.mask2, inl_cnt=v.inl2, best_hyp=v.best_hyp2,
-                                                               best_cnt=v.best_cnt2, mask_best=v.mask2_best, H_best=v.extra["H2_best"]))
+                                                               best_cnt=v.best_cnt2, mask_best=v.mask2_best, H_best=v.extra["H2_best"],
+                                                               n_used=v.extra.get("n_used2")), confidence=confidence)
 
-    def alloc_results(self, st: FrameStore, pair_q, pair_t) -> PairResults:
-        """Workspace for `process_pairs_into`: every per-pair / per-row output of the path, allocated once."""
+    def alloc_results(self, st: FrameStore, pair_q, pair_t, confidence=None) -> PairResults:
+        """Workspace for `process_pairs_into`: every per-pair / per-row output of the path, allocated once.  With a
+        confidence it also holds extra["n_used1"] / extra["n_used2"], the hypotheses each pair consumed per level."""
         r = self._match_results(st, pair_q, pair_t)
         P, rows = int(r.pair_q.numel()), st.rows
         e, z = self._empty, lambda shape, dt: torch.zeros(shape, dtype=dt, device=self.device)
@@ -448,20 +466,24 @@ class GeometryEngine:
         r.best_hyp1 = torch.full((P,), -1, dtype=i32, device=self.device)
         r.best_hyp2 = torch.full((P,), -1, dtype=i32, device=self.device)
         r.extra["H1_best"], r.extra["H2_best"] = z((P, 9), f64), z((P, 9), f64)
+        if confidence is not None:
+            r.extra["n_used1"], r.extra["n_used2"] = z((P,), i32), z((P,), i32)
         r.static_pts, r.static_cnt = e((rows, 4), torch.float32), e((P,), i32)
         r.static_r, r.flags = e((P,), i32), e((P,), i32)
         return r
 
     def process_pairs_into(self, st: FrameStore, r: PairResults, n_hyp=1024, seed=0, pair_id_base=0, ratio=0.5, thresh=3.0,
-                           after_match=None) -> PairResults:
+                           after_match=None, confidence=None) -> PairResults:
         """`process_pairs` into a workspace from `alloc_results`: no allocation, no memset, nothing but the kernels of the
         path on the current stream (what a steady-state caller -- and bench.py's timed region -- runs per batch).
-        after_match: optional callable invoked between the match stage and the first RANSAC (event recording)."""
-        self._pairs_range(st, r, 0, int(r.pair_q.numel()), n_hyp, seed, pair_id_base, ratio, thresh, after_match=after_match)
+        after_match: optional callable invoked between the match stage and the first RANSAC (event recording).
+        confidence: see `find_homography`; n_used goes to r.extra["n_used1"] / ["n_used2"] when `alloc_results` made them."""
+        self._pairs_range(st, r, 0, int(r.pair_q.numel()), n_hyp, seed, pair_id_base, ratio, thresh, after_match=after_match,
+                          confidence=confidence)
         return r
 
     def video_geometry(self, desc, coords, n_kp=None, n_hyp=1024, seed=0, none_h_processing=True,
-                       ratio=0.5, thresh=3.0, pair_id_base=0, chunk_frames=None):
+                       ratio=0.5, thresh=3.0, pair_id_base=0, chunk_frames=None, confidence=None):
         """Frame chain -> per-pair G, status, cumulative S and fixed-plane H (parallel formulation).
         Host arrays in, host arrays out: this is the call bench.py times end to end.
 
@@ -476,15 +498,16 @@ class GeometryEngine:
             # small or device-resident input: one ingest, one batch
             st = self.ingest(desc_t, coords_t, n_kp_h)
             r = self.process_pairs(st, torch.arange(1, F, dtype=torch.int32), torch.arange(0, F - 1, dtype=torch.int32),
-                                   n_hyp, seed, pair_id_base, ratio, thresh)
+                                   n_hyp, seed, pair_id_base, ratio, thresh, confidence=confidence)
         else:
             st, r = self._video_streamed(desc_t, coords_t, n_kp_h, d, is_f32, chunk_frames, n_hyp, seed, pair_id_base,
-                                         ratio, thresh)
+                                         ratio, thresh, confidence)
         S, Hf, _ = self.chain_scan(r.H, r.status, none_h_processing)
         return dict(G=r.H.cpu().numpy().reshape(-1, 3, 3), status=r.status.cpu().numpy(),
                     S=S.cpu().numpy().reshape(-1, 3, 3), H_fixed=Hf.cpu().numpy().reshape(-1, 3, 3), results=r, store=st)
 
-    def _video_streamed(self, desc_t, coords_t, n_kp_h, d, is_f32, chunk_frames, n_hyp, seed, pair_id_base, ratio, thresh):
+    def _video_streamed(self, desc_t, coords_t, n_kp_h, d, is_f32, chunk_frames, n_hyp, seed, pair_id_base, ratio, thresh,
+                        confidence=None):
         coords_t = coords_t.to(torch.float32)
         F = len(n_kp_h)
         dev = self.device
@@ -497,7 +520,7 @@ class GeometryEngine:
         coords_raw = torch.empty(coords_t.shape, dtype=torch.float32, device=dev)
         st.keep += (desc_raw, coords_raw)
         r = self.alloc_results(st, torch.arange(1, F, dtype=torch.int32, device=dev),
-                               torch.arange(0, F - 1, dtype=torch.int32, device=dev))
+                               torch.arange(0, F - 1, dtype=torch.int32, device=dev), confidence)
         copy.wait_stream(compute)            # the staging buffers were allocated on the compute stream
         for f0 in range(0, F, chunk_frames):
             f1 = min(F, f0 + chunk_frames)
@@ -510,7 +533,7 @@ class GeometryEngine:
             compute.wait_event(landed)
             self._ingest_frames(st, desc_raw, coords_raw, raw_off, is_f32, bad, f0, f1)
             # pairs whose query frame is in this chunk (their train frame landed with this or an earlier chunk)
-            self._pairs_range(st, r, max(f0, 1) - 1, f1 - 1, n_hyp, seed, pair_id_base, ratio, thresh)
+            self._pairs_range(st, r, max(f0, 1) - 1, f1 - 1, n_hyp, seed, pair_id_base, ratio, thresh, confidence=confidence)
         desc_raw.record_stream(copy); coords_raw.record_stream(copy)
         st.keep = (bad,)                     # every consumer of the raw staging copies is enqueued: let them go
         if is_f32:

@@ -74,14 +74,15 @@ class KeyPoints:
         return [p for p in pts[:, :2].copy()], [p for p in pts[:, 2:].copy()]
 
     def match_static_kps(self, acceding_kps, reproj_thresh=THRESHOLD_FOR_FIND_HOMOGRAPHY,
-                         n_hyp=None, seed=None, pair_id=0):
+                         n_hyp=None, seed=None, pair_id=0, confidence=None):
         """Matches that lie on static objects (reference matching.py:131-163): RANSAC homography,
-        then the largest group of equal rounded displacement.  Returns two (Ms,2) float32 arrays."""
+        then the largest group of equal rounded displacement.  Returns two (Ms,2) float32 arrays.
+        confidence: None scores n_hyp hypotheses; a float in (0, 1) stops where cv2's RANSAC would (n_hyp = maxIters)."""
         eng, st, r = self._match_device(acceding_kps, LOWES_RATIO, MINIMUM_MATCHING_POINTS)
         n_hyp = RANSAC_HYPOTHESES if n_hyp is None else n_hyp
         seed = RANSAC_SEED if seed is None else seed
         h1 = eng.find_homography(r.m_pts, r.out_off, r.m_cnt, r.status, st.max_kp, n_hyp, seed, pair_id, 1,
-                                 reproj_thresh, 0.0, _lib.ST_NO_MODEL_1)
+                                 reproj_thresh, 0.0, _lib.ST_NO_MODEL_1, confidence=confidence)
         s = int(r.status[0])
         if s == _lib.ST_FEW_POINTS:
             raise NoMatchesException("fewer than 4 matching points after de-duplication", "couldn't process")

@@ -160,10 +160,11 @@ def get_largest_group_points(r_moving_dict, pts_a, pts_b):
     return np.array([pts_a[i] for i in idx]), np.array([pts_b[i] for i in idx])
 
 
-def compute_homography(pts_a, pts_b, matrix_H_prev=None, n_hyp=None, seed=None, pair_id=0):
+def compute_homography(pts_a, pts_b, matrix_H_prev=None, n_hyp=None, seed=None, pair_id=0, confidence=None):
     """Second-level RANSAC homography with the 70 % inlier gate (reference utils.py:328-363).
     matrix_H_prev: superposition between the origin and frame_a; both point sets are mapped through
-    it first, so that H lives in the fixed plane.  Raises HomographyException."""
+    it first, so that H lives in the fixed plane.  confidence: None scores n_hyp hypotheses; a float in (0, 1) stops
+    where cv2's RANSAC would (n_hyp = maxIters).  Raises HomographyException."""
     eng = _engine()
     pts, off, cnt, n = _pack_points(eng, pts_a, pts_b)
     if n < 4:
@@ -174,7 +175,7 @@ def compute_homography(pts_a, pts_b, matrix_H_prev=None, n_hyp=None, seed=None, 
         pre = torch.from_numpy(np.asarray(matrix_H_prev, np.float64).reshape(1, 9)).to(eng.device)
     out = eng.find_homography(pts, off, cnt, status, max(n, 4), RANSAC_HYPOTHESES if n_hyp is None else n_hyp,
                               RANSAC_SEED if seed is None else seed, pair_id, 2, THRESHOLD_FOR_FIND_HOMOGRAPHY,
-                              LENGTH_ACCOUNTED_POINTS, _lib.ST_NO_MODEL_2, pre_H=pre)
+                              LENGTH_ACCOUNTED_POINTS, _lib.ST_NO_MODEL_2, pre_H=pre, confidence=confidence)
     s = int(status[0])
     if s == _lib.ST_FEW_INLIERS:
         raise HomographyException("not enough points in homography calculation")

@@ -44,11 +44,12 @@ def read_and_describe(capture, resize_width=400, features_type_list=None):
     return feats, shape
 
 
-def geometry_from_features(feats, none_H_processing=True, mode="reference", n_hyp=None, seed=None, engine=None):
+def geometry_from_features(feats, none_H_processing=True, mode="reference", n_hyp=None, seed=None, engine=None,
+                           confidence=None):
     """The hot path for a whole video given per-frame features: `geometry_from_features_batch` of one video.  Returns
     (H_list, status): H_list[k] is the 3x3 matrix stored under frame k+2, after the None-H policy (identity where the
     policy leaves it undefined); status int32 [F-1]."""
-    return geometry_from_features_batch([feats], none_H_processing, mode, n_hyp, seed, engine)[0]
+    return geometry_from_features_batch([feats], none_H_processing, mode, n_hyp, seed, engine, confidence)[0]
 
 
 class PairLayout:
@@ -110,7 +111,7 @@ def _level2_bound(feats_list, types):
     return bound
 
 
-def _level2_input(eng, feats_list, lay, ids, n_hyp, seed):
+def _level2_input(eng, feats_list, lay, ids, n_hyp, seed, confidence=None):
     """Match, RANSAC #1 (pair p seeded with ids[p]) and the static filter of every pair of `lay`, for every feature type,
     then the input of RANSAC #2: the static points of all types concatenated and de-duplicated per pair
     (frame_processing.py:91-104).  Returns (pts, off, cnt, status, max_cnt); a pair that failed for any type has status
@@ -130,7 +131,7 @@ def _level2_input(eng, feats_list, lay, ids, n_hyp, seed):
         st = _ingest_frames(eng, [f[t] for f in feats_list], d)
         r = eng.match(st, pq, pt)
         h1 = eng.find_homography(r.m_pts, r.out_off, r.m_cnt, r.status, st.max_kp, n_hyp, seed, 0, 1,
-                                 THRESHOLD_FOR_FIND_HOMOGRAPHY, 0.0, _lib.ST_NO_MODEL_1, pair_ids=ids)
+                                 THRESHOLD_FOR_FIND_HOMOGRAPHY, 0.0, _lib.ST_NO_MODEL_1, pair_ids=ids, confidence=confidence)
         sp, sc, _, _ = eng.static_filter(r.m_pts, r.out_off, r.m_cnt, h1["H"], r.status, max_cnt=st.max_kp)
         status = torch.where(status == 0, r.status, status)      # any failing feature type fails the pair
         per_type.append((st, r, sp, sc))
@@ -150,12 +151,16 @@ def _level2_input(eng, feats_list, lay, ids, n_hyp, seed):
     return pts2, off2, cnt2, status, max_cnt
 
 
-def geometry_from_features_batch(feats_list, none_H_processing=True, mode="reference", n_hyp=None, seed=None, engine=None):
+def geometry_from_features_batch(feats_list, none_H_processing=True, mode="reference", n_hyp=None, seed=None, engine=None,
+                                 confidence=None):
     """The geometry of many videos in one call: returns [(H_list, status)] in input order, entry i the same as for
     feats_list[i] alone.  All videos share one frame store per feature type and one launch of every per-pair stage;
     pair k of every video keeps RANSAC id k.  mode="parallel" ends in one segmented scan;
     mode="reference" runs the reference-exact chains of all videos in lockstep on the device (one RANSAC #2 launch and
-    one chain-step launch per step, no host round trip inside the loop)."""
+    one chain-step launch per step, no host round trip inside the loop).
+    confidence: None (default) scores n_hyp hypotheses per pair and level.  A float in (0, 1) gives both RANSAC calls
+    cv2.findHomography's stop rule at that confidence, with n_hyp as its maxIters (cv2's defaults: confidence=0.995,
+    n_hyp=2000)."""
     from .. import default_engine
     eng = engine or default_engine()
     n_hyp = RANSAC_HYPOTHESES if n_hyp is None else n_hyp
@@ -174,34 +179,35 @@ def geometry_from_features_batch(feats_list, none_H_processing=True, mode="refer
     _level2_bound(feats_list, types)                 # an unsupported size is refused before the engine is used
     dev = eng.device
     ids = torch.from_numpy(lay.k).to(dev)
-    pts2, off2, cnt2, status, max_cnt = _level2_input(eng, feats_list, lay, ids, n_hyp, seed)
+    pts2, off2, cnt2, status, max_cnt = _level2_input(eng, feats_list, lay, ids, n_hyp, seed, confidence)
     if mode == "parallel":
         h2 = eng.find_homography(pts2, off2, cnt2, status, max_cnt, n_hyp, seed, 0, 2, THRESHOLD_FOR_FIND_HOMOGRAPHY,
-                                 LENGTH_ACCOUNTED_POINTS, _lib.ST_NO_MODEL_2, pair_ids=ids)
+                                 LENGTH_ACCOUNTED_POINTS, _lib.ST_NO_MODEL_2, pair_ids=ids, confidence=confidence)
         seg_off = torch.from_numpy(lay.seg_off.astype(np.int32)).to(dev)
         _, H = eng.chain_scan_segments(h2["H"], status, seg_off, none_H_processing)
     else:
         H = eng.reference_chains(pts2, off2, cnt2, status, max_cnt, lay.step_off, n_hyp, seed, none_H_processing,
-                                 THRESHOLD_FOR_FIND_HOMOGRAPHY, LENGTH_ACCOUNTED_POINTS, _lib.ST_NO_MODEL_2)
+                                 THRESHOLD_FOR_FIND_HOMOGRAPHY, LENGTH_ACCOUNTED_POINTS, _lib.ST_NO_MODEL_2, confidence)
     H = H.cpu().numpy().reshape(P, 3, 3)
     st_h = status.cpu().numpy()
     return [([Hv[k] for k in range(len(Hv))], sv) for Hv, sv in zip(lay.split(H), lay.split(st_h))]
 
 
 def get_homography_dict(capture, resize_width=400, matching_path=None, none_H_processing=True,
-                        features_type_list=None, mode="reference", n_hyp=None, seed=None):
+                        features_type_list=None, mode="reference", n_hyp=None, seed=None, confidence=None):
     """reference video_processing.py:27-108.  `matching_path` (match visualisation PNGs) belongs to the
-    out-of-scope visualisation layer and is ignored."""
+    out-of-scope visualisation layer and is ignored.  confidence: see `geometry_from_features_batch`."""
     return get_homography_dicts([capture], resize_width, matching_path, none_H_processing, features_type_list, mode,
-                                n_hyp, seed)[0]
+                                n_hyp, seed, confidence)[0]
 
 
 def get_homography_dicts(captures, resize_width=400, matching_path=None, none_H_processing=True,
-                         features_type_list=None, mode="reference", n_hyp=None, seed=None):
+                         features_type_list=None, mode="reference", n_hyp=None, seed=None, confidence=None):
     """`get_homography_dict` for several captures: every capture is decoded and described (`read_and_describe`), then
     the geometry of all of them runs in one `geometry_from_features_batch` call.  Returns one dict per capture, in order."""
     described = [read_and_describe(c, resize_width, features_type_list) for c in captures]
-    results = geometry_from_features_batch([f for f, _ in described], none_H_processing, mode, n_hyp, seed)
+    results = geometry_from_features_batch([f for f, _ in described], none_H_processing, mode, n_hyp, seed,
+                                           confidence=confidence)
     out = []
     for (_, shape), (H_list, _) in zip(described, results):
         homography_dict = {k + 2: {"H": np.asarray(H, np.float64).tolist()} for k, H in enumerate(H_list)}

@@ -209,6 +209,36 @@ int evz_find_homography_ids(evz_handle* h, const float* pts, const int32_t* off,
                             int32_t* status, double* H, uint8_t* mask, int32_t* inl_cnt,
                             int32_t* best_hyp, int32_t* best_cnt, uint8_t* mask_best, double* H_best,
                             void* stream);
+/* The same with OpenCV's confidence-bounded stop (RANSACPointSetRegistrator::run / RANSACUpdateNumIters): n_hyp is the
+ * iteration cap (cv2's maxIters) and the search ends as soon as `confidence` says enough hypotheses were tried.  For a
+ * pair with m > 4 points:
+ *   stream   hypotheses 0, 1, .., n_hyp - 1 of the sampler above (seed, pair id, level), in index order; one that fails
+ *            the orientation / collinearity / finiteness test consumes no iteration (cv2's getSubset draws again)
+ *   state    best = 0, niters = n_hyp, it = 0
+ *   update   after every valid hypothesis with count c (f32 computeError <= thresh^2): it += 1; if c > max(best, 3):
+ *            best = c, the hypothesis becomes the winner, niters = upd(confidence, (double)(m - c) / m, niters)
+ *   stop     when it >= niters, or when the stream ends
+ *   upd(p, ep, maxIters)  num = max(1 - p, DBL_MIN), denom = 1 - pow(1 - ep, 4); 0 if denom < DBL_MIN; else with
+ *            num = log(num), denom = log(denom): maxIters if denom >= 0 || -num >= maxIters * (-denom), else
+ *            num / denom rounded half to even (e.g. at confidence 0.995, maxIters 1024: 10 at 80 % inliers, 82 at 50 %,
+ *            651 at 30 %, the cap at 20 %)
+ * The winner is the (count desc, index asc) arg-max over the consumed hypotheses; refit, masks, the 70 % gate, the m == 4
+ * path and the status codes are those of evz_find_homography.  (The device's log / pow may differ from glibc's in the
+ * last ulp, which can move a bound that lies within ~1e-9 of a rounding or cap boundary.)
+ *   pair_id    DEV int64 [P] sampler id of every pair, or NULL for pair_id_base + p
+ *   confidence in (0, 1) (cv2 asserts the same; 0.995 is cv2's default), else EVZ_E_ARG before any work is enqueued
+ *   n_used     DEV int32 [P] or NULL: one past the index of the last hypothesis consumed (n_hyp when the stream ran out);
+ *              0 for pairs that never sample (status set on entry, fewer than 5 points, cnt[p] > max_cnt)
+ * Every output of pair p equals what evz_find_homography[_ids] returns for it with n_hyp = n_used[p], bit for bit.
+ * The scoring kernel keeps only lists of up to 512 hypotheses in shared memory, so it needs no list scratch at any n_hyp.
+ */
+int evz_find_homography_adaptive(evz_handle* h, const float* pts, const int32_t* off, const int32_t* cnt, int n_pairs,
+                                 int max_cnt, const double* pre_H, int n_hyp, uint32_t seed, int64_t pair_id_base,
+                                 const int64_t* pair_id, int level, double thresh, double min_inlier_frac, int fail_status,
+                                 double confidence,
+                                 int32_t* status, double* H, uint8_t* mask, int32_t* inl_cnt,
+                                 int32_t* best_hyp, int32_t* best_cnt, uint8_t* mask_best, double* H_best,
+                                 int32_t* n_used, void* stream);
 
 /* ---- K5: displacement-mode static-point filter.  Replaces find_point_displacement
  * (utils.py:289-325) + get_largest_group_points (utils.py:258-286).
