@@ -119,7 +119,15 @@ struct FhArgs {
     int no_prune;
     float4* hcache;     // [n_pairs][n_hyp][2] f32 models of the hypotheses that passed pass 0 (null: solved again where needed)
     const int64_t* pair_ids;   // [n_pairs] sampler id of every pair (null: pair_id_base + p)
+    // the threshold's share of the fused_thresholds cuts, the same for every hypothesis (set_fused_cut)
+    float thresh_sqrt, cut_k, cut_rnd;
 };
+
+__host__ __device__ inline void set_fused_cut(FhArgs& a) {
+    a.thresh_sqrt = sqrtf(a.thresh2);                                    // correctly rounded on host and device
+    a.cut_k = 2.5f * a.thresh_sqrt;
+    a.cut_rnd = fmaxf(1e-4f, 8.f * 5.9604645e-8f * a.thresh2);          // max(1e-4, 8u t)
+}
 
 // fused (FFMA + approximate reciprocal) evaluation of the same quantity as reproj_err32
 __device__ __forceinline__ float reproj_err_fused(const float (&h)[8], const float4 p) {
@@ -141,11 +149,16 @@ __device__ __forceinline__ float reproj_err_fused(const float (&h)[8], const flo
 // Then, for either path,
 //   rel. error of ww            <= rho = 4u Bd/dm + 2u                     (rcp.approx: 2^-23)
 //   abs. error of X ww - u_i    <= (Bx/dm)(6u + rho) + u cmax
-// so the paths differ by at most dX (dY) below (x1.25 safety) and, with D = dX + dY,
-//   |err_exact - err_fused| <= 2 D sqrt(max err) + 6u max err.
-// Solving the two one-sided implications for the fused value gives
-//   err_fused >= t + 2D^2 + 2D sqrt(D^2 + t)  =>  err_exact >  t      (thi, margin x1.25 + 1e-4)
-//   err_fused <= t - 6D            (D < 2)    =>  err_exact <= t      (tlo, margin x1.25 + 1e-4)
+// so the paths differ by at most dX (dY) below (twice that, x1.25 safety) and, with D = dX + dY, the residual vectors r = (dx, dy)
+// of the two paths satisfy  | |r_exact| - |r_fused| | <= D  (triangle inequality).  The two f32 squares and the sum
+// round with at most 2u relative error on either path: err = |r|^2 (1 +- 2.0001u).  With s = sqrt(t):
+//   err_fused <= (s - D)^2 (1 - 4u) = t - 2 s D + D^2 - ..  =>  err_exact <= t      (needs D < s)
+//   err_fused >= (s + D)^2 (1 + 4u) = t + 2 s D + D^2 + ..  =>  err_exact >  t
+// The cuts below take the D terms x1.25 (which also absorbs the rounding of these few f32 operations on them) and a
+// rounding term 8u t >= the 4u t above plus the two roundings of t +- ..; it never falls below 1e-4, which keeps the
+// cuts of small thresholds at their earlier values:
+//   thi = t + 1.25 (2D^2 + 2D sqrt(D^2 + t)) + max(1e-4, 8u t)          (2D sqrt(D^2 + t) >= 2 s D)
+//   tlo = t - 2.5 s D - max(1e-4, 8u t)                  (D < s; tlo < 0 never fires, err_fused >= 0)
 // Everything else (inside the band, |den| small, NaN) is "unsure" and counted in hi only.
 constexpr float kDenMin = 0.0625f;
 // true when |den| >= kDenMin is guaranteed on both the fused and the exact path for every point with
@@ -156,8 +169,10 @@ __device__ __forceinline__ bool den_safe(float h6, float h7, float cmax) {
     const float Bd = a6 * cmax + 1.f;
     return (8.f * u * Bd <= 0.1f * kDenMin) && ((1.f - a6 * cmax - 8.f * u * Bd) * 0.999999f >= kDenMin);
 }
-__device__ __forceinline__ void fused_thresholds(const float (&h)[8], float cmax, float t, bool exact_only,
+// t, s = sqrt(t), 2.5 s and the rounding term come from a (set_fused_cut)
+__device__ __forceinline__ void fused_thresholds(const float (&h)[8], float cmax, const FhArgs& a, bool exact_only,
                                                  float& tlo, float& thi) {
+    const float t = a.thresh2, s = a.thresh_sqrt, rnd = a.cut_rnd;
     const float u = 5.9604645e-8f;
     const float a6 = fabsf(h[6]) + fabsf(h[7]);
     const float Bd = a6 * cmax + 1.f;
@@ -171,8 +186,8 @@ __device__ __forceinline__ void fused_thresholds(const float (&h)[8], float cmax
     tlo = -INFINITY;
     thi = INFINITY;
     if (exact_only || !(8.f * u * Bd <= 0.1f * kDenMin) || !(D < 1e6f)) return;      // no usable bound: all unsure
-    thi = t + 1.25f * (2.f * D * D + 2.f * D * sqrtf(D * D + t)) + 1e-4f;
-    if (D < 2.f) tlo = t - 1.25f * 6.f * D - 1e-4f;
+    thi = t + 1.25f * (2.f * D * D + 2.f * D * sqrtf(D * D + t)) + rnd;
+    if (D < s) tlo = t - a.cut_k * D - rnd;
 }
 
 // Fused scoring of NJ hypotheses per thread (slots s0 + j*kRsThreads + tid) against all matches;
@@ -236,7 +251,7 @@ __device__ __forceinline__ int score_batch(const FhArgs& a, const float4* pts, c
         // hypotheses behind the cut (see the pruning note in ransac_score_kernel) stay idle: lo = hi = 0
         if (slot < n_valid && static_cast<int>(vlist[slot]) < cutv) {
             hyp_model(a, pts, pos, vlist[slot], m, pair_level, hf[j]);
-            fused_thresholds(hf[j], cmax, a.thresh2, a.exact_only != 0, tlo[j], thi[j]);
+            fused_thresholds(hf[j], cmax, a, a.exact_only != 0, tlo[j], thi[j]);
             any_live = true;
             if (rg.mode == kSuffix || rg.mode == kMid) { lo[j] = lo_s[slot]; out[j] = hi_s[slot]; }
         }
@@ -298,7 +313,7 @@ __device__ __forceinline__ void score_partial_row(const FhArgs& a, const float4*
     for (int i = 0; i < 8; ++i) hf[i] = 0.f;
     if (live) {
         hyp_model(a, pts, pos, vlist[r0 + k], m, pair_level, hf);
-        fused_thresholds(hf, cmax, a.thresh2, a.exact_only != 0, tlo, thi);
+        fused_thresholds(hf, cmax, a, a.exact_only != 0, tlo, thi);
     }
     part[tid] = 0; part[kRsThreads + tid] = 0;
     __syncthreads();
@@ -435,7 +450,7 @@ __device__ __forceinline__ bool first_perfect_search(const FhArgs& a, const floa
                 float hf[8], tlo, thi;
 #pragma unroll
                 for (int i = 0; i < 8; ++i) { hf[i] = static_cast<float>(H[i]); grp[tid * 10 + i] = hf[i]; }
-                fused_thresholds(hf, cmax, a.thresh2, false, tlo, thi);
+                fused_thresholds(hf, cmax, a, false, tlo, thi);
                 grp[tid * 10 + 8] = tlo; grp[tid * 10 + 9] = thi;
             }
             dead[tid] = ok ? 0 : 1;

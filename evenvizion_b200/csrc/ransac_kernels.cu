@@ -419,7 +419,7 @@ ransac_score_kernel(const FhArgs a, double* __restrict__ Hbest_out, int32_t* __r
                 solve4(q, H);
                 float hf[8], tlo, thi;
                 for (int i = 0; i < 8; ++i) { hf[i] = static_cast<float>(H[i]); lead_s[i] = hf[i]; }
-                fused_thresholds(hf, cmax, a.thresh2, a.exact_only != 0, tlo, thi);
+                fused_thresholds(hf, cmax, a, a.exact_only != 0, tlo, thi);
                 lead_s[8] = tlo;
             }
             __syncthreads();
@@ -890,6 +890,7 @@ static int find_homography(const char* fn, evz_handle* h, const float* pts, cons
     evz::FhArgs a{pts, off, cnt, pre_H, n_hyp, seed, pair_id_base, level, t, min_inlier_frac, fail_status,
                   status, H, mask, inl_cnt, best_hyp, best_cnt, mask_best, H_best, max_cnt, h->opt_ransac_exact, h->opt_ransac_no_prune, hcache,
                   pair_ids};
+    evz::set_fused_cut(a);
     if (adaptive) {
         rc = evz_launch_adaptive_score(h, a, confidence, n_used, hb, phase, n_pairs, smem_pts, st);
         if (rc) return rc;

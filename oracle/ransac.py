@@ -122,6 +122,232 @@ def reproj_err32(H, a, b):
         return dx * dx + dy * dy
 
 
+# ----------------------------------------------------------------------------- fused count bounds
+# Restatements of the device's fast classification (csrc/ransac_device.cuh): the fused evaluation reproj_err_fused (FFMA
+# and rcp.approx), the cuts fused_thresholds and the den_safe test.  The scoring kernels count a match as a sure inlier
+# when its fused error is <= tlo and as a sure outlier when it is >= thi; both rest on the bound proved in the header.
+F32 = np.float32
+U = F32(2.0 ** -24)
+DEN_MIN = F32(0.0625)          # kDenMin
+
+
+def reproj_err32_pairs(h, a, b):
+    """reproj_err32 with one f32 model per point: h (N,8) f32, a, b (N,2) f32 -> (N,) f32."""
+    h = np.asarray(h, F32)
+    x, y, z, w = a[:, 0].astype(F32), a[:, 1].astype(F32), b[:, 0].astype(F32), b[:, 1].astype(F32)
+    with np.errstate(all="ignore"):
+        ww = F32(1) / ((h[:, 6] * x + h[:, 7] * y) + F32(1))
+        dx = ((h[:, 0] * x + h[:, 1] * y) + h[:, 2]) * ww - z
+        dy = ((h[:, 3] * x + h[:, 4] * y) + h[:, 5]) * ww - w
+        return dx * dx + dy * dy
+
+
+def fma32(a, b, c):
+    """Correctly rounded f32 fma(a, b, c) of f32 arrays (round to nearest even).  The product is exact in f64; the f64
+    sum s and its error e (TwoSum) hold a*b + c exactly, and rounding s to f32 is wrong only when s is an f32 midpoint
+    and e != 0 (double rounding), where e decides the side.  Overflow and subnormal results are not handled."""
+    a, b, c = (np.asarray(v, F32).astype(np.float64) for v in (a, b, c))
+    p = a * b
+    s = p + c
+    bb = s - p
+    e = (p - (s - bb)) + (c - bb)
+    r = s.astype(F32)
+    other = np.nextafter(r, np.where(s > r, F32(np.inf), F32(-np.inf)).astype(F32))
+    mid = (r.astype(np.float64) + other.astype(np.float64)) * 0.5
+    fix = (s == mid) & (e != 0) & (s != r.astype(np.float64))
+    side = np.where(e > 0, np.maximum(r, other), np.minimum(r, other))
+    return np.where(fix, side, r).astype(F32)
+
+
+def fused_den32(h, a):
+    """den of reproj_err_fused: fma(h6, x, fma(h7, y, 1))."""
+    h = np.asarray(h, F32)
+    return fma32(h[:, 6], a[:, 0], fma32(h[:, 7], a[:, 1], np.ones(len(a), F32)))
+
+
+def reproj_err_fused32(h, a, b, ww):
+    """reproj_err_fused with the reciprocal given: h (N,8), a, b (N,2), ww (N,) f32 -> (N,) f32."""
+    h = np.asarray(h, F32)
+    x, y = a[:, 0].astype(F32), a[:, 1].astype(F32)
+    X = fma32(h[:, 0], x, fma32(h[:, 1], y, h[:, 2]))
+    Y = fma32(h[:, 3], x, fma32(h[:, 4], y, h[:, 5]))
+    dx = fma32(X, ww, -b[:, 0].astype(F32))
+    dy = fma32(Y, ww, -b[:, 1].astype(F32))
+    with np.errstate(all="ignore"):
+        return fma32(dx, dx, dy * dy)
+
+
+def rcp_candidates(den, k=4):
+    """Every f32 within 2^-23 relative of 1/den (what the bound assumes of rcp.approx): (N, 2k+1) f32 candidates and a
+    mask of the admissible ones.  |w - 1/den| <= 2^-23 |1/den|  <=>  |w den - 1| <= 2^-23, exact in f64."""
+    den = np.asarray(den, F32)
+    with np.errstate(all="ignore"):
+        w0 = (1.0 / den.astype(np.float64)).astype(F32)
+    cand = [w0]
+    lo = hi = w0
+    for _ in range(k):
+        lo = np.nextafter(lo, F32(-np.inf))
+        hi = np.nextafter(hi, F32(np.inf))
+        cand = [lo] + cand + [hi]
+    w = np.stack(cand, 1)
+    with np.errstate(all="ignore"):
+        ok = np.abs(w.astype(np.float64) * den.astype(np.float64)[:, None] - 1.0) <= 2.0 ** -23
+    return w, ok
+
+
+def fused_err_range32(h, a, b):
+    """(min, max) of reproj_err_fused over every admissible reciprocal, and the fused denominator."""
+    den = fused_den32(h, a)
+    w, ok = rcp_candidates(den)
+    e = np.stack([reproj_err_fused32(h, a, b, w[:, j]) for j in range(w.shape[1])], 1)
+    with np.errstate(all="ignore"):
+        emin = np.where(ok, e, F32(np.inf)).min(1)
+        emax = np.where(ok, e, F32(-np.inf)).max(1)
+    return emin, emax, den
+
+
+def _bound_terms32(h, cmax):
+    h = np.abs(np.asarray(h, F32))
+    cmax = np.asarray(cmax, F32)
+    with np.errstate(all="ignore"):
+        a6 = h[:, 6] + h[:, 7]
+        Bd = a6 * cmax + F32(1)
+        Bx = (h[:, 0] + h[:, 1]) * cmax + h[:, 2]
+        By = (h[:, 3] + h[:, 4]) * cmax + h[:, 5]
+        lim = (F32(8) * U) * Bd <= F32(0.1) * DEN_MIN
+        dm = np.fmax(F32(0.9) * DEN_MIN, ((F32(1) - a6 * cmax) - (F32(8) * U) * Bd) * F32(0.999999))
+        rho = ((F32(4) * U) * Bd) / dm + F32(2) * U
+        dX = F32(2.5) * ((Bx / dm) * (F32(6) * U + rho) + U * cmax)
+        dY = F32(2.5) * ((By / dm) * (F32(6) * U + rho) + U * cmax)
+        return a6, Bd, lim, dX + dY
+
+
+def fused_D32(h, cmax):
+    """D of fused_thresholds (bound on |dx_exact - dx_fused| + |dy_exact - dy_fused|)."""
+    return _bound_terms32(h, cmax)[3]
+
+
+def den_safe32(h, cmax):
+    """den_safe(h6, h7, cmax) in the device's operation order: h (N,8) f32."""
+    a6, Bd, lim, _ = _bound_terms32(h, cmax)
+    cmax = np.asarray(cmax, F32)
+    with np.errstate(all="ignore"):
+        return lim & (((F32(1) - a6 * cmax) - (F32(8) * U) * Bd) * F32(0.999999) >= DEN_MIN)
+
+
+def fused_thresholds32(h, cmax, t, exact_only=False):
+    """(tlo, thi) of fused_thresholds in the device's operation order: h (N,8) f32, cmax and t scalars or (N,) f32."""
+    _, _, lim, D = _bound_terms32(h, cmax)
+    t = np.broadcast_to(np.asarray(t, F32), D.shape)
+    tlo = np.full(D.shape, -np.inf, F32)
+    thi = np.full(D.shape, np.inf, F32)
+    use = lim & (D < F32(1e6)) & (not exact_only)
+    with np.errstate(all="ignore"):
+        s = np.sqrt(t)
+        rnd = np.fmax(F32(1e-4), (F32(8) * U) * t)
+        th = (t + F32(1.25) * ((F32(2) * D) * D + (F32(2) * D) * np.sqrt(D * D + t))) + rnd
+        tl = (t - (F32(2.5) * s) * D) - rnd
+    thi = np.where(use, th, thi)
+    tlo = np.where(use & (D < s), tl, tlo)
+    return tlo.astype(F32), thi.astype(F32)
+
+
+FUSED_BOUND_THRESHOLDS = (0.5, 0.75, 1.0, 3.0, 5.0, 12.5, 32.0, 64.0, 100.0, 256.0)
+
+
+def fused_bound_family(rng, name, n):
+    """Parameters of near_threshold_cases for the families the fused bound is tested on (n base points)."""
+    pick = lambda: rng.choice(FUSED_BOUND_THRESHOLDS, n)
+    if name.startswith("thresh_"):                  # one threshold, near-identity models on a 1920 x 1080 frame
+        return dict(thresh=np.full(n, float(name[7:])))
+    if name == "scale":                             # frames of 0.05x to 100x 1920 x 1080
+        s = 10.0 ** rng.uniform(np.log10(0.05), 2.0, n)
+        return dict(thresh=pick(), scale=s, trans=8.0 * s)
+    if name == "translation":                       # translations up to 8 000 px
+        return dict(thresh=pick(), trans=rng.uniform(-8000, 8000, (n, 2)))
+    if name == "perspective":                       # (|h6| + |h7|) 1920 up to and just past the den_safe limit 15/16
+        return dict(thresh=pick(), persp_sum=rng.uniform(0.5, 1.0, n) * 0.9375 / 1920)
+    if name == "low_den":                           # denominators in [1, 1.5] kDenMin of either sign (dm floor)
+        return dict(thresh=pick(), persp_sum=rng.uniform(1.0, 3.0, n) / 1920, low_den=True)
+    if name == "small_coords":                      # points within 16 px, 100 px threshold
+        return dict(thresh=np.full(n, 100.0), scale=np.full(n, 16 / 1920), trans=rng.uniform(-1, 1, (n, 2)))
+    if name == "D_both_sides":                      # D on both sides of sqrt(t), the condition of the sure-inlier cut
+        s = 10.0 ** rng.uniform(1.0, 2.0, n)
+        return dict(thresh=rng.choice([0.5, 0.75], n), scale=s, trans=8.0 * s)
+    raise ValueError(name)
+
+
+FUSED_BOUND_FAMILIES = tuple(f"thresh_{t:g}" for t in FUSED_BOUND_THRESHOLDS) + (
+    "scale", "translation", "perspective", "low_den", "small_coords", "D_both_sides")
+
+
+def near_threshold_b(h, a, thresh, phi, walk=3):
+    """b = f32(pi(h a) + thresh (cos phi, sin phi)), projected in f64, and its f32 neighbours within `walk` ulps in each
+    coordinate: h (n,8) f32, a (n,2) f32 -> (n, (2 walk + 1)^2, 2) f32."""
+    n = len(h)
+    h64, a64 = h.astype(np.float64), a.astype(np.float64)
+    den = h64[:, 6] * a64[:, 0] + h64[:, 7] * a64[:, 1] + 1.0
+    px = (h64[:, 0] * a64[:, 0] + h64[:, 1] * a64[:, 1] + h64[:, 2]) / den
+    py = (h64[:, 3] * a64[:, 0] + h64[:, 4] * a64[:, 1] + h64[:, 5]) / den
+    with np.errstate(all="ignore"):
+        b0 = np.stack([px + thresh * np.cos(phi), py + thresh * np.sin(phi)], 1).astype(F32)
+    k = 2 * walk + 1
+    bz = np.repeat(b0[:, 0], k * k).reshape(n, k, k)
+    bw = np.repeat(b0[:, 1], k * k).reshape(n, k, k)
+    for s in range(1, walk + 1):       # bz[:, i, :] = b0.x moved i - walk ulps, bw[:, :, j] = b0.y moved j - walk ulps
+        for arr, ax in ((bz, 1), (bw, 2)):
+            for sgn, idx in ((1, walk + s), (-1, walk - s)):
+                sl = [slice(None)] * 3
+                sl[ax] = idx
+                prev = [slice(None)] * 3
+                prev[ax] = idx - sgn
+                arr[tuple(sl)] = np.nextafter(arr[tuple(prev)], F32(sgn * np.inf))
+    return np.stack([bz.reshape(n, -1), bw.reshape(n, -1)], 2).astype(F32)
+
+
+def near_threshold_cases(rng, n, thresh, scale=1.0, trans=8.0, persp=1e-5, persp_sum=None, low_den=False, walk=3):
+    """Point pairs whose exact error lies within a few ulps of thresh^2 on both sides, under random f32 models.
+
+    n base points (every argument a scalar or one value per base point): a near-identity model h (rotation ~0.02 rad,
+    scale ~1e-3; translation ~N(0, trans), or trans itself when it has shape (n, 2); perspective ~N(0, persp / scale),
+    or of random signs with |h6| + |h7| = persp_sum), a point a in the frame [0, 1920 scale] x [0, 1080 scale] (low_den:
+    moved to where the f64 denominator lies in [1, 1.5] kDenMin, of either sign), b = f32(pi(h a) + thresh (cos phi,
+    sin phi)) in f64, then every f32 neighbour of b within `walk` ulps in each coordinate.  Returns h (N,8) f32, a, b
+    (N,2) f32, t = f32(thresh^2) and cmax (N,) f32 (the frame, or the largest |coordinate| of the pair when larger) with
+    N = n (2 walk + 1)^2."""
+    thresh = np.broadcast_to(np.asarray(thresh, np.float64), (n,))
+    scale = np.broadcast_to(np.asarray(scale, np.float64), (n,))
+    th = rng.normal(size=n) * 0.02
+    sc = 1 + rng.normal(size=n) * 1e-3
+    tr = np.asarray(trans, np.float64)
+    tr = tr if tr.shape == (n, 2) else rng.normal(size=(n, 2)) * np.broadcast_to(tr, (n,))[:, None]
+    if persp_sum is None:
+        pp = rng.normal(size=(n, 2)) * (np.broadcast_to(np.asarray(persp, np.float64), (n,)) / scale)[:, None]
+    else:
+        f = rng.random(n)
+        pp = np.stack([f, 1 - f], 1) * np.broadcast_to(np.asarray(persp_sum, np.float64), (n,))[:, None]
+        pp *= rng.choice([-1.0, 1.0], (n, 2))
+    h = np.stack([sc * np.cos(th), -sc * np.sin(th), tr[:, 0], sc * np.sin(th), sc * np.cos(th), tr[:, 1],
+                  pp[:, 0], pp[:, 1]], 1).astype(F32)
+    frame = np.array([1920.0, 1080.0]) * scale[:, None]
+    a = rng.random((n, 2)) * frame
+    if low_den:
+        # move a along the gradient of the denominator until den = target (in f64), inside the frame when possible
+        g = h[:, 6:8].astype(np.float64)
+        target = rng.uniform(1.0, 1.5, n) * float(DEN_MIN) * rng.choice([-1.0, 1.0], n)
+        d0 = 1.0 + (g * a).sum(1)
+        a = a + ((target - d0) / (g * g).sum(1))[:, None] * g
+    a = a.astype(F32)
+    b = near_threshold_b(h, a, thresh, rng.uniform(0, 2 * np.pi, n), walk).reshape(-1, 2)
+    k = 2 * walk + 1
+    a = np.repeat(a, k * k, 0)
+    h = np.repeat(h, k * k, 0)
+    t = np.repeat((thresh * thresh).astype(F32), k * k)
+    with np.errstate(all="ignore"):
+        cmax = np.maximum(np.repeat(frame.max(1), k * k).astype(F32), np.maximum(np.abs(a).max(1), np.abs(b).max(1)))
+    return h, a, b, t, cmax.astype(F32)
+
+
 # ----------------------------------------------------------------------------- refit
 def dlt_normalised(a, b):
     """OpenCV HomographyEstimatorCallback::runKernel: per-axis mean-abs-deviation
